@@ -5,6 +5,7 @@ configs[1]) through the B200 render path, one process per GPU.
     python bench.py --gpus 1 --steps 5 --warmup 3
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # CPU arm: the oracle port on the host cores
+    python bench.py --dump-outputs DIR ...    # also write what the last timed step returned, DIR/<name>.npy
 
 A step renders ONE full frame: the 640,000 rays are sharded over the ranks by contiguous pixel rows
 (no data-path collective; the final image gather is the only exchange), so scaling is "strong".
@@ -71,7 +72,35 @@ def parse():
                     help="render = the headline NeRF 800x800 frame (default; BASELINE.json configs[1]); the others are the "
                          "secondary BASELINE configs: train = 4096-ray NeRF training step (configs[2]), pigan = pi-GAN 128x128 "
                          "24+24 x 64 latents (configs[3]), grid = 256^3 density query (configs[4])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="headline render on one GPU: after the timed steps, write the six per-ray maps the last timed step returned "
+                         "(rgb_c, depth_c, acc_c, rgb_f, depth_f, acc_f) as DIR/<name>.npy in float32, so that two builds can be "
+                         "compared output for output; inputs are seeded, so the same arguments give the same inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "b200" or args.config != "render"):
+        ap.error("--dump-outputs applies to the headline render (--impl b200 --config render)")
+    return args
+
+
+DUMP_LIMIT_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir: str, maps: dict) -> None:
+    """Writes each per-ray map (first dimension = rays) as out_dir/<name>.npy in float32.  When the maps together exceed
+    DUMP_LIMIT_BYTES, every map is cut to the same fixed, seeded sample of rays, whose indices go to ray_index.npy (float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    maps = {k: v.detach().float().cpu().numpy() for k, v in maps.items()}
+    n = len(next(iter(maps.values())))
+    ray_bytes = sum(a[:1].nbytes for a in maps.values())
+    if n * ray_bytes > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - 4096) // (ray_bytes + 8)         # 4096: room for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(n, size=keep, replace=False))
+        maps = {k: a[idx] for k, a in maps.items()}
+        maps["ray_index"] = idx.astype(np.float64)
+    for k, a in maps.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 def peaks():
@@ -310,6 +339,8 @@ def run_b200(args):
         os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
         dist.init_process_group("nccl", device_id=dev)
     assert _lib.lib().b2r_device_ok() == 1
+    if args.dump_outputs is not None and world > 1:
+        raise SystemExit("--dump-outputs writes the maps of one process's render: run it on one GPU")
 
     W, H, sc, sf = args.width, args.height, args.coarse, args.fine
     n_rays = W * H
@@ -344,19 +375,21 @@ def run_b200(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """(total ms of `steps` calls of fn, what the last call returned)"""
         barrier()
         gc.collect(); gc.disable()              # no cyclic-GC pause of the interpreter inside a timed region
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()                             # kept: the earlier steps free their outputs before the next step allocates
         e1.record()
         barrier()
         gc.enable()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item())
+        return float(ms.item()), last
 
     for _ in range(max(args.warmup, 3)):
         step_device()
@@ -364,10 +397,13 @@ def run_b200(args):
     if rank == 0:
         clocks.start()
     stats0 = dict(ops.last_sample_stats)
-    total_ms = timed(step_device, args.steps)
+    total_ms, last = timed(step_device, args.steps)
     if rank == 0:                       # clocks are sampled during the headline's timed region only: every nvidia-smi query takes a driver
         clocks.stop_flag = True         # lock, which the host-synchronous end-to-end loop below would feel as stalls of several ms
         clocks.join(timeout=6)
+    if args.dump_outputs is not None:
+        dump_outputs(args.dump_outputs, dict(zip(("rgb_c", "depth_c", "acc_c", "rgb_f", "depth_f", "acc_f"), last)))
+    del last
     ms_per_step = total_ms / args.steps
     value = n_rays / (ms_per_step * 1e-3)
     # the headline runs with the last-sample sign check ON (the tolerance-conformant default, DESIGN.md 3.2); the same frame with the
@@ -378,7 +414,7 @@ def run_b200(args):
         passes = max(stats1["calls"] - stats0["calls"], 1)
         ops.set_exact_last_sample(False)
         step_device()
-        off_ms = timed(step_device, args.steps) / args.steps
+        off_ms = timed(step_device, args.steps)[0] / args.steps
         ops.set_exact_last_sample(True)
         last_sample = dict(check="on (default)", rays_checked_per_step=(stats1["rays"] - stats0["rays"]) // args.steps,
                            rays_reevaluated_fp32_per_step=(stats1["flagged"] - stats0["flagged"]) // args.steps,
@@ -400,7 +436,7 @@ def run_b200(args):
         same = all(bool(torch.equal(full[i], alt[i])) for i in (3, 4, 5))
         del full, alt
         step_dce()
-        dce_ms = timed(step_dce, args.steps) / args.steps
+        dce_ms = timed(step_dce, args.steps)[0] / args.steps
         dce = dict(metric=METRIC + " (coarse pass sigma-only)", value=n_rays / (dce_ms * 1e-3), unit="rays/s", ms_per_step=dce_ms, dtype="bf16",
                    scaling="strong", n_gpus=world, steps=args.steps, warmup=max(args.warmup, 3), higher_is_better=True, vs_baseline=None,
                    data="synthetic", fine_maps_bit_identical_to_headline=same,
@@ -458,7 +494,7 @@ def run_b200(args):
 
     def step_e2e_clocked():
         t1 = time.perf_counter(); step_e2e(); per_frame.append(round((time.perf_counter() - t1) * 1e3, 2))
-    e2e_event_ms = timed(step_e2e_clocked, args.steps)
+    e2e_event_ms = timed(step_e2e_clocked, args.steps)[0]
     wall_ms = float(sum(per_frame))                     # every frame ends with its own synchronisation: the frames' wall clocks add up
     stage_pool = [(_u, _i) for _b, _i in nerf_render._host_stage.get((dev.index, n_rays), []) for _u in [nerf_render._storage_uses(_b)]]
     e2e_ms = max(e2e_event_ms, wall_ms) / args.steps    # the D2H copies block the host: take the larger clock
@@ -764,7 +800,7 @@ def run_secondary(args, config=None, embedded=False):
             else:                                    # more ranks than latents: this rank only joins the all-reduce and applies the update
                 dist.all_reduce(gstep.grads.zero_())
                 gstep._opt()
-        ms = timed(step, min(args.steps, 3), args.warmup)
+        ms = timed(step, args.steps, args.warmup)
         rows = n_lat * res * res * 2 * s_
         line = dict(metric="rays/s, pi-GAN gradient step through the renderer (4 latents x 64x64, 24+24 samples; d/dfilm + d/dweights)",
                     value=n_lat * res * res / (ms * 1e-3), unit="rays/s", ms_per_step=ms, dtype="bf16", scaling="strong",

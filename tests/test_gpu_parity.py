@@ -1672,6 +1672,30 @@ def test_bench_contract_one_json_line_with_all_keys():
         assert k in d["roofline"]
 
 
+def test_bench_dump_outputs_are_the_seeded_render(tmp_path):
+    """bench.py --dump-outputs writes the six per-ray maps of the last timed step as float32 .npy files, and they are the maps
+    render_image_device returns for the bench's seeded inputs (weights seed 0, jitter seed 5, its camera)."""
+    import sys
+    w = h = 96
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--width", str(w), "--height", str(h), "--steps", "2", "--warmup", "3",
+                        "--no-cpu-baseline", "--no-secondary", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    names = ("rgb_c", "depth_c", "acc_c", "rgb_f", "depth_f", "acc_f")
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(n + ".npy" for n in names)
+    torch.manual_seed(0)
+    coarse, fine = models.NeRF().cuda(), models.NeRF().cuda()
+    pose = pigan_render.camera_pos_to_transform_matrix(4.0, 0.3, -30 * np.pi / 180)
+    torch.manual_seed(5)
+    t_rand = torch.rand((w * h, 64), device="cuda")
+    with torch.no_grad():
+        want = nerf_render.render_image_device(w, h, w * 1.3875, pose, 2.0, 6.0, coarse, fine, 64, 128, t_rand=t_rand, precision="bf16",
+                                               exact_last_sample=True, coarse_outputs_unused=True)
+    for name, ref in zip(names, want):
+        got = np.load(tmp_path / (name + ".npy"))
+        assert got.dtype == np.float32 and np.isfinite(got).all(), name
+        assert np.array_equal(got, ref.cpu().numpy()), name
+
+
 def test_film_batched_training_random_shapes():
     """tools/stress_film_train.py (random latent counts, rows per latent, samples per ray: odd tile counts, latents that
     start in the middle of a CTA's tile walk): the batched fused training call reproduces latent 0's rows bit-exactly and its
