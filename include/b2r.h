@@ -173,9 +173,7 @@ typedef struct b2r_last_sample {
  * the `saved` argument of b2r_mlp_f32_bwd.  use_dir: FilmSirenNeRF(use_dir=...) flag. */
 size_t b2r_mlp_f32_workspace_bytes(int model_kind, long long rows, int save_activations);
 /* gemm_mode: 0 = fp32 FMAs on the CUDA cores (exact: the fp32 parity path), 1 = the same layer-wise algorithm with the
- * GEMMs on the tensor cores in TF32 (tcgen05 kind::tf32, fp32 accumulate; ~1e-3 relative), 2 = GEMMs in bf16 (tcgen05
- * kind::f16: the fp32 buffers are converted while staging, fp32 accumulate; bf16 class: the fast layer-wise training path
- * of FiLM-SIREN and SirenNeRF). */
+ * GEMMs on the tensor cores in TF32 (tcgen05 kind::tf32, fp32 accumulate; ~1e-3 relative).  Any other value is rejected. */
 int b2r_mlp_f32_fwd(int model_kind, const float* params, const float* film, int use_dir,
                     const b2r_mlp_input* in, float* raw_out, void* workspace, size_t workspace_bytes,
                     int save_activations, int gemm_mode, void* stream);

@@ -10,7 +10,6 @@
 //                          pi_GAN/synthesis.py:107); formulas SURVEY.md A.5 / A.6
 #include "sgemm.cuh"
 #include "tgemm.cuh"
-#include "bgemm.cuh"
 
 namespace b2r {
 
@@ -292,8 +291,7 @@ __global__ void __launch_bounds__(256) siren_first_layer_kernel(const float* __r
     if (pre) *reinterpret_cast<float4*>(pre + row * 256 + n0) = make_float4(a[0], a[1], a[2], a[3]);
 }
 
-// GEMM engine of the current call on this host thread: 0 = fp32 CUDA cores (exact), 1 = tf32 tensor cores (tgemm.cuh),
-// 2 = bf16 tensor cores (bgemm.cuh: fp32 buffers converted while staging, MN-major operands instead of transposes).
+// GEMM engine of the current call on this host thread: 0 = fp32 CUDA cores (exact), 1 = tf32 tensor cores (tgemm.cuh).
 // thread_local, set at every API entry: the library stays re-entrant (nn.DataParallel calls it from one thread per GPU).
 static thread_local int t_gemm_mode = 0;
 // b2r_mlp_f32_last_sigma on a latent batch: latent of every gathered row (FiLM scale / shift row of the sine epilogue)
@@ -302,7 +300,6 @@ static thread_local const int* t_row_lat = nullptr;
 template <bool kPT, bool kQT>
 static int launch_gemm(GemmArgs g, cudaStream_t st, const char* what) {
     // tiny reductions (K = 3 input layer) stay on the CUDA cores
-    if (t_gemm_mode == 2 && g.R >= 16) return bg::launch_bgemm<kPT, kQT>(g, st, what);
     if (t_gemm_mode == 1 && g.R >= 16) return tg::launch_tgemm<kPT, kQT>(g, st, what);
     return launch_sgemm<kPT, kQT>(g, st, what);
 }
@@ -314,8 +311,8 @@ static inline Lin lin(const float* params, LayerDesc d) { return Lin{params + d.
 static int fwd_layer(const float* X, long long ldx, Lin L, int k_off, int K, float* Y, long long ldy, long long rows,
                      int epi, cudaStream_t st, const float* gamma = nullptr, const float* beta = nullptr,
                      float* pre = nullptr) {
-    if (t_gemm_mode != 0 && K == 3 && L.in == 3 && L.out == 256 && epi == EPI_FILM_SIN && ldy % 4 == 0 && aligned16(Y) && (!pre || aligned16(pre))) {
-        // tensor-core modes: the K = 3 first layer is no GEMM (the exact fp32 mode keeps the sgemm path its parity fixtures were made with)
+    if (t_gemm_mode == 1 && K == 3 && L.in == 3 && L.out == 256 && epi == EPI_FILM_SIN && ldy % 4 == 0 && aligned16(Y) && (!pre || aligned16(pre))) {
+        // tf32 mode: the K = 3 first layer is no GEMM (the exact fp32 mode keeps the sgemm path its parity fixtures were made with)
         const long long threads = rows * 64;
         siren_first_layer_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, st>>>(X, ldx, L.W, L.b, gamma, beta, rows, Y, ldy, pre);
         return cuda_result(cudaGetLastError(), "siren first layer");
@@ -341,7 +338,7 @@ static int wgrad_layer(const float* G, long long ldg, const float* X, long long 
                        long long rows, cudaStream_t st) {
     GemmArgs g{};
     g.P = G; g.ldp = ldg; g.Q = X; g.ldq = ldx; g.C = d_params + d.w_off; g.ldc = d.in;
-    g.I = d.out; g.J = d.in; g.R = rows; g.r_chunk = t_gemm_mode >= 1 ? 8192 : 2048; g.epi = EPI_ATOMIC;
+    g.I = d.out; g.J = d.in; g.R = rows; g.r_chunk = t_gemm_mode == 1 ? 8192 : 2048; g.epi = EPI_ATOMIC;
     int rc = launch_gemm<true, true>(g, st, "mlp_f32 wgrad gemm");
     if (rc) return rc;
     int rpc = 512;
@@ -468,7 +465,7 @@ extern "C" int b2r_mlp_f32_fwd(int model_kind, const float* params, const float*
                                const b2r_mlp_input* in, float* raw_out, void* workspace, size_t workspace_bytes,
                                int save_activations, int gemm_mode, void* stream) {
     using namespace b2r;
-    B2R_CHECK_ARG(gemm_mode >= 0 && gemm_mode <= 2, "b2r_mlp_f32_fwd: gemm_mode must be 0 (fp32), 1 (tf32) or 2 (bf16)");
+    B2R_CHECK_ARG(gemm_mode == 0 || gemm_mode == 1, "b2r_mlp_f32_fwd: gemm_mode must be 0 (fp32) or 1 (tf32)");
     t_gemm_mode = gemm_mode;
     B2R_CHECK_ARG(known_kind(model_kind), "b2r_mlp_f32_fwd: unknown model kind %d", model_kind);
     B2R_CHECK_ARG(params && raw_out && workspace, "b2r_mlp_f32_fwd: NULL pointer");
@@ -565,7 +562,7 @@ extern "C" int b2r_mlp_f32_bwd(int model_kind, const float* params, const float*
                                const b2r_mlp_input* in, const float* raw, const float* d_raw, const void* saved,
                                void* scratch, size_t scratch_bytes, float* d_params, float* d_film, int gemm_mode, void* stream) {
     using namespace b2r;
-    B2R_CHECK_ARG(gemm_mode >= 0 && gemm_mode <= 2, "b2r_mlp_f32_bwd: gemm_mode must be 0 (fp32), 1 (tf32) or 2 (bf16)");
+    B2R_CHECK_ARG(gemm_mode == 0 || gemm_mode == 1, "b2r_mlp_f32_bwd: gemm_mode must be 0 (fp32) or 1 (tf32)");
     t_gemm_mode = gemm_mode;
     B2R_CHECK_ARG(known_kind(model_kind), "b2r_mlp_f32_bwd: unknown model kind %d", model_kind);
     B2R_CHECK_ARG(params && raw && d_raw && saved && scratch, "b2r_mlp_f32_bwd: NULL pointer");

@@ -18,7 +18,8 @@ from . import _lib, models
 from ._lib import LastSample, MlpInput, check, lib, ptr
 
 # MLP arithmetic used when no gradient is required: "bf16" = fused tcgen05 kernel (mlp_tc.cu),
-# "fp32" = layer-wise CUDA-core path (mlp_f32.cu).  The arithmetic of the gradient path is _GRAD_PRECISION below.
+# "fp32" = layer-wise path on CUDA-core FMAs (mlp_f32.cu, sgemm.cuh), "tf32" = the same layer-wise path with its GEMMs on
+# tcgen05 kind::tf32 (tgemm.cuh).  The arithmetic of the gradient path is _GRAD_PRECISION below.
 _MLP_PRECISION = "bf16"
 
 
@@ -34,18 +35,18 @@ def get_mlp_precision() -> str:
     return _MLP_PRECISION
 
 
-# Arithmetic of the path used whenever gradients are required: "fp32" = layer-wise, CUDA-core FMAs (exact: the parity path),
-# "tf32" = the same algorithm with every GEMM on the tensor cores (tcgen05 kind::tf32, fp32 accumulate), "bf16" = the fused
-# tensor-core training path (mlp_tc.cu forward with kept bf16 activations + mlp_tc_train.cu reverse mode, fp32 master weights /
-# gradients; NeRF model only -- other models run the layer-wise algorithm with bf16 tensor-core GEMMs, bgemm.cuh), "auto" (default) = "bf16":
-# the same arithmetic class the no-grad render path uses by default.  "fp32" is the exact path the gradient parity fixtures are checked on.
-_GRAD_PRECISION = "auto"
+# Arithmetic of the path used whenever gradients are required, one engine each: "fp32" = layer-wise, CUDA-core FMAs (sgemm.cuh;
+# exact: the path the gradient parity fixtures are checked on), "tf32" = the same layer-wise algorithm with every GEMM on the
+# tensor cores (tgemm.cuh, tcgen05 kind::tf32, fp32 accumulate), "bf16" (default) = the fused tensor-core training path of all
+# three model kinds (mlp_tc.cu / mlp_tc_siren.cu forward with kept bf16 activations + mlp_tc_train.cu reverse mode, fp32 master
+# weights / gradients): the same arithmetic class the no-grad render path uses by default.
+_GRAD_PRECISION = "bf16"
 
 
 def set_grad_precision(p: str) -> str:
     global _GRAD_PRECISION
-    if p not in ("auto", "fp32", "tf32", "bf16"):
-        raise ValueError("grad precision must be 'auto', 'fp32', 'tf32' or 'bf16'")
+    if p not in ("fp32", "tf32", "bf16"):
+        raise ValueError("grad precision must be 'fp32', 'tf32' or 'bf16'")
     old, _GRAD_PRECISION = _GRAD_PRECISION, p
     return old
 
@@ -705,14 +706,11 @@ def mlp(model, rays: torch.Tensor | None = None, z: torch.Tensor | None = None, 
     if needs_grad:
         if grid is not None:
             raise RuntimeError("grid queries are inference-only")
-        gp = _GRAD_PRECISION
-        if gp == "auto":
-            gp = "bf16"
-        if gp == "bf16" and kind in (models.KIND_NERF, models.KIND_SIREN):
+        if _GRAD_PRECISION == "bf16":
+            if kind == models.KIND_FILM:
+                return _MlpTcTrainFilm.apply(flat, film, rays, z, x, 0, use_dir)
             return _MlpTcTrain.apply(flat, net, kind, rays, z, x)
-        if gp == "bf16" and kind == models.KIND_FILM:
-            return _MlpTcTrainFilm.apply(flat, film, rays, z, x, 0, use_dir)
-        return _MlpF32.apply(flat, film, kind, use_dir, rays, z, x, {"fp32": 0, "tf32": 1, "bf16": 2}[gp])
+        return _MlpF32.apply(flat, film, kind, use_dir, rays, z, x, 1 if _GRAD_PRECISION == "tf32" else 0)
     inp, rows, keep = _make_input(rays, z, x, grid)
     raw = torch.empty((rows, 4), dtype=torch.float32, device=dev)
     if rows == 0:

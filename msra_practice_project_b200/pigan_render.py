@@ -101,7 +101,7 @@ def render_batch(model, film_params, poses, width, height, focal, near, far, coa
         raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
     used = precision or ops.get_mlp_precision()
     grad = torch.is_grad_enabled() and _needs_grad(model, film_params)
-    grad_ok = ops.get_grad_precision() in ("auto", "bf16") and isinstance(film_params, torch.Tensor)
+    grad_ok = ops.get_grad_precision() == "bf16" and isinstance(film_params, torch.Tensor)
     batched = (not grad or grad_ok) and used == "bf16" and b > 0 and (w * h * sc) % 512 == 0 and (w * h * (sc + sf)) % 512 == 0
     if not batched:
         imgs = []

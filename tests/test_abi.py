@@ -48,6 +48,21 @@ def test_bad_arguments_return_negative_and_set_message():
     assert rc < 0 and b"exactly one" in lib.b2r_last_error()
     with pytest.raises(RuntimeError):
         _lib.check(rc, "b2r_mlp_tc_fwd")
+    # the layer-wise path has two GEMM engines, 0 (fp32) and 1 (tf32); gemm_mode is checked before anything else (the calls
+    # below would otherwise fail on the 64-byte workspace / on having nothing to differentiate)
+    inp.x, inp.n_rays, inp.n_samples = 256, 512, 1
+    assert lib.b2r_mlp_f32_fwd(0, 16, None, 1, C.byref(inp), 16, 16, 64, 1, 2, None) < 0 and b"gemm_mode" in lib.b2r_last_error()
+    assert lib.b2r_mlp_f32_bwd(0, 16, None, 1, C.byref(inp), 16, 16, 16, 16, 1 << 30, None, None, 2, None) < 0 \
+        and b"gemm_mode" in lib.b2r_last_error()
+
+
+def test_grad_precision_names():
+    """One engine per gradient precision: fp32 / tf32 = the layer-wise path, bf16 (default) = the fused training path."""
+    from msra_practice_project_b200 import ops
+    assert ops.get_grad_precision() == "bf16"
+    with pytest.raises(ValueError):
+        ops.set_grad_precision("auto")
+    assert ops.get_grad_precision() == "bf16"
 
 
 def test_training_and_batched_entry_points_sizes_and_argument_checks():

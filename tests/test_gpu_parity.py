@@ -1050,10 +1050,10 @@ def test_siren_nerf_forward_and_training_gradients(golden, exact_grads):
     m = models.SirenNeRF().cuda()
     with torch.no_grad():
         out = ops.mlp(m, x=cu(g["x"]), precision="fp32").cpu().numpy()
-        out_tf32 = ops.mlp(m, x=cu(g["x"])).cpu().numpy()              # default precision -> tf32 tensor-core GEMMs
+        out_bf16 = ops.mlp(m, x=cu(g["x"])).cpu().numpy()              # default precision -> fused bf16 tensor-core kernel
     np.testing.assert_allclose(out[:, :3], g["out"][:, :3], atol=2e-4, rtol=0)
     np.testing.assert_allclose(out[:, 3], g["out"][:, 3], atol=2e-4, rtol=1e-3)
-    assert np.abs(out_tf32[:, :3] - g["out"][:, :3]).max() < 2e-2
+    assert np.abs(out_bf16[:, :3] - g["out"][:, :3]).max() < 2e-2
     torch.manual_seed(0)
     c, f = models.SirenNeRF().cuda(), models.SirenNeRF().cuda()
     rc, _, _, rf, _, _ = nerf_render.render_rays(cu(g["rays"]), 2.0, 6.0, c, f, 16, 16, t_rand=cu(g["t_rand"]), z_lin=g["z_lin"], u=g["u"],
@@ -1178,63 +1178,12 @@ def test_fused_train_step_draws_its_own_jitter_inside_the_graph(golden):
     assert (step.params - step2.params).abs().max().item() <= 2 * 5e-4 + 1e-6
 
 
-@pytest.mark.parametrize("kind", ["nerf", "siren", "film"])
-def test_bf16_layerwise_engine_matches_fp32(golden, kind):
-    """The bf16 tensor-core GEMM engine of the layer-wise path (bgemm.cuh: fp32 buffers converted while staging, K-major
-    and MN-major operands -- no transposes) for all three model kinds: forward values and every gradient against the
-    fp32 CUDA-core engine on the same inputs.  It is the engine FiLM-SIREN / SirenNeRF training uses under
-    ops.set_grad_precision("bf16"); ragged row counts, the 316 / 280 / 259-wide skip layers and the K = 3 input layers."""
-    g = torch.Generator().manual_seed(21)
-    n, s = 330, 7                                               # 2310 rows: ragged 128-row tiles
-    o = torch.tensor([0.0, 0.0, 1.2]).expand(n, 3)
-    d = torch.nn.functional.normalize(torch.randn(n, 3, generator=g) * 0.25 + torch.tensor([0.0, 0.0, -1.0]), dim=-1)
-    rays = torch.stack([o, d], 1).cuda()
-    z = (torch.sort(torch.rand(n, s, generator=g), -1).values * 1.0 + 0.5).cuda()
-    up = torch.randn(n * s, 4, generator=g).cuda()
-    torch.manual_seed(0)
-    film = None
-    if kind == "nerf":
-        net = models.damp_nerf_(models.NeRF()).cuda()
-    elif kind == "siren":
-        net = models.SirenNeRF().cuda()
-    else:
-        net = models.FilmSirenNeRF().cuda()
-        film = torch.cat([1.0 + 0.1 * torch.randn(9, 256, generator=g), 0.1 * torch.randn(9, 256, generator=g)], -1).cuda().requires_grad_(True)
-    res = {}
-    for mode, gm in (("fp32", 0), ("bf16", 2)):
-        net.zero_grad(set_to_none=True)
-        if film is not None:
-            film.grad = None
-            net.set_film_params(film)
-        ps = models.param_list(net)
-        flat = models.flat_params(net)
-        raw = ops._MlpF32.apply(flat, film, models.model_kind(net), True, rays, z, None, gm)
-        (raw * up).sum().backward()
-        grads = {k: p.grad.detach().clone() for k, p in net.named_parameters()}
-        if film is not None:
-            grads["film"] = film.grad.detach().clone()
-        res[mode] = (raw.detach().clone(), grads)
-        del ps
-    a, b = res["fp32"][0], res["bf16"][0]
-    err_rgb = (a[:, :3] - b[:, :3]).abs().max().item()
-    err_sig = ((a[:, 3] - b[:, 3]).abs() / (1 + a[:, 3].abs())).max().item()
-    worst = 0.0
-    for k in res["fp32"][1]:
-        gf, gb = res["fp32"][1][k].reshape(-1), res["bf16"][1][k].reshape(-1)
-        rel = (gf - gb).norm().item() / max(gf.norm().item(), 1e-20)
-        cos = torch.dot(gf, gb).item() / max(gf.norm().item() * gb.norm().item(), 1e-30)
-        worst = max(worst, rel)
-        assert cos > 0.9 and rel < 0.45, (kind, k, rel, cos)    # zero-mean random upstream: see test_bf16_tensor_core_training_path
-    print("bf16 layer-wise engine, %s: raw max-abs rgb %.3g, sigma rel %.3g; worst relative gradient error %.3g" % (kind, err_rgb, err_sig, worst))
-    assert err_rgb < 2e-2 and err_sig < 8e-2
-
-
 @pytest.mark.parametrize("rows_shape", [(37, 24), (700, 32), (1, 1)])
 def test_siren_nerf_fused_training_path(rows_shape):
     """SirenNeRF on the fused tensor-core training path (siren_tc_kernel<true> with bf16 activation + cosine checkpoints,
     nerf_tc_bwd_kernel<true>, MN-major wgrad with the aux tile): the training forward is bit-identical to the inference
     kernel; every parameter gradient against the exact fp32 layer-wise path (direction cosine >= 0.98, <= 0.12 relative L2
-    with >= 512 rows) and against the bf16 layer-wise engine (the same arithmetic class)."""
+    with >= 4096 rows)."""
     n, s = rows_shape
     g = torch.Generator().manual_seed(n + 5)
     torch.manual_seed(0)

@@ -1,4 +1,4 @@
-"""SirenNeRF fused training path bring-up: forward-train raw vs inference kernel; gradients vs fp32 / bf16 layer-wise."""
+"""SirenNeRF fused training path bring-up: forward-train raw vs inference kernel; gradients vs the fp32 layer-wise path."""
 import sys
 import torch
 from msra_practice_project_b200 import models, ops
