@@ -274,6 +274,24 @@ int b2r_mlp_tc_fwd_film_batched(const void* packed, int n_latents, long long row
  * train_nerf.py:199 quantise every frame on the host); lets frames leave the device as 1 byte per channel. */
 int b2r_to8b(const float* x, long long n, unsigned char* out, void* stream);
 
+/* ---- marching cubes ------------------------------------------- create_mesh  pi_GAN/utils.py:99-180 ----------------
+ * The level set of field[n0,n1,n2] (fp32, axis 0 slowest) as a triangle mesh; the table, the numbering and the rule that
+ * generates it: oracle/marching_cubes.py.  Two calls, because the output size is data-dependent:
+ *   b2r_mc_count: writes the per-point codes into scratch (b2r_mc_scratch_bytes(n0, n1, n2) bytes, 16-byte aligned) and
+ *                 totals_dev[2] = (V, F), the vertex and triangle counts, as two long long in DEVICE memory;
+ *   b2r_mc_emit:  given the scratch b2r_mc_count wrote for the same field and level, writes verts[V,3] (fp32) and
+ *                 faces[F,3] (int32 vertex indices).  The caller reads (V, F) first and must not call it when V or F
+ *                 exceeds INT32_MAX.
+ * Vertices are ordered by owner lattice point (linear index), then edge axis; the vertex on the edge from point p along
+ * axis a is origin + (p + t e_a) * spacing, t = (level - f(p)) / (f(p + e_a) - f(p)), every operation rounded separately.
+ * Triangles are ordered by cell (linear index of its minimum corner), then table order; their normals
+ * (v1-v0) x (v2-v0) point from below (f < level) to above.  Both calls need n >= 2 on every axis and n0*n1*n2 <= INT32_MAX;
+ * b2r_mc_scratch_bytes returns 0 for any other shape. */
+size_t b2r_mc_scratch_bytes(int n0, int n1, int n2);
+int b2r_mc_count(const float* field, int n0, int n1, int n2, float level, void* scratch, long long* totals_dev, void* stream);
+int b2r_mc_emit(const float* field, int n0, int n1, int n2, float level, float spacing, float ox, float oy, float oz,
+                const void* scratch, float* verts, int* faces, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

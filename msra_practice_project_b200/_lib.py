@@ -81,6 +81,10 @@ SIGNATURES = {
     "b2r_mlp_tc_pack_bwd_film": (C.c_int, [c_float_p, c_float_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "b2r_mlp_tc_train_bwd_film": (C.c_int, [C.c_void_p, c_float_p, c_float_p, C.c_int, C.c_int, c_ll, c_ll, c_float_p, c_float_p, C.c_void_p,
                                             C.c_void_p, C.c_size_t, c_float_p, c_float_p, c_float_p, C.c_void_p]),
+    "b2r_mc_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "b2r_mc_count": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b2r_mc_emit": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
+                              C.c_void_p, c_float_p, C.c_void_p, C.c_void_p]),
 }
 
 _lock = threading.Lock()

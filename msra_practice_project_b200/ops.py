@@ -784,3 +784,36 @@ def to8b(x: torch.Tensor) -> torch.Tensor:
     with torch.cuda.device(x.device):
         check(lib().b2r_to8b(ptr(x), x.numel(), ptr(out), _stream(x)), "b2r_to8b")
     return out
+
+
+_INT32_MAX = 2 ** 31 - 1
+
+
+def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, origin=(0.0, 0.0, 0.0)):
+    """Marching cubes of ``field`` [n0,n1,n2] (axis 0 slowest) at ``level`` on the device (b2r_mc_count / b2r_mc_emit; the
+    table and its rule: oracle/marching_cubes.py).  Returns ``(verts [V,3] float32, faces [F,3] int32)`` on the field's
+    device; vertex ``origin + (p + t e_a) * spacing`` lies on the lattice edge from point ``p`` along axis ``a``, and the
+    triangle normals point from ``field < level`` to ``field >= level``.  Synchronises once with the host to read the
+    mesh size (V, F), as ``torch.nonzero`` does.  Empty meshes are ``[0,3]`` tensors."""
+    field = _cuda_f32(field, "field")
+    if field.dim() != 3 or min(field.shape) < 2:
+        raise RuntimeError(f"field must be [n0,n1,n2] with every n >= 2, got {list(field.shape)}")
+    if field.numel() > _INT32_MAX:
+        raise RuntimeError(f"field has {field.numel()} points; marching_cubes takes at most 2^31 - 1")
+    n0, n1, n2 = (int(s) for s in field.shape)
+    level, spacing = float(level), float(spacing)
+    ox, oy, oz = (float(o) for o in origin)
+    dev = field.device
+    scratch = torch.empty((lib().b2r_mc_scratch_bytes(n0, n1, n2),), dtype=torch.uint8, device=dev)
+    totals = torch.empty((2,), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().b2r_mc_count(ptr(field), n0, n1, n2, level, ptr(scratch), ptr(totals), _stream(field)), "b2r_mc_count")
+        n_verts, n_faces = (int(v) for v in totals.tolist())
+        if n_verts > _INT32_MAX or n_faces > _INT32_MAX:
+            raise RuntimeError(f"mesh of {n_verts} vertices / {n_faces} triangles: int32 vertex indices hold at most 2^31 - 1")
+        verts = torch.empty((n_verts, 3), dtype=torch.float32, device=dev)
+        faces = torch.empty((n_faces, 3), dtype=torch.int32, device=dev)
+        if n_verts and n_faces:
+            check(lib().b2r_mc_emit(ptr(field), n0, n1, n2, level, spacing, ox, oy, oz, ptr(scratch), ptr(verts), ptr(faces),
+                                    _stream(field)), "b2r_mc_emit")
+    return verts, faces

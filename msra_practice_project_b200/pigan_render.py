@@ -160,12 +160,8 @@ def density_grid(model, N=256, max_batch=64 ** 3, *, begin=0, count=None, precis
     return out[0] if len(out) == 1 else torch.cat(out)
 
 
-def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=None):
-    """The sampling half of ``create_mesh`` (pi_GAN/utils.py:42-97; called by extract_mesh.py:49): draw z ~ N(0,1) on the
-    device, map it to FiLM parameters, condition the field and query -sigma on the N^3 lattice of [-0.1, 0.1]^3 with zero view
-    direction.  Returns what the reference hands to ``convert_sdf_samples_to_ply`` -- ``sdf_values`` as a CPU tensor
-    [N,N,N] (x slowest) -- plus ``voxel_origin`` and ``voxel_size``; marching cubes / PLY writing stay with the reference
-    (CPU, skimage: out of scope).  ``generator``: models.Generator or the reference's Generator (same attributes)."""
+def _sdf_device(generator, N, max_batch, z, precision):
+    """-sigma of the generator conditioned on z (drawn when None) on the N^3 lattice, as a CUDA tensor [N,N,N] (x slowest)."""
     dev = next(generator.parameters()).device
     if dev.type != "cuda":
         raise RuntimeError("generator parameters must live on a CUDA device: the B200 render path has no CPU fallback")
@@ -175,4 +171,44 @@ def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=No
         film_params = generator.get_mapping(z.to(dev))
         generator.set_film_params(film_params[0])
         sdf = density_grid(generator.film_siren_nerf, N=N, max_batch=max_batch, precision=precision)
-    return sdf.reshape(N, N, N).cpu(), [-0.1, -0.1, -0.1], 0.2 / (N - 1)
+    return sdf.reshape(N, N, N)
+
+
+def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=None):
+    """The sampling half of ``create_mesh`` (pi_GAN/utils.py:42-97; called by extract_mesh.py:49): draw z ~ N(0,1) on the
+    device, map it to FiLM parameters, condition the field and query -sigma on the N^3 lattice of [-0.1, 0.1]^3 with zero view
+    direction.  Returns what the reference hands to ``convert_sdf_samples_to_ply`` -- ``sdf_values`` as a CPU tensor
+    [N,N,N] (x slowest) -- plus ``voxel_origin`` and ``voxel_size``; ``create_mesh`` below keeps the sdf on the device and
+    extracts the mesh there.  ``generator``: models.Generator or the reference's Generator (same attributes)."""
+    return _sdf_device(generator, N, max_batch, z, precision).cpu(), [-0.1, -0.1, -0.1], 0.2 / (N - 1)
+
+
+def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None):
+    """``create_mesh`` (pi_GAN/utils.py:42-180) on the device: the sdf of ``create_mesh_sdf`` never leaves the GPU,
+    ``ops.marching_cubes`` extracts its level set (the reference's skimage call at level -20: below = sigma > 20, so the
+    triangle normals point out of the object), and only the mesh crosses to the host.  Returns ``(verts [V,3] float32,
+    faces [F,3] int32)`` on the device, in world coordinates (voxel origin -0.1, voxel size 0.2/(N-1)).  With
+    ``ply_filename`` the mesh is also written as the binary PLY the reference writes with plyfile (``vertex`` x/y/z f4,
+    ``face`` vertex_indices as a uchar-counted list of i4).  Synchronises with the host once to size the mesh."""
+    sdf = _sdf_device(generator, N, max_batch, z, precision)
+    verts, faces = ops.marching_cubes(sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1))
+    if ply_filename is not None:
+        write_ply(ply_filename, verts.cpu().numpy(), faces.cpu().numpy())
+    return verts, faces
+
+
+def write_ply(filename, verts, faces):
+    """Binary little-endian PLY of a triangle mesh, byte for byte what plyfile writes for the reference's elements
+    (pi_GAN/utils.py:158-180): ``vertex`` with float x/y/z, ``face`` with ``property list uchar int vertex_indices``."""
+    verts = np.ascontiguousarray(verts, dtype="<f4").reshape(-1, 3)
+    faces = np.asarray(faces).reshape(-1, 3)
+    body = np.empty(len(faces), dtype=[("n", "u1"), ("vertex_indices", "<i4", (3,))])
+    body["n"] = 3
+    body["vertex_indices"] = faces
+    header = ("ply\nformat binary_little_endian 1.0\n"
+              f"element vertex {len(verts)}\nproperty float x\nproperty float y\nproperty float z\n"
+              f"element face {len(faces)}\nproperty list uchar int vertex_indices\nend_header\n")
+    with open(filename, "wb") as fh:
+        fh.write(header.encode("ascii"))
+        verts.view([("x", "<f4"), ("y", "<f4"), ("z", "<f4")]).reshape(-1).tofile(fh)
+        body.tofile(fh)
