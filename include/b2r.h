@@ -130,12 +130,21 @@ int b2r_sample_pdf_generic(const float* bins, long long bins_stride, const float
 
 /* ---- K3: radiance-field MLP --- run_network nerf/render.py:59-75 + NeRF.forward nerf/nerf.py:75-94
  *                                 + FilmSirenNeRF.forward pi_GAN/modules.py:101-118 ------------
- * Input rows are described in one of three ways (exactly one must be given):
+ * Input rows are described in one of four ways (exactly one must be given):
  *   rays != NULL : rows = n_rays*n_samples, point = o + d*z[r,s], dir = d/|d|   (render_rays)
  *   x    != NULL : rows = n_rays (n_samples must be 1), x[rows,6] = (pos, dir)  (network(x))
  *   grid_n  > 0  : rows = n_rays = count of grid indices starting at grid_begin of an
  *                  N^3 lattice in [-0.1,0.1]^3, dir = 0            (create_mesh, pi_GAN/utils.py:59-91)
+ *   lattice_dims != 0 : box lattice, rows = n_rays = count of lattice indices starting at grid_begin of an
+ *                  n0 x n1 x n2 lattice (axis 0 slowest); index (i,j,k) is the point
+ *                  origin + (i,j,k) * voxel (each component a rounded fp32 multiply, then a rounded add), dir = 0.
+ *                  Needs every n >= 2, n0*n1*n2 <= INT32_MAX and a finite voxel > 0.  grid_n = N is the box lattice
+ *                  (N, N, N), origin -0.1, voxel (float)(0.2/(N-1)), row for row.
+ * Grid and lattice rows are for inference and mesh extraction: the last-sample check rejects them, and box-lattice rows go to
+ * b2r_mlp_tc_fwd / b2r_mlp_f32_fwd (the batched FiLM and tensor-core training entry points reject them).
  * raw_out[rows,4] = (sigmoid rgb, relu sigma).
+ * The struct grew by the three lattice_* fields after grid_begin (B2R_VERSION unchanged): a caller that zero-initialises
+ * it and sets only the older fields gets the older behaviour.
  */
 typedef struct b2r_mlp_input {
     const float* rays;      /* [n_rays,2,3] or NULL */
@@ -144,7 +153,10 @@ typedef struct b2r_mlp_input {
     long long n_rays;
     int n_samples;
     int grid_n;             /* >0: lattice mode */
-    long long grid_begin;
+    long long grid_begin;   /* first lattice index (grid_n or box-lattice mode) */
+    int lattice_dims[3];    /* any non-zero: box-lattice mode, points per axis (n0, n1, n2) */
+    float lattice_origin[3];
+    float lattice_voxel;
 } b2r_mlp_input;
 
 /* ---- the last interval of every ray ------------------------------------ raw_to_outputs nerf/render.py:91-93 ----
@@ -291,6 +303,13 @@ size_t b2r_mc_scratch_bytes(int n0, int n1, int n2);
 int b2r_mc_count(const float* field, int n0, int n1, int n2, float level, void* scratch, long long* totals_dev, void* stream);
 int b2r_mc_emit(const float* field, int n0, int n1, int n2, float level, float spacing, float ox, float oy, float oz,
                 const void* scratch, float* verts, int* faces, void* stream);
+/* Vertex normals of the same mesh: given the scratch b2r_mc_count wrote for the same field and level, writes normals[V,3] (fp32)
+ * in the vertex order of b2r_mc_emit.  g(p) is the field's gradient at lattice point p by differences along each axis,
+ * 0.5 (f[i+1] - f[i-1]) inside and f[i+1] - f[i] / f[i] - f[i-1] on the faces (np.gradient's scheme; the spacing is isotropic
+ * and dropped).  The vertex on the edge p -> p + e_a with parameter t gets n = g(p) + t (g(p + e_a) - g(p)) divided by |n|,
+ * every operation rounded separately (sqrt and division correctly rounded), so it points toward increasing field, the side
+ * the triangle normals face.  A zero-length n (a flat field there) gives (0, 0, 0). */
+int b2r_mc_normals(const float* field, int n0, int n1, int n2, float level, const void* scratch, float* normals, void* stream);
 
 #ifdef __cplusplus
 }

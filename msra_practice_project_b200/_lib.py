@@ -21,7 +21,8 @@ c_ll = C.c_longlong
 class MlpInput(C.Structure):
     """struct b2r_mlp_input (include/b2r.h)."""
     _fields_ = [("rays", C.c_void_p), ("z", C.c_void_p), ("x", C.c_void_p), ("n_rays", c_ll),
-                ("n_samples", C.c_int), ("grid_n", C.c_int), ("grid_begin", c_ll)]
+                ("n_samples", C.c_int), ("grid_n", C.c_int), ("grid_begin", c_ll), ("lattice_dims", C.c_int * 3),
+                ("lattice_origin", C.c_float * 3), ("lattice_voxel", C.c_float)]
 
 
 class LastSample(C.Structure):
@@ -85,6 +86,7 @@ SIGNATURES = {
     "b2r_mc_count": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b2r_mc_emit": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                               C.c_void_p, c_float_p, C.c_void_p, C.c_void_p]),
+    "b2r_mc_normals": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, c_float_p, C.c_void_p]),
 }
 
 _lock = threading.Lock()

@@ -88,9 +88,12 @@ struct RowSource {
     const float* x;
     long long n_rays;
     int n_samples;
-    int grid_n;
-    long long grid_begin;
-    float voxel;   // 0.2/(N-1) rounded to float (pi_GAN/utils.py:57)
+    // lattice rows: row r is lattice index lat_begin + r (axis 0 slowest) of the N^3 pi-GAN cube (grid_n > 0: origin -0.1) or of
+    // the n0 x n1 x n2 box lattice at lat_origin
+    long long lat_begin;
+    int grid_n, lat_n1, lat_n2;
+    float lat_origin[3];
+    float voxel;
     // gather mode (b2r_mlp_f32_last_sigma): row i of the launch is the LAST sample of ray pick[i], i.e. source row
     // pick[i] * pick_s + pick_s - 1 of the rays / x description above
     const int* pick;
@@ -98,12 +101,22 @@ struct RowSource {
 };
 
 inline RowSource make_row_source(const b2r_mlp_input* in) {
-    RowSource s;
+    RowSource s = {};
     s.rays = in->rays; s.z = in->z; s.x = in->x; s.n_rays = in->n_rays; s.n_samples = in->n_samples;
-    s.grid_n = in->grid_n; s.grid_begin = in->grid_begin;
-    s.voxel = in->grid_n > 1 ? (float)(0.2 / (double)(in->grid_n - 1)) : 0.f;
+    s.lat_begin = in->grid_begin;
+    s.grid_n = in->grid_n;
+    if (in->grid_n > 0) {
+        s.voxel = in->grid_n > 1 ? (float)(0.2 / (double)(in->grid_n - 1)) : 0.f;   // 0.2/(N-1) rounded to float (pi_GAN/utils.py:57)
+    } else {
+        s.lat_n1 = in->lattice_dims[1]; s.lat_n2 = in->lattice_dims[2];
+        for (int c = 0; c < 3; ++c) s.lat_origin[c] = in->lattice_origin[c];
+        s.voxel = in->lattice_voxel;
+    }
     s.pick = nullptr; s.pick_s = 0;
     return s;
+}
+inline bool lattice_mode(const b2r_mlp_input* in) {
+    return in->lattice_dims[0] != 0 || in->lattice_dims[1] != 0 || in->lattice_dims[2] != 0;
 }
 inline long long row_count(const b2r_mlp_input* in) {
     return in->rays ? in->n_rays * (long long)in->n_samples : in->n_rays;
@@ -111,8 +124,13 @@ inline long long row_count(const b2r_mlp_input* in) {
 int check_mlp_input(const b2r_mlp_input* in);
 
 // position = o + d*z as two rounded ops (torch: mul then add, nerf/render.py:134), unit view
-// direction = d/|d| (render.py:122), lattice coordinates as pi_GAN/utils.py:64-72.
+// direction = d/|d| (render.py:122), lattice point = origin + index * voxel as two rounded ops (pi_GAN/utils.py:64-72).
 // ray_out (optional): the ray the row belongs to (rays mode; the row itself otherwise).
+// The pi-GAN cube keeps its own branch: its N^3 may pass 2^32 and needs 64-bit index arithmetic, while the box lattice has at most
+// INT32_MAX points and uses 32-bit; one 64-bit path with per-axis divisors and origins costs the register-capped tensor-core
+// kernels spills.  kBoxLattice = false compiles the box branch out: the tensor-core kernels have an instantiation for box-lattice
+// rows and one for every other mode, so the other modes run the code they ran before the box lattice existed.
+template <bool kBoxLattice = true>
 __device__ __forceinline__ void load_row(const RowSource& s, long long row, float p[3], float v[3], long long* ray_out = nullptr) {
     if (s.pick) row = (long long)s.pick[row] * s.pick_s + (s.pick_s - 1);
     if (ray_out) *ray_out = row;
@@ -131,12 +149,19 @@ __device__ __forceinline__ void load_row(const RowSource& s, long long row, floa
         const float* x = s.x + row * 6;
         p[0] = x[0]; p[1] = x[1]; p[2] = x[2]; v[0] = x[3]; v[1] = x[4]; v[2] = x[5];
     } else {
-        long long idx = s.grid_begin + row;
-        long long n = s.grid_n;
-        float iz = (float)(idx % n), iy = (float)((idx / n) % n), ix = (float)((idx / n / n) % n);
-        p[0] = __fadd_rn(__fmul_rn(ix, s.voxel), -0.1f);
-        p[1] = __fadd_rn(__fmul_rn(iy, s.voxel), -0.1f);
-        p[2] = __fadd_rn(__fmul_rn(iz, s.voxel), -0.1f);
+        if (!kBoxLattice || s.grid_n) {
+            const long long idx = s.lat_begin + row, n = s.grid_n;
+            float iz = (float)(idx % n), iy = (float)((idx / n) % n), ix = (float)((idx / n / n) % n);
+            p[0] = __fadd_rn(__fmul_rn(ix, s.voxel), -0.1f);
+            p[1] = __fadd_rn(__fmul_rn(iy, s.voxel), -0.1f);
+            p[2] = __fadd_rn(__fmul_rn(iz, s.voxel), -0.1f);
+        } else {
+            const unsigned idx = (unsigned)(s.lat_begin + row), n1 = (unsigned)s.lat_n1, n2 = (unsigned)s.lat_n2, r = idx / n2;
+            float iz = (float)(idx % n2), iy = (float)(r % n1), ix = (float)(r / n1);
+            p[0] = __fadd_rn(s.lat_origin[0], __fmul_rn(ix, s.voxel));
+            p[1] = __fadd_rn(s.lat_origin[1], __fmul_rn(iy, s.voxel));
+            p[2] = __fadd_rn(s.lat_origin[2], __fmul_rn(iz, s.voxel));
+        }
         v[0] = v[1] = v[2] = 0.f;
     }
 }

@@ -9,6 +9,8 @@
 //   mc_scan_kernel      exclusive scan of the tile counts (one CTA) + the totals (V, F)
 //   mc_vertices_kernel  reads the words, and the field at crossing points only; writes the vertices
 //   mc_faces_kernel     reads the words of the cell corners; writes the triangles
+//   mc_normals_kernel   (optional, b2r_mc_normals) like mc_vertices_kernel; reads the field around both ends of every crossing
+//                       edge and writes the unit vertex normals in vertex order
 // HBM traffic: 4 B (field) + 4 B (word) written, 4 B read twice, plus the field at the crossing points and the output.
 // Every vertex component is formed with separately rounded operations (no FMA), so numpy float32 reproduces it bit for bit.
 #include "common.cuh"
@@ -194,6 +196,54 @@ __global__ void __launch_bounds__(kThreads) mc_vertices_kernel(const float* __re
     }
 }
 
+// Component of the field's gradient along one axis at lattice coordinate c of n (np.gradient's scheme with the isotropic spacing
+// dropped): central difference inside, one-sided on the faces.  step = the axis' linear-index stride.
+__device__ __forceinline__ float grad_axis(const float* __restrict__ f, unsigned idx, unsigned c, unsigned n, unsigned step) {
+    if (c == 0) return __fsub_rn(f[idx + step], f[idx]);
+    if (c + 1 == n) return __fsub_rn(f[idx], f[idx - step]);
+    return __fmul_rn(0.5f, __fsub_rn(f[idx + step], f[idx - step]));
+}
+
+// The normal of the vertex on the edge p -> p + e_a is g(p) + t (g(p + e_a) - g(p)) with the vertex's own t, divided by its length;
+// it points toward increasing field (the side the triangle normals face).  Zero length gives (0, 0, 0).
+__global__ void __launch_bounds__(kThreads) mc_normals_kernel(const float* __restrict__ f, int n0, int n1, int n2, float level,
+                                                              const unsigned* __restrict__ words,
+                                                              const longlong2* __restrict__ offsets, float* __restrict__ normals) {
+    const unsigned n = (unsigned)n0 * n1 * n2, s1 = (unsigned)n2, s0 = (unsigned)n1 * n2;
+    const unsigned base = blockIdx.x * (unsigned)kTile;
+    const long long tile_v = offsets[blockIdx.x].x;
+#pragma unroll 1
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned idx = base + q * kThreads + threadIdx.x;
+        if (idx >= n) break;
+        const unsigned w = words[idx];
+        if (!(w & 7u)) continue;
+        const unsigned k = idx % s1, r = idx / s1, j = r % (unsigned)n1, i = r / (unsigned)n1;
+        const float f0 = f[idx];
+        const unsigned p[3] = {i, j, k}, dims[3] = {(unsigned)n0, (unsigned)n1, (unsigned)n2}, step[3] = {s0, s1, 1u};
+        float g0[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) g0[c] = grad_axis(f, idx, p[c], dims[c], step[c]);
+        float* out = normals + 3 * (tile_v + (w >> kVertShift));
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            if (!(w >> a & 1u)) continue;
+            const unsigned at = idx + step[a];
+            const float t = __fdiv_rn(__fsub_rn(level, f0), __fsub_rn(f[at], f0));
+            float g[3];
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const float g1 = grad_axis(f, at, c == a ? p[c] + 1 : p[c], dims[c], step[c]);
+                g[c] = __fadd_rn(g0[c], __fmul_rn(t, __fsub_rn(g1, g0[c])));
+            }
+            const float len = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(g[0], g[0]), __fmul_rn(g[1], g[1])), __fmul_rn(g[2], g[2])));
+#pragma unroll
+            for (int c = 0; c < 3; ++c) out[c] = len > 0.f ? __fdiv_rn(g[c], len) : 0.f;
+            out += 3;
+        }
+    }
+}
+
 __global__ void __launch_bounds__(kThreads) mc_faces_kernel(int n0, int n1, int n2, const unsigned* __restrict__ words,
                                                             const longlong2* __restrict__ offsets, int* __restrict__ faces) {
     __shared__ uint64_t s_tri[256];
@@ -275,5 +325,21 @@ extern "C" int b2r_mc_emit(const float* field, int n0, int n1, int n2, float lev
     mc_vertices_kernel<<<tiles, kThreads, 0, st>>>(field, n0, n1, n2, level, spacing, ox, oy, oz, words, offsets, verts);
     mc_faces_kernel<<<tiles, kThreads, 0, st>>>(n0, n1, n2, words, offsets, faces);
     B2R_LAUNCH_CHECK("b2r_mc_emit");
+    return 0;
+}
+
+extern "C" int b2r_mc_normals(const float* field, int n0, int n1, int n2, float level, const void* scratch, float* normals,
+                              void* stream) {
+    using namespace b2r::mc;
+    if (int rc = check_grid("b2r_mc_normals", n0, n1, n2)) return rc;
+    B2R_CHECK_ARG(field && scratch && normals, "b2r_mc_normals: NULL pointer");
+    B2R_CHECK_ARG(((uintptr_t)scratch & 15) == 0, "b2r_mc_normals: scratch must be 16-byte aligned");
+    const long long n = (long long)n0 * n1 * n2;
+    const Layout l = layout(n);
+    const int tiles = (int)((n + kTile - 1) / kTile);
+    const char* s = static_cast<const char*>(scratch);
+    mc_normals_kernel<<<tiles, kThreads, 0, (cudaStream_t)stream>>>(field, n0, n1, n2, level, (const unsigned*)(s + l.words),
+                                                                    (const longlong2*)(s + l.offsets), normals);
+    B2R_LAUNCH_CHECK("b2r_mc_normals");
     return 0;
 }

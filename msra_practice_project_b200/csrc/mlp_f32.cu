@@ -517,7 +517,7 @@ extern "C" int b2r_mlp_f32_last_sigma(int model_kind, const float* params, const
     B2R_CHECK_ARG(params && raw_io && workspace && ray_ids, "b2r_mlp_f32_last_sigma: NULL pointer");
     B2R_CHECK_ARG(model_kind != B2R_MODEL_FILM || film, "b2r_mlp_f32_last_sigma: FiLM model needs film params");
     B2R_TRY(check_mlp_input(in));
-    B2R_CHECK_ARG(in->grid_n == 0, "b2r_mlp_f32_last_sigma: rays / x rows only");
+    B2R_CHECK_ARG(in->grid_n == 0 && !lattice_mode(in), "b2r_mlp_f32_last_sigma: rays / x rows only");
     B2R_CHECK_ARG(samples_per_ray >= 1 && (!in->rays || samples_per_ray == in->n_samples), "b2r_mlp_f32_last_sigma: samples_per_ray (%d) must equal n_samples in rays mode", samples_per_ray);
     B2R_CHECK_ARG(n_ids >= 0 && n_latents >= 1 && (n_latents == 1 || rows_per_latent > 0), "b2r_mlp_f32_last_sigma: bad n_ids / n_latents / rows_per_latent");
     const size_t lat_bytes = ((size_t)n_ids * 4 + 15) & ~(size_t)15;

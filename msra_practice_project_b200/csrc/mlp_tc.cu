@@ -256,7 +256,7 @@ __device__ __forceinline__ void nerf_epi(uint32_t t_half, uint32_t bias_half, ui
 // kSigmaOnly (inference): the walk stops after layers_pos.7 + the sigma head (steps 0..7); raw = (0, 0, 0, relu sigma).  For passes
 // whose colour nobody reads -- the coarse pass of render_image, which returns the fine maps only (nerf/render.py:150-167) and needs
 // the coarse weights, a function of sigma alone, for sample_pdf: sigma is bit-identical to the full walk's (same MMAs, same epilogue).
-template <bool kSave, bool kSigmaOnly = false>
+template <bool kSave, bool kSigmaOnly = false, bool kBox = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 nerf_tc_kernel(const uint8_t* __restrict__ packed, RowSource src, long long rows, float4* __restrict__ raw_out, uint8_t* __restrict__ saved,
                LastFlag lf) {
@@ -340,7 +340,7 @@ nerf_tc_kernel(const uint8_t* __restrict__ packed, RowSource src, long long rows
             };
             float pnt[3], vdir[3];
             long long ray = 0;
-            load_row(src, valid ? row : rows - 1, pnt, vdir, &ray);
+            load_row<kBox>(src, valid ? row : rows - 1, pnt, vdir, &ray);
             const bool check_last = valid && last_of_ray(lf, src, row, ray);      // this row decides its ray's last interval
             const bool warp_checks = __any_sync(0xffffffffu, check_last);
             float asum = 0.f;
@@ -531,7 +531,7 @@ __device__ __forceinline__ void film_epi(uint32_t t_q, uint32_t head, uint32_t h
 // (rows_per_latent is a multiple of the 512 rows of a CTA pair, which shares one set of weights); the producer streams the tile's latent's weights and the epilogue
 // warps reload the small fp32 tables when their next tile is another latent's.
 // kSave = training forward (one latent): tiles + cosine checkpoints for the reverse mode, as in siren_tc_kernel<true>.
-template <bool kSave>
+template <bool kSave, bool kBox = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 film_tc_kernel(const uint8_t* __restrict__ packed, RowSource src, long long rows, int sigma_only, float4* __restrict__ raw_out,
                int n_latents, long long rows_per_latent, uint8_t* __restrict__ saved, LastFlag lf) {
@@ -656,7 +656,7 @@ film_tc_kernel(const uint8_t* __restrict__ packed, RowSource src, long long rows
                 valid[g] = row[g] < rows;
                 float pnt[3], vdir[3];
                 long long ray_ll = 0;
-                load_row(src, valid[g] ? row[g] : rows - 1, pnt, vdir, &ray_ll);
+                load_row<kBox>(src, valid[g] ? row[g] : rows - 1, pnt, vdir, &ray_ll);
                 chk[g] = valid[g] && last_of_ray(lf, src, row[g], ray_ll);
                 ray[g] = (int)ray_ll;
                 if (!first_tile) spill_wait(g);                      // previous tile's last copy
@@ -845,7 +845,7 @@ namespace tc {
 int check_last_sample(const b2r_last_sample* last, const b2r_mlp_input* in, const char* who) {
     if (!last) return 0;
     B2R_CHECK_ARG(last->count && last->ray_ids && last->capacity >= 0, "%s: last-sample check needs count / ray_ids", who);
-    B2R_CHECK_ARG(in->grid_n == 0, "%s: the last-sample check is for rays / x rows, not grid queries", who);
+    B2R_CHECK_ARG(in->grid_n == 0 && !lattice_mode(in), "%s: the last-sample check is for rays / x rows, not grid queries", who);
     B2R_CHECK_ARG(last->samples_per_ray >= 1 && (!in->rays || last->samples_per_ray == in->n_samples),
                   "%s: samples_per_ray (%d) must equal n_samples in rays mode", who, last->samples_per_ray);
     B2R_CHECK_ARG(last->rel >= 0.f && last->abs >= 0.f, "%s: negative last-sample thresholds", who);
@@ -872,13 +872,17 @@ extern "C" int b2r_mlp_tc_fwd(int model_kind, const void* packed, int use_dir, c
     rc = tc::pair_grid(rows, &grid);
     if (rc) return rc;
     cudaStream_t st = (cudaStream_t)stream;
+    // box-lattice rows run their own instantiations, so the index arithmetic they need costs the other modes nothing
+    const bool box = lattice_mode(in);
     if (model_kind == B2R_MODEL_FILM) {
-        rc = cuda_result(cudaFuncSetAttribute(tc::film_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::MapC::kSmem), "tc smem attribute");
+        auto kern = box ? tc::film_tc_kernel<false, true> : tc::film_tc_kernel<false>;
+        rc = cuda_result(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::MapC::kSmem), "tc smem attribute");
         if (rc) return rc;
-        tc::film_tc_kernel<false><<<grid, tc::kThreads, tc::MapC::kSmem, st>>>((const uint8_t*)packed, make_row_source(in), rows, sigma_only, (float4*)raw_out, 1, 0, nullptr,
-                                                                              tc::make_last_flag(last));
+        kern<<<grid, tc::kThreads, tc::MapC::kSmem, st>>>((const uint8_t*)packed, make_row_source(in), rows, sigma_only, (float4*)raw_out, 1, 0, nullptr,
+                                                          tc::make_last_flag(last));
     } else {
-        auto kern = sigma_only ? tc::nerf_tc_kernel<false, true> : tc::nerf_tc_kernel<false, false>;
+        auto kern = box ? (sigma_only ? tc::nerf_tc_kernel<false, true, true> : tc::nerf_tc_kernel<false, false, true>)
+                        : (sigma_only ? tc::nerf_tc_kernel<false, true> : tc::nerf_tc_kernel<false, false>);
         rc = cuda_result(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tc::kSmemBytes), "tc smem attribute");
         if (rc) return rc;
         kern<<<grid, tc::kThreads, tc::kSmemBytes, st>>>((const uint8_t*)packed, make_row_source(in), rows, (float4*)raw_out, nullptr, tc::make_last_flag(last));
@@ -908,6 +912,7 @@ extern "C" int b2r_mlp_tc_fwd_film_batched(const void* packed, int n_latents, lo
     int rc = check_mlp_input(in);
     if (rc) return rc;
     long long rows = row_count(in);
+    B2R_CHECK_ARG(!lattice_mode(in), "b2r_mlp_tc_fwd_film_batched: box-lattice rows go to b2r_mlp_tc_fwd");
     // a CTA pair (2 x 256 rows) shares one set of weights: both of its tiles must belong to the same latent
     B2R_CHECK_ARG(rows_per_latent > 0 && rows_per_latent % (2 * tc::kRowsTile) == 0,
                   "b2r_mlp_tc_fwd_film_batched: rows_per_latent (%lld) must be a positive multiple of %d", rows_per_latent, 2 * tc::kRowsTile);
@@ -936,6 +941,7 @@ extern "C" int b2r_mlp_tc_train_fwd_film_batched(const void* packed, int n_laten
     int rc = check_mlp_input(in);
     if (rc) return rc;
     long long rows = row_count(in);
+    B2R_CHECK_ARG(!lattice_mode(in), "b2r_mlp_tc_train_fwd_film_batched: box-lattice rows are for inference");
     B2R_CHECK_ARG(rows_per_latent > 0 && rows_per_latent % (2 * tc::kRowsTile) == 0,
                   "b2r_mlp_tc_train_fwd_film_batched: rows_per_latent (%lld) must be a positive multiple of %d", rows_per_latent, 2 * tc::kRowsTile);
     B2R_CHECK_ARG(n_latents >= 1 && rows <= rows_per_latent * (long long)n_latents, "b2r_mlp_tc_train_fwd_film_batched: %lld rows need more than %d latents", rows, n_latents);
@@ -972,6 +978,7 @@ extern "C" int b2r_mlp_tc_train_fwd(int model_kind, const void* packed, const b2
     int rc = check_mlp_input(in);
     if (rc) return rc;
     long long rows = row_count(in);
+    B2R_CHECK_ARG(!lattice_mode(in), "b2r_mlp_tc_train_fwd: box-lattice rows are for inference");
     B2R_CHECK_ARG(saved_bytes >= b2r_mlp_tc_train_saved_bytes(model_kind, rows), "b2r_mlp_tc_train_fwd: saved buffer too small (%zu B)", saved_bytes);
     if (rows == 0) return 0;
     rc = tc::check_last_sample(last, in, "b2r_mlp_tc_train_fwd");

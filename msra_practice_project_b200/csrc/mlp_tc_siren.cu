@@ -149,7 +149,7 @@ __device__ __forceinline__ void siren_epi(uint32_t t_q, uint32_t head, uint32_t 
 // kSave = training forward: the layer inputs (aux, h0..h7, layers_dir.0 output, h_d) leave shared memory as tiled bf16 tensors
 // through the bulk-copy engine (warps 2 / 3: one spill thread per sub-tile, as in nerf_tc_kernel<true>) and cos(t) of every
 // sine layer is stored thread-major for the reverse mode (mlp_tc_train.cu).
-template <bool kSave>
+template <bool kSave, bool kBox = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads, 1)
 siren_tc_kernel(const uint8_t* __restrict__ packed, RowSource src, long long rows, float4* __restrict__ raw_out, uint8_t* __restrict__ saved,
                 LastFlag lf) {
@@ -255,7 +255,7 @@ siren_tc_kernel(const uint8_t* __restrict__ packed, RowSource src, long long row
                 valid[g] = row[g] < rows;
                 float pnt[3], vdir[3];
                 long long ray_ll = 0;
-                load_row(src, valid[g] ? row[g] : rows - 1, pnt, vdir, &ray_ll);
+                load_row<kBox>(src, valid[g] ? row[g] : rows - 1, pnt, vdir, &ray_ll);
                 chk[g] = valid[g] && last_of_ray(lf, src, row[g], ray_ll);
                 ray[g] = (int)ray_ll;
                 if (!first_tile) spill_wait(g);                      // previous tile's h_d copy
@@ -393,9 +393,10 @@ int siren_fwd(const void* packed, const b2r_mlp_input* in, long long rows, float
     unsigned grid = 0;
     int rc = pair_grid(rows, &grid);
     if (rc) return rc;
-    rc = cuda_result(cudaFuncSetAttribute(siren_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MapC::kSmem), "tc smem attribute");
+    auto kern = lattice_mode(in) ? siren_tc_kernel<false, true> : siren_tc_kernel<false>;      // box-lattice rows: own instantiation
+    rc = cuda_result(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)MapC::kSmem), "tc smem attribute");
     if (rc) return rc;
-    siren_tc_kernel<false><<<grid, kThreads, MapC::kSmem, st>>>((const uint8_t*)packed, make_row_source(in), rows, (float4*)raw_out, nullptr, make_last_flag(last));
+    kern<<<grid, kThreads, MapC::kSmem, st>>>((const uint8_t*)packed, make_row_source(in), rows, (float4*)raw_out, nullptr, make_last_flag(last));
     B2R_LAUNCH_CHECK("b2r_mlp_tc_fwd (SirenNeRF)");
     return 0;
 }

@@ -20,7 +20,7 @@ import numpy as np
 import torch
 from tqdm import tqdm
 
-from . import ops
+from . import mesh, ops
 
 __all__ = ["np", "torch", "tqdm", "to8b", "get_rays", "sample_pdf", "run_network", "raw_to_outputs", "render_rays",
            "render_image", "render_video", "render_video_u8"]
@@ -288,3 +288,33 @@ def render_video_u8(width, height, focal, poses, near, far, coarse_model, fine_m
             events[slot].synchronize()
             out[pending[slot]] = pinned[slot].numpy()
     return out
+
+
+def density_lattice(model, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), N=256, *, max_batch=256 ** 3, precision=None):
+    """Density of ``model`` (NeRF or SirenNeRF) on the box lattice of [box_min, box_max] with ``N`` points along the longest
+    edge (mesh.box_lattice): ``(sigma [n0,n1,n2] on the device, origin, voxel)``, axis 0 slowest.  The points are made on the
+    device from the lattice index with zero view direction; the bf16 NeRF path stops after the sigma head.  ``max_batch``
+    bounds the points per launch."""
+    dev = _model_device(model)
+    if dev.type != "cuda":
+        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    dims, origin, voxel = mesh.box_lattice(box_min, box_max, N)
+    total = dims[0] * dims[1] * dims[2]
+    sigma = torch.empty((total,), dtype=torch.float32, device=dev)
+    with torch.no_grad():
+        for b in range(0, total, int(max_batch)):
+            c = min(int(max_batch), total - b)
+            sigma[b:b + c] = ops.mlp(model, lattice=(dims, origin, voxel, b, c), precision=precision, sigma_only=True)[:, 3]
+    return sigma.reshape(dims), origin, voxel
+
+
+def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), threshold=50.0,
+                normals=True, colors=True, precision=None, max_batch=256 ** 3):
+    """Mesh of a trained NeRF / SirenNeRF field on the device: the level set ``sigma = threshold`` of ``density_lattice``
+    (marching cubes on -sigma at -threshold, so triangle and vertex normals point out of the object, toward lower density),
+    the unit vertex normals, and the uint8 colour the model's rgb head gives each vertex seen by a camera looking along the
+    inward normal (rows x = [vertex, -normal]).  Returns ``(verts [V,3] float32, faces [F,3] int32, normals [V,3] | None,
+    colors [V,3] uint8 | None)`` on the device; with ``ply_filename`` also writes them as a binary PLY.  Synchronises with the
+    host once to size the mesh.  The default box and threshold fit the Blender scenes (camera radius 4, near 2, far 6)."""
+    sigma, origin, voxel = density_lattice(model, box_min, box_max, N, max_batch=max_batch, precision=precision)
+    return mesh.export(model, sigma.neg_(), -float(threshold), voxel, origin, ply_filename, normals, colors, precision)

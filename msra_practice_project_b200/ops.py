@@ -397,9 +397,15 @@ def _packed_weights(model, kind: int, flat: torch.Tensor, film: torch.Tensor | N
     return packed
 
 
-def _make_input(rays, z, x, grid):
+def _make_input(rays, z, x, grid, lattice=None):
     """(MlpInput, rows, tensors to keep alive)"""
     inp = MlpInput()
+    if lattice is not None:
+        dims, origin, voxel, begin, count = lattice
+        inp.lattice_dims[:] = [int(d) for d in dims]
+        inp.lattice_origin[:] = [float(o) for o in origin]
+        inp.lattice_voxel, inp.grid_begin, inp.n_rays, inp.n_samples = float(voxel), int(begin), int(count), 1
+        return inp, int(count), ()
     if rays is not None:
         rays = _cuda_f32(rays, "rays")
         z = _cuda_f32(z, "z_vals")
@@ -677,10 +683,13 @@ def mlp_film_batched_train(model, film: torch.Tensor, rays: torch.Tensor, z: tor
 
 def mlp(model, rays: torch.Tensor | None = None, z: torch.Tensor | None = None, x: torch.Tensor | None = None,
         grid: tuple | None = None, precision: str | None = None, sigma_only: bool = False,
-        exact_last_sample: bool | None = None, samples_per_ray: int | None = None) -> torch.Tensor:
-    """Evaluate the radiance field on rows described by (rays, z) | x | grid -> raw[rows,4]
+        exact_last_sample: bool | None = None, samples_per_ray: int | None = None, lattice: tuple | None = None) -> torch.Tensor:
+    """Evaluate the radiance field on rows described by (rays, z) | x | grid | lattice -> raw[rows,4]
     (run_network + network.forward, nerf/render.py:59-75).  Differentiable wrt the model's
     parameters (and FiLM parameters) when any of them requires grad and grad mode is on.
+    ``grid = (N, begin, count)``: indices [begin, begin+count) of the N^3 lattice of [-0.1,0.1]^3 (pi-GAN's create_mesh);
+    ``lattice = ((n0, n1, n2), (ox, oy, oz), voxel, begin, count)``: indices of a box lattice, point origin + index * voxel in
+    fp32 (axis 0 slowest).  Both have zero view direction and are inference-only.
 
     bf16 inference on ray samples -- (rays, z), or x with ``samples_per_ray`` given -- also runs the last-sample sign check
     (see _EXACT_LAST above) unless ``exact_last_sample`` is False."""
@@ -704,14 +713,14 @@ def mlp(model, rays: torch.Tensor | None = None, z: torch.Tensor | None = None, 
     flat = models.flat_params(net, kind) if needs_grad else torch.cat([p.detach().reshape(-1) for p in ps]).float()
     precision = precision or _MLP_PRECISION
     if needs_grad:
-        if grid is not None:
-            raise RuntimeError("grid queries are inference-only")
+        if grid is not None or lattice is not None:
+            raise RuntimeError("grid / lattice queries are inference-only")
         if _GRAD_PRECISION == "bf16":
             if kind == models.KIND_FILM:
                 return _MlpTcTrainFilm.apply(flat, film, rays, z, x, 0, use_dir)
             return _MlpTcTrain.apply(flat, net, kind, rays, z, x)
         return _MlpF32.apply(flat, film, kind, use_dir, rays, z, x, 1 if _GRAD_PRECISION == "tf32" else 0)
-    inp, rows, keep = _make_input(rays, z, x, grid)
+    inp, rows, keep = _make_input(rays, z, x, grid, lattice)
     raw = torch.empty((rows, 4), dtype=torch.float32, device=dev)
     if rows == 0:
         return raw
@@ -789,12 +798,14 @@ def to8b(x: torch.Tensor) -> torch.Tensor:
 _INT32_MAX = 2 ** 31 - 1
 
 
-def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, origin=(0.0, 0.0, 0.0)):
+def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, origin=(0.0, 0.0, 0.0), *, normals: bool = False):
     """Marching cubes of ``field`` [n0,n1,n2] (axis 0 slowest) at ``level`` on the device (b2r_mc_count / b2r_mc_emit; the
     table and its rule: oracle/marching_cubes.py).  Returns ``(verts [V,3] float32, faces [F,3] int32)`` on the field's
     device; vertex ``origin + (p + t e_a) * spacing`` lies on the lattice edge from point ``p`` along axis ``a``, and the
     triangle normals point from ``field < level`` to ``field >= level``.  Synchronises once with the host to read the
-    mesh size (V, F), as ``torch.nonzero`` does.  Empty meshes are ``[0,3]`` tensors."""
+    mesh size (V, F), as ``torch.nonzero`` does.  Empty meshes are ``[0,3]`` tensors.
+    ``normals=True`` also returns the unit vertex normals [V,3] (b2r_mc_normals: the field's central-difference gradient
+    interpolated along the vertex's edge, pointing toward increasing field; (0, 0, 0) where it vanishes)."""
     field = _cuda_f32(field, "field")
     if field.dim() != 3 or min(field.shape) < 2:
         raise RuntimeError(f"field must be [n0,n1,n2] with every n >= 2, got {list(field.shape)}")
@@ -816,4 +827,9 @@ def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, orig
         if n_verts and n_faces:
             check(lib().b2r_mc_emit(ptr(field), n0, n1, n2, level, spacing, ox, oy, oz, ptr(scratch), ptr(verts), ptr(faces),
                                     _stream(field)), "b2r_mc_emit")
-    return verts, faces
+        if not normals:
+            return verts, faces
+        nrm = torch.empty((n_verts, 3), dtype=torch.float32, device=dev)
+        if n_verts and n_faces:
+            check(lib().b2r_mc_normals(ptr(field), n0, n1, n2, level, ptr(scratch), ptr(nrm), _stream(field)), "b2r_mc_normals")
+    return verts, faces, nrm

@@ -12,6 +12,7 @@ import torch
 from tqdm import tqdm
 
 from . import ops
+from .mesh import export as _export_mesh, write_ply  # noqa: F401  (pigan_render.write_ply is public)
 from .nerf_render import (REFERENCE_RAY_CHUNK, _draw_t_rand, get_rays, maps_to_numpy, raw_to_outputs, render_image_device, render_rays,
                           run_network, sample_pdf, to8b)
 
@@ -183,32 +184,18 @@ def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=No
     return _sdf_device(generator, N, max_batch, z, precision).cpu(), [-0.1, -0.1, -0.1], 0.2 / (N - 1)
 
 
-def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None):
+def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None, normals=False,
+                colors=False):
     """``create_mesh`` (pi_GAN/utils.py:42-180) on the device: the sdf of ``create_mesh_sdf`` never leaves the GPU,
     ``ops.marching_cubes`` extracts its level set (the reference's skimage call at level -20: below = sigma > 20, so the
     triangle normals point out of the object), and only the mesh crosses to the host.  Returns ``(verts [V,3] float32,
     faces [F,3] int32)`` on the device, in world coordinates (voxel origin -0.1, voxel size 0.2/(N-1)).  With
     ``ply_filename`` the mesh is also written as the binary PLY the reference writes with plyfile (``vertex`` x/y/z f4,
-    ``face`` vertex_indices as a uchar-counted list of i4).  Synchronises with the host once to size the mesh."""
+    ``face`` vertex_indices as a uchar-counted list of i4).  Synchronises with the host once to size the mesh.
+    ``normals`` / ``colors``: also compute the unit vertex normals (out of the object) and the uint8 colours the conditioned
+    generator's rgb head gives each vertex seen along the inward normal; the PLY then carries nx/ny/nz and red/green/blue,
+    and the return value is ``(verts, faces, normals | None, colors | None)``."""
     sdf = _sdf_device(generator, N, max_batch, z, precision)
-    verts, faces = ops.marching_cubes(sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1))
-    if ply_filename is not None:
-        write_ply(ply_filename, verts.cpu().numpy(), faces.cpu().numpy())
-    return verts, faces
-
-
-def write_ply(filename, verts, faces):
-    """Binary little-endian PLY of a triangle mesh, byte for byte what plyfile writes for the reference's elements
-    (pi_GAN/utils.py:158-180): ``vertex`` with float x/y/z, ``face`` with ``property list uchar int vertex_indices``."""
-    verts = np.ascontiguousarray(verts, dtype="<f4").reshape(-1, 3)
-    faces = np.asarray(faces).reshape(-1, 3)
-    body = np.empty(len(faces), dtype=[("n", "u1"), ("vertex_indices", "<i4", (3,))])
-    body["n"] = 3
-    body["vertex_indices"] = faces
-    header = ("ply\nformat binary_little_endian 1.0\n"
-              f"element vertex {len(verts)}\nproperty float x\nproperty float y\nproperty float z\n"
-              f"element face {len(faces)}\nproperty list uchar int vertex_indices\nend_header\n")
-    with open(filename, "wb") as fh:
-        fh.write(header.encode("ascii"))
-        verts.view([("x", "<f4"), ("y", "<f4"), ("z", "<f4")]).reshape(-1).tofile(fh)
-        body.tofile(fh)
+    out = _export_mesh(generator.film_siren_nerf, sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1), ply_filename, normals, colors,
+                       precision)
+    return out if (normals or colors) else out[:2]

@@ -3,7 +3,13 @@ marching cubes (b2r_mc_count + b2r_mc_emit, device events, median of 20 after wa
 calls timed on its own), the mesh's size and bytes moved, and the mesh D2H + PLY write.  Prints the card and its power limit
 and one JSON line.  The field is the sdf of a seeded models.Generator(256, 16) at the reference's level -20; untrained, its
 sigma is 0 on the whole box, so (as in tests/test_gpu_mesh.py) the input layer's frequencies are raised and the sigma head is
-centred and scaled.  The 256^3 field (67 MB) fits in the 126 MB L2, the 512^3 one (537 MB) does not.  Also times the numpy oracle at 128^3 on the host, for scale."""
+centred and scaled.  The 256^3 field (67 MB) fits in the 126 MB L2, the 512^3 one (537 MB) does not.  Also times the numpy oracle at 128^3 on the host, for scale.
+
+The NeRF lines time nerf_render.create_mesh stage by stage on the default box [-1.5, 1.5]^3 of a seeded models.NeRF whose sigma
+head is scaled by 100 with a zeroed bias (the threshold is the 70th percentile of its sigma): the box-lattice density query
+(bf16 sigma-only kernel) in ms and points/s, marching cubes, the vertex normals (b2r_mc_normals), the colour query at
+x = [vertex, -normal] with to8b, the D2H copy + PLY write with normals and colours, and one whole create_mesh call that writes the
+coloured PLY."""
 import json
 import os
 import statistics
@@ -16,7 +22,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
-from msra_practice_project_b200 import models, ops, pigan_render  # noqa: E402
+from msra_practice_project_b200 import mesh, models, nerf_render, ops, pigan_render  # noqa: E402
 from msra_practice_project_b200._lib import check, lib, ptr  # noqa: E402
 from oracle import marching_cubes as mc  # noqa: E402
 
@@ -80,6 +86,72 @@ def mc_bytes(n0, n1, n2, nv, nf):
     return 16 * n + 8 * nv + 12 * nv + 12 * nf + tiles * (4 + 4 + 16 + 16 + 16)
 
 
+def _timed(fn, reps):
+    """(median device ms over reps after one warm-up, last result) of fn() between two events."""
+    ts, res = [], None
+    for i in range(reps + 1):
+        a, b = _events()
+        a.record()
+        res = fn()
+        b.record()
+        torch.cuda.synchronize()
+        if i:
+            ts.append(a.elapsed_time(b))
+    return statistics.median(ts), res
+
+
+NERF_TRUNK_FLOP = 2 * (60 * 256 + 4 * 256 * 256 + 316 * 256 + 2 * 256 * 256 + 256)    # 8-layer trunk + sigma head, per point
+
+
+def nerf_lines():
+    torch.manual_seed(0)
+    net = models.NeRF().cuda()
+    with torch.no_grad():
+        net.output_layer_sigma.weight.mul_(100.0)
+        net.output_layer_sigma.bias.zero_()
+    res = {}
+    for n in (256, 512):
+        q_ms, (sigma, origin, voxel) = _timed(lambda: nerf_render.density_lattice(net, N=n), 3)
+        pts = sigma.numel()
+        thr = float(torch.quantile(sigma.flatten()[::97].float(), 0.7))
+        field = -sigma
+        dev_ms, host_ms, verts, faces = mc_times(field, -thr, voxel, origin)
+        n0, n1, n2 = field.shape
+        scratch = torch.empty((lib().b2r_mc_scratch_bytes(n0, n1, n2),), dtype=torch.uint8, device=field.device)
+        totals = torch.empty((2,), dtype=torch.int64, device=field.device)
+        st = torch.cuda.current_stream().cuda_stream
+        check(lib().b2r_mc_count(ptr(field), n0, n1, n2, -thr, ptr(scratch), ptr(totals), st), "b2r_mc_count")
+        nrm = torch.empty_like(verts)
+        nrm_ms, _ = _timed(lambda: check(lib().b2r_mc_normals(ptr(field), n0, n1, n2, -thr, ptr(scratch), ptr(nrm), st), "b2r_mc_normals"),
+                           REPS)
+        col_ms, rgb = _timed(lambda: mesh.vertex_colors(net, verts, nrm), 5)
+        with tempfile.TemporaryDirectory() as tmp:
+            path = os.path.join(tmp, "mesh.ply")
+            ts = []
+            for _ in range(2):
+                torch.cuda.synchronize()
+                t0 = time.perf_counter()
+                mesh.write_ply(path, verts.cpu().numpy(), faces.cpu().numpy(), nrm.cpu().numpy(), rgb.cpu().numpy())
+                ts.append((time.perf_counter() - t0) * 1e3)
+            ply_bytes = os.path.getsize(path)
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            whole = nerf_render.create_mesh(net, path, n, threshold=thr)
+            torch.cuda.synchronize()
+            whole_ms = (time.perf_counter() - t0) * 1e3
+        same = bool(torch.equal(whole[0], verts) and torch.equal(whole[1], faces) and torch.equal(whole[2], nrm) and torch.equal(whole[3], rgb))
+        res[str(n)] = {
+            "dims": list(field.shape), "points": pts, "density_query_ms": round(q_ms, 3), "points_per_s": round(pts / (q_ms * 1e-3) / 1e9, 3),
+            "points_per_s_unit": "G/s", "trunk_TFLOPs": round(pts * NERF_TRUNK_FLOP / (q_ms * 1e-3) / 1e12, 1), "threshold": thr,
+            "marching_cubes_device_ms": round(dev_ms, 4), "host_read_VF_ms": round(host_ms, 4), "normals_ms": round(nrm_ms, 4),
+            "color_query_ms": round(col_ms, 3), "V": int(verts.shape[0]), "F": int(faces.shape[0]),
+            "d2h_plus_ply_ms": round(statistics.median(ts), 2), "ply_bytes": ply_bytes, "create_mesh_call_ms": round(whole_ms, 1),
+            "create_mesh_equals_stages": same}
+        del sigma, field, verts, faces, nrm, rgb, whole, scratch
+        torch.cuda.empty_cache()
+    return res
+
+
 def main():
     smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
     print("gpu:", smi.stdout.strip().splitlines()[0] if smi.returncode == 0 and smi.stdout.strip() else "unknown")
@@ -120,6 +192,7 @@ def main():
             "repeat_run_identical": same, "field_fits_l2": n ** 3 * 4 < 126e6}
         del sdf, verts, faces, ref_v, ref_f
         torch.cuda.empty_cache()
+    out["nerf_sizes"] = nerf_lines()
     # the numpy oracle at 128^3, host only, for scale
     sdf = pigan_render.density_grid(gen.film_siren_nerf, N=128).reshape(128, 128, 128).cpu().numpy()
     t0 = time.perf_counter()
