@@ -311,6 +311,28 @@ int b2r_mc_emit(const float* field, int n0, int n1, int n2, float level, float s
  * the triangle normals face.  A zero-length n (a flat field there) gives (0, 0, 0). */
 int b2r_mc_normals(const float* field, int n0, int n1, int n2, float level, const void* scratch, float* normals, void* stream);
 
+/* ---- connected components of a triangle mesh (no reference counterpart: clean-up of exported meshes) ----------------------
+ * faces[F,3] (int32) index verts[V,3]; two vertices are connected when a face has them as (v0,v1) or (v1,v2).  PRECONDITION:
+ * every face index lies in [0, n_verts) (not checked: the indices are in device memory; ops.py checks them first).  Counts are
+ * in [0, INT32_MAX]; faces / labels / verts may be NULL only when their count is 0.  scratch: b2r_mesh_cc_scratch_bytes(V, F)
+ * bytes, 16-byte aligned (0 for counts outside [0, INT32_MAX]).
+ *   b2r_mesh_cc_label:   labels[V] (int32) = the smallest vertex index of each vertex's component (a vertex no face uses is its
+ *                        own component), the same whatever the schedule of the union-find that computes it.
+ *   b2r_mesh_cc_select:  given those labels, marks the vertices and faces of every component with t triangles where t >= 1 and
+ *                        t >= ratio * t_max in float64 (t_max = the largest component's count; ratio finite, in [0, 1]; ratio 0
+ *                        keeps everything) and writes totals_dev[2] = (V', F'), two long long in DEVICE memory.
+ *   b2r_mesh_cc_compact: given the scratch b2r_mesh_cc_select wrote for the same mesh, writes the kept vertices (and normals,
+ *                        when normals_or_null is not NULL) to verts_out[V',3] / normals_out[V',3] and the kept faces, indices
+ *                        remapped to the new vertex order, to faces_out[F',3]; both in their original relative order.  Its
+ *                        output pointers must be valid whenever n_verts / n_faces is not 0, so the caller reads (V', F') first
+ *                        and skips the call when V' = 0 (nothing is kept). */
+size_t b2r_mesh_cc_scratch_bytes(long long n_verts, long long n_faces);
+int b2r_mesh_cc_label(const int* faces, long long n_faces, long long n_verts, int* labels, void* scratch, void* stream);
+int b2r_mesh_cc_select(const int* faces, long long n_faces, long long n_verts, const int* labels, float ratio, void* scratch,
+                       long long* totals_dev, void* stream);
+int b2r_mesh_cc_compact(const float* verts, const float* normals_or_null, const int* faces, long long n_faces, long long n_verts,
+                        const void* scratch, float* verts_out, float* normals_out, int* faces_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

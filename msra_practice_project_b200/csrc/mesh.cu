@@ -13,6 +13,8 @@
 //                       edge and writes the unit vertex normals in vertex order
 // HBM traffic: 4 B (field) + 4 B (word) written, 4 B read twice, plus the field at the crossing points and the output.
 // Every vertex component is formed with separately rounded operations (no FMA), so numpy float32 reproduces it bit for bit.
+#include <cmath>
+
 #include "common.cuh"
 #include "mc_tables.cuh"
 
@@ -278,6 +280,186 @@ __global__ void __launch_bounds__(kThreads) mc_faces_kernel(int n0, int n1, int 
     }
 }
 
+// ---- connected components of a triangle mesh (b2r_mesh_cc_*) ----------------------------------------------------------------
+// Vertices are joined by the edges (v0,v1), (v1,v2) of every face.  Labelling is union-find over the faces, ECL-CC style: a
+// union hooks the larger root under the smaller with atomicCAS, so parent[v] <= v always, the minimum vertex of a component is
+// its only root once every union is done, and the labels (root of each vertex) are the minimum-index labels whatever the
+// schedule.  Selection counts the faces per label (warp-aggregated: faces arrive in lattice order, so one dominant component
+// would otherwise serialise nearly every atomic on one address), takes their integer maximum and marks what is kept.
+// Compaction writes the kept vertices and faces in their relative order, no sort and no atomics.
+//
+// Scratch: a[V] (the parent array while labelling, triangle counts per label while selecting), vword[V] (bit 31 = kept, bits
+// 0..15 = rank of the vertex among the kept ones of its tile), tile counts and offsets as in marching cubes, and the maximum.
+// Tile b covers vertices AND faces [b*kTile, +kTile): its kept-vertex and kept-face counts are the two 16-bit fields
+// mc_scan_kernel expects, so the scan writes (V', F') and every tile's (first vertex, first face).
+struct CcLayout {
+    size_t a, vword, counts, offsets, max, total;
+};
+
+inline long long cc_tiles(long long n_verts, long long n_faces) { return ((n_verts > n_faces ? n_verts : n_faces) + kTile - 1) / kTile; }
+
+inline CcLayout cc_layout(long long n_verts, long long n_faces) {
+    const long long tiles = cc_tiles(n_verts, n_faces);
+    CcLayout l;
+    l.a = 0;
+    l.vword = l.a + align256((size_t)n_verts * 4);
+    l.counts = l.vword + align256((size_t)n_verts * 4);
+    l.offsets = l.counts + align256((size_t)tiles * 4);
+    l.max = l.offsets + align256((size_t)tiles * sizeof(longlong2));
+    l.total = l.max + 256;
+    return l;
+}
+
+constexpr unsigned kKept = 1u << 31;
+
+__global__ void cc_init_kernel(unsigned* __restrict__ parent, unsigned n_verts) {
+    const unsigned v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v < n_verts) parent[v] = v;
+}
+
+// Root of v with path halving.  Other threads hook roots and halve paths at the same time; every store replaces a parent by one
+// of its ancestors, so any value read is an ancestor and the walk ends at the current root.
+__device__ __forceinline__ unsigned cc_find(unsigned* parent, unsigned v) {
+    volatile unsigned* p = parent;
+    unsigned u = p[v];
+    while (u != v) {
+        const unsigned w = p[u];
+        if (w == u) return u;
+        p[v] = w;
+        v = w;
+        u = p[v];
+    }
+    return v;
+}
+
+__device__ __forceinline__ void cc_union(unsigned* parent, unsigned a, unsigned b) {
+    a = cc_find(parent, a);
+    b = cc_find(parent, b);
+    while (a != b) {
+        const unsigned lo = min(a, b), hi = max(a, b);
+        const unsigned old = atomicCAS(parent + hi, hi, lo);
+        if (old == hi) return;
+        a = cc_find(parent, old);      // hi was hooked meanwhile: retry from its new root
+        b = lo;
+    }
+}
+
+__global__ void cc_hook_kernel(const int* __restrict__ faces, unsigned n_faces, unsigned* __restrict__ parent) {
+    const unsigned f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= n_faces) return;
+    const unsigned v0 = (unsigned)faces[3 * (size_t)f], v1 = (unsigned)faces[3 * (size_t)f + 1], v2 = (unsigned)faces[3 * (size_t)f + 2];
+    cc_union(parent, v0, v1);
+    cc_union(parent, v1, v2);
+}
+
+__global__ void cc_labels_kernel(unsigned* __restrict__ parent, unsigned n_verts, int* __restrict__ labels) {
+    const unsigned v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v < n_verts) labels[v] = (int)cc_find(parent, v);
+}
+
+// tri[label of v0] += 1 per face, one atomic per distinct label per warp.
+__global__ void cc_count_kernel(const int* __restrict__ faces, unsigned n_faces, const int* __restrict__ labels,
+                                unsigned* __restrict__ tri) {
+    const unsigned f = blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned l = f < n_faces ? (unsigned)labels[faces[3 * (size_t)f]] : ~0u;
+    const unsigned same = __match_any_sync(kFull, l);
+    if (l != ~0u && (threadIdx.x & (kWarp - 1)) == (unsigned)(__ffs(same) - 1)) atomicAdd(tri + l, (unsigned)__popc(same));
+}
+
+__global__ void __launch_bounds__(kThreads) cc_max_kernel(const unsigned* __restrict__ tri, unsigned n_verts, unsigned* __restrict__ out) {
+    __shared__ unsigned s[kWarps];
+    unsigned m = 0;
+    for (unsigned v = blockIdx.x * kThreads + threadIdx.x; v < n_verts; v += gridDim.x * kThreads) m = max(m, tri[v]);
+    m = __reduce_max_sync(kFull, m);
+    if ((threadIdx.x & (kWarp - 1)) == 0) s[threadIdx.x >> 5] = m;
+    __syncthreads();
+    if (threadIdx.x < kWarp) {
+        m = __reduce_max_sync(kFull, threadIdx.x < kWarps ? s[threadIdx.x] : 0u);
+        if (threadIdx.x == 0) atomicMax(out, m);
+    }
+}
+
+// A component with t triangles is kept iff t > 0 and t >= ratio * t_max in float64 (ratio 0 keeps everything).
+__device__ __forceinline__ unsigned cc_keep(unsigned t, float ratio, unsigned t_max) {
+    return ratio == 0.f || (t > 0 && (double)t >= __dmul_rn((double)ratio, (double)t_max)) ? 1u : 0u;
+}
+
+__global__ void __launch_bounds__(kThreads) cc_mark_kernel(const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
+                                                           const int* __restrict__ labels, const unsigned* __restrict__ tri,
+                                                           const unsigned* __restrict__ t_max_p, float ratio,
+                                                           unsigned* __restrict__ vword, unsigned* __restrict__ tile_counts) {
+    __shared__ unsigned s_scan[kPer * kWarps + 1];
+    const unsigned t_max = *t_max_p;
+    const unsigned base = blockIdx.x * (unsigned)kTile;
+    unsigned cnt[kPer], kept = 0;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned idx = base + q * kThreads + threadIdx.x;
+        const unsigned kv = idx < n_verts ? cc_keep(tri[labels[idx]], ratio, t_max) : 0u;
+        const unsigned kf = idx < n_faces ? cc_keep(tri[labels[faces[3 * (size_t)idx]]], ratio, t_max) : 0u;
+        kept |= kv << q;
+        cnt[q] = kv | kf << 16;
+    }
+    const unsigned total = tile_scan(cnt, s_scan);
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned idx = base + q * kThreads + threadIdx.x;
+        if (idx < n_verts) vword[idx] = (kept >> q & 1u ? kKept : 0u) | (cnt[q] & 0xffffu);
+    }
+    if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
+}
+
+// Kept vertex v goes to offsets[v / kTile].x + its rank; a face is kept iff its first vertex is (its three vertices share one
+// component), and goes to its tile's first face + its rank among the tile's kept faces, with its indices remapped.
+__global__ void __launch_bounds__(kThreads) cc_compact_kernel(const float* __restrict__ verts, const float* __restrict__ normals,
+                                                              const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
+                                                              const unsigned* __restrict__ vword,
+                                                              const longlong2* __restrict__ offsets, float* __restrict__ verts_out,
+                                                              float* __restrict__ normals_out, int* __restrict__ faces_out) {
+    __shared__ unsigned s_scan[kPer * kWarps + 1];
+    const unsigned base = blockIdx.x * (unsigned)kTile;
+    const longlong2 off = offsets[blockIdx.x];
+#pragma unroll 2
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned v = base + q * kThreads + threadIdx.x;
+        if (v >= n_verts) break;
+        const unsigned w = vword[v];
+        if (!(w & kKept)) continue;
+        const size_t to = 3 * (size_t)(off.x + (w & 0xffffu)), from = 3 * (size_t)v;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) verts_out[to + c] = verts[from + c];
+        if (normals) {
+#pragma unroll
+            for (int c = 0; c < 3; ++c) normals_out[to + c] = normals[from + c];
+        }
+    }
+    unsigned cnt[kPer];
+    int tri[kPer][3];
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned f = base + q * kThreads + threadIdx.x;
+        cnt[q] = 0;
+        if (f >= n_faces) continue;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) tri[q][c] = faces[3 * (size_t)f + c];
+        cnt[q] = vword[tri[q][0]] >> 31;
+    }
+    unsigned kept = 0;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) kept |= cnt[q] << q;
+    tile_scan(cnt, s_scan);
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        if (!(kept >> q & 1u)) continue;
+        int* out = faces_out + 3 * (off.y + cnt[q]);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const unsigned u = (unsigned)tri[q][c];
+            out[c] = (int)(offsets[u / kTile].x + (vword[u] & 0xffffu));
+        }
+    }
+}
+
 int check_grid(const char* what, int n0, int n1, int n2) {
     B2R_CHECK_ARG(n0 >= 2 && n1 >= 2 && n2 >= 2, "%s: every axis needs n >= 2 (got %d x %d x %d)", what, n0, n1, n2);
     B2R_CHECK_ARG((long long)n0 * n1 * n2 <= INT32_MAX, "%s: n0*n1*n2 = %lld exceeds INT32_MAX", what, (long long)n0 * n1 * n2);
@@ -341,5 +523,97 @@ extern "C" int b2r_mc_normals(const float* field, int n0, int n1, int n2, float 
     mc_normals_kernel<<<tiles, kThreads, 0, (cudaStream_t)stream>>>(field, n0, n1, n2, level, (const unsigned*)(s + l.words),
                                                                     (const longlong2*)(s + l.offsets), normals);
     B2R_LAUNCH_CHECK("b2r_mc_normals");
+    return 0;
+}
+
+namespace {
+
+int check_counts(const char* what, long long n_faces, long long n_verts) {
+    B2R_CHECK_ARG(n_faces >= 0 && n_faces <= INT32_MAX, "%s: n_faces = %lld must be in [0, INT32_MAX]", what, n_faces);
+    B2R_CHECK_ARG(n_verts >= 0 && n_verts <= INT32_MAX, "%s: n_verts = %lld must be in [0, INT32_MAX]", what, n_verts);
+    return 0;
+}
+
+int check_scratch(const char* what, const void* scratch) {
+    B2R_CHECK_ARG(scratch, "%s: NULL scratch", what);
+    B2R_CHECK_ARG(((uintptr_t)scratch & 15) == 0, "%s: scratch must be 16-byte aligned", what);
+    return 0;
+}
+
+unsigned blocks_of(long long n, int threads) { return (unsigned)((n + threads - 1) / threads); }
+
+constexpr unsigned kMaxBlocks = 8 * 148;      // cc_max_kernel: grid-stride, a few CTAs per SM, one atomic per CTA
+
+}  // namespace
+
+extern "C" size_t b2r_mesh_cc_scratch_bytes(long long n_verts, long long n_faces) {
+    if (n_verts < 0 || n_verts > INT32_MAX || n_faces < 0 || n_faces > INT32_MAX) return 0;
+    return b2r::mc::cc_layout(n_verts, n_faces).total;
+}
+
+extern "C" int b2r_mesh_cc_label(const int* faces, long long n_faces, long long n_verts, int* labels, void* scratch, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_cc_label";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG((faces || !n_faces) && (labels || !n_verts), "%s: NULL pointer (faces and labels may be NULL only when their count is 0)",
+                  what);
+    if (int rc = check_scratch(what, scratch)) return rc;
+    if (!n_verts) return 0;
+    unsigned* parent = (unsigned*)((char*)scratch + cc_layout(n_verts, n_faces).a);
+    cudaStream_t st = (cudaStream_t)stream;
+    cc_init_kernel<<<blocks_of(n_verts, kThreads), kThreads, 0, st>>>(parent, (unsigned)n_verts);
+    if (n_faces) cc_hook_kernel<<<blocks_of(n_faces, kThreads), kThreads, 0, st>>>(faces, (unsigned)n_faces, parent);
+    cc_labels_kernel<<<blocks_of(n_verts, kThreads), kThreads, 0, st>>>(parent, (unsigned)n_verts, labels);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_cc_select(const int* faces, long long n_faces, long long n_verts, const int* labels, float ratio, void* scratch,
+                                  long long* totals_dev, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_cc_select";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG((faces || !n_faces) && (labels || !n_verts) && totals_dev,
+                  "%s: NULL pointer (faces and labels may be NULL only when their count is 0)", what);
+    B2R_CHECK_ARG(std::isfinite(ratio) && ratio >= 0.f && ratio <= 1.f, "%s: ratio = %g must be finite and in [0, 1]", what, (double)ratio);
+    if (int rc = check_scratch(what, scratch)) return rc;
+    const CcLayout l = cc_layout(n_verts, n_faces);
+    const int tiles = (int)cc_tiles(n_verts, n_faces);
+    char* s = static_cast<char*>(scratch);
+    unsigned* tri = (unsigned*)(s + l.a);
+    unsigned* t_max = (unsigned*)(s + l.max);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = b2r::cuda_result(cudaMemsetAsync(tri, 0, (size_t)n_verts * 4, st), what)) return rc;
+    if (int rc = b2r::cuda_result(cudaMemsetAsync(t_max, 0, 4, st), what)) return rc;
+    if (n_faces) cc_count_kernel<<<blocks_of(n_faces, kThreads), kThreads, 0, st>>>(faces, (unsigned)n_faces, labels, tri);
+    if (n_verts) {
+        const unsigned blocks = blocks_of(n_verts, kThreads);
+        cc_max_kernel<<<blocks < kMaxBlocks ? blocks : kMaxBlocks, kThreads, 0, st>>>(tri, (unsigned)n_verts, t_max);
+    }
+    if (tiles)
+        cc_mark_kernel<<<tiles, kThreads, 0, st>>>(faces, (unsigned)n_faces, (unsigned)n_verts, labels, tri, t_max, ratio,
+                                                   (unsigned*)(s + l.vword), (unsigned*)(s + l.counts));
+    mc_scan_kernel<<<1, kScanThreads, 0, st>>>((const unsigned*)(s + l.counts), tiles, (longlong2*)(s + l.offsets), totals_dev);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_cc_compact(const float* verts, const float* normals_or_null, const int* faces, long long n_faces, long long n_verts,
+                                   const void* scratch, float* verts_out, float* normals_out, int* faces_out, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_cc_compact";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG((faces && faces_out) || !n_faces, "%s: NULL faces / faces_out with n_faces > 0", what);
+    B2R_CHECK_ARG((verts && verts_out && (!normals_or_null || normals_out)) || !n_verts,
+                  "%s: NULL verts / verts_out, or normals given and NULL normals_out, with n_verts > 0", what);
+    if (int rc = check_scratch(what, scratch)) return rc;
+    const CcLayout l = cc_layout(n_verts, n_faces);
+    const int tiles = (int)cc_tiles(n_verts, n_faces);
+    if (!tiles) return 0;
+    const char* s = static_cast<const char*>(scratch);
+    cc_compact_kernel<<<tiles, kThreads, 0, (cudaStream_t)stream>>>(verts, normals_or_null, faces, (unsigned)n_faces, (unsigned)n_verts,
+                                                                    (const unsigned*)(s + l.vword), (const longlong2*)(s + l.offsets),
+                                                                    verts_out, normals_out, faces_out);
+    B2R_LAUNCH_CHECK(what);
     return 0;
 }

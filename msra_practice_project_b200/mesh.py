@@ -80,10 +80,15 @@ def write_ply(filename, verts, faces, normals=None, colors=None):
         fbody.tofile(fh)
 
 
-def export(model, field, level, spacing, origin, ply_filename, normals, colors, precision):
+def export(model, field, level, spacing, origin, ply_filename, normals, colors, precision, min_component_ratio=0.0):
     """Extract the level set of ``field`` (vertex normals toward increasing field), colour it with ``model`` and write the PLY.
-    Returns (verts, faces, normals | None, colors | None) on the device."""
+    Returns (verts, faces, normals | None, colors | None) on the device.  A ``min_component_ratio`` above 0 removes the
+    components with fewer triangles than that share of the largest one (ops.filter_components) before the colour query, so
+    dropped vertices cost no MLP rows; it synchronises with the host once more, to size the filtered mesh."""
     verts, faces, nrm = extract(field, level, spacing, origin, normals or colors)
+    if min_component_ratio:
+        # marching-cubes faces index their own vertices, so the index check of ops.filter_components is not needed
+        verts, faces, nrm = ops._filter_components(verts, faces, ops._check_ratio(min_component_ratio), nrm)
     rgb = vertex_colors(model, verts, nrm, precision) if colors else None
     if not normals:
         nrm = None

@@ -309,12 +309,17 @@ def density_lattice(model, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), 
 
 
 def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), threshold=50.0,
-                normals=True, colors=True, precision=None, max_batch=256 ** 3):
+                normals=True, colors=True, precision=None, max_batch=256 ** 3, min_component_ratio=0.0):
     """Mesh of a trained NeRF / SirenNeRF field on the device: the level set ``sigma = threshold`` of ``density_lattice``
     (marching cubes on -sigma at -threshold, so triangle and vertex normals point out of the object, toward lower density),
     the unit vertex normals, and the uint8 colour the model's rgb head gives each vertex seen by a camera looking along the
     inward normal (rows x = [vertex, -normal]).  Returns ``(verts [V,3] float32, faces [F,3] int32, normals [V,3] | None,
     colors [V,3] uint8 | None)`` on the device; with ``ply_filename`` also writes them as a binary PLY.  Synchronises with the
-    host once to size the mesh.  The default box and threshold fit the Blender scenes (camera radius 4, near 2, far 6)."""
+    host once to size the mesh.  The default box and threshold fit the Blender scenes (camera radius 4, near 2, far 6).
+    ``min_component_ratio`` (finite, in [0, 1]) above 0 removes the floaters: every connected component with fewer triangles
+    than that share of the largest component's (ops.filter_components; 1 keeps the largest and any tied with it), before the
+    colour query; the call then synchronises with the host twice, once for the marching-cubes size and once for the filtered
+    size.  0 (the default) keeps every triangle."""
     sigma, origin, voxel = density_lattice(model, box_min, box_max, N, max_batch=max_batch, precision=precision)
-    return mesh.export(model, sigma.neg_(), -float(threshold), voxel, origin, ply_filename, normals, colors, precision)
+    return mesh.export(model, sigma.neg_(), -float(threshold), voxel, origin, ply_filename, normals, colors, precision,
+                       min_component_ratio)

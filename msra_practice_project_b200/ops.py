@@ -8,6 +8,7 @@ tensors and raises otherwise -- there is no CPU or PyTorch-op fallback.
 from __future__ import annotations
 
 import ctypes as C
+import math
 import threading
 import weakref
 
@@ -833,3 +834,87 @@ def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, orig
         if n_verts and n_faces:
             check(lib().b2r_mc_normals(ptr(field), n0, n1, n2, level, ptr(scratch), ptr(nrm), _stream(field)), "b2r_mc_normals")
     return verts, faces, nrm
+
+
+def _mesh_faces(faces: torch.Tensor, n_verts: int) -> torch.Tensor:
+    """``faces`` as a contiguous [F,3] int32 CUDA tensor whose every index lies in [0, n_verts); raises RuntimeError otherwise,
+    before anything is launched on the mesh (reads the indices' min / max: one host synchronisation when F > 0)."""
+    if not isinstance(faces, torch.Tensor) or not faces.is_cuda or faces.dtype != torch.int32 or faces.dim() != 2 or faces.shape[1] != 3:
+        raise RuntimeError("faces must be an [F,3] int32 CUDA tensor")
+    if not 0 <= n_verts <= _INT32_MAX or faces.shape[0] > _INT32_MAX:
+        raise RuntimeError(f"{n_verts} vertices / {faces.shape[0]} faces: the mesh kernels take at most 2^31 - 1 of each")
+    if faces.numel():
+        lo, hi = (int(v) for v in torch.aminmax(faces))
+        if lo < 0 or hi >= n_verts:
+            raise RuntimeError(f"face indices span [{lo}, {hi}], outside [0, {n_verts}) for {n_verts} vertices")
+    return faces.contiguous()
+
+
+def _cc_label(faces: torch.Tensor, n_verts: int, scratch: torch.Tensor) -> torch.Tensor:
+    labels = torch.empty((n_verts,), dtype=torch.int32, device=faces.device)
+    check(lib().b2r_mesh_cc_label(ptr(faces), faces.shape[0], n_verts, ptr(labels), ptr(scratch), _stream(faces)), "b2r_mesh_cc_label")
+    return labels
+
+
+def mesh_components(faces: torch.Tensor, n_verts: int) -> torch.Tensor:
+    """Connected components of the mesh ``faces`` [F,3] (int32, on the device) over ``n_verts`` vertices, joined by the edges
+    of its triangles (b2r_mesh_cc_label): int32 labels [V], the smallest vertex index of each vertex's component (a vertex no
+    face uses is its own component), equal to ``oracle.mesh_components.component_labels``.  Checks that every index lies in
+    [0, n_verts) first (RuntimeError otherwise; one host synchronisation)."""
+    n_verts = int(n_verts)
+    faces = _mesh_faces(faces, n_verts)
+    with torch.cuda.device(faces.device):
+        scratch = torch.empty((lib().b2r_mesh_cc_scratch_bytes(n_verts, faces.shape[0]),), dtype=torch.uint8, device=faces.device)
+        return _cc_label(faces, n_verts, scratch)
+
+
+def _check_ratio(ratio) -> float:
+    r = float(ratio)
+    if not (math.isfinite(r) and 0.0 <= r <= 1.0):
+        raise ValueError(f"ratio must be finite and in [0, 1], got {ratio}")
+    return float(np.float32(r))
+
+
+def _filter_components(verts: torch.Tensor, faces: torch.Tensor, ratio: float, normals: torch.Tensor | None):
+    """filter_components for faces already known to index [0, V) (label, select, one host read of (V', F'), compact)."""
+    dev, n_verts, n_faces = verts.device, verts.shape[0], faces.shape[0]
+    with torch.cuda.device(dev):
+        st = _stream(verts)
+        scratch = torch.empty((lib().b2r_mesh_cc_scratch_bytes(n_verts, n_faces),), dtype=torch.uint8, device=dev)
+        labels = _cc_label(faces, n_verts, scratch)
+        totals = torch.empty((2,), dtype=torch.int64, device=dev)
+        check(lib().b2r_mesh_cc_select(ptr(faces), n_faces, n_verts, ptr(labels), ratio, ptr(scratch), ptr(totals), st),
+              "b2r_mesh_cc_select")
+        kv, kf = (int(v) for v in totals.tolist())
+        v_out = torch.empty((kv, 3), dtype=torch.float32, device=dev)
+        f_out = torch.empty((kf, 3), dtype=torch.int32, device=dev)
+        n_out = None if normals is None else torch.empty((kv, 3), dtype=torch.float32, device=dev)
+        if kv:
+            check(lib().b2r_mesh_cc_compact(ptr(verts), ptr(normals), ptr(faces), n_faces, n_verts, ptr(scratch), ptr(v_out), ptr(n_out),
+                                            ptr(f_out), st), "b2r_mesh_cc_compact")
+    return v_out, f_out, n_out
+
+
+def filter_components(verts: torch.Tensor, faces: torch.Tensor, ratio: float, normals: torch.Tensor | None = None):
+    """Removes the small connected components of a mesh on the device (b2r_mesh_cc_label / _select / _compact).  A component
+    (vertices joined by the edges of its triangles) with t triangles is kept iff t >= 1 and t >= ratio * t_max, compared in
+    float64 with ``ratio`` rounded to float32, where t_max is the largest component's count: ratio 1 keeps the largest component
+    and any tied with it, and a vertex no face uses is dropped.  Kept vertices (and their ``normals``) and faces keep their
+    relative order; face indices are remapped.  Returns ``(verts [V',3], faces [F',3] int32, normals [V',3] | None)``, equal to
+    ``oracle.mesh_components.filter_components``.  ``ratio`` must be finite and in [0, 1] (ValueError); 0 returns the inputs
+    unchanged without a launch.  Otherwise checks that ``faces`` is [F,3] int32 on the device with every index in [0, V)
+    (RuntimeError otherwise, before any launch; one host synchronisation), then synchronises once more to read (V', F')."""
+    r = _check_ratio(ratio)
+    if r == 0.0:
+        return verts, faces, normals
+    verts = _cuda_f32(verts, "verts")
+    if verts.dim() != 2 or verts.shape[1] != 3:
+        raise RuntimeError(f"verts must be [V,3], got {list(verts.shape)}")
+    if normals is not None:
+        normals = _cuda_f32(normals, "normals")
+        if normals.shape != verts.shape:
+            raise RuntimeError(f"normals must have the shape of verts {list(verts.shape)}, got {list(normals.shape)}")
+    faces = _mesh_faces(faces, verts.shape[0])
+    if faces.device != verts.device or (normals is not None and normals.device != verts.device):
+        raise RuntimeError("verts, faces and normals must be on the same device")
+    return _filter_components(verts, faces, r, normals)

@@ -185,7 +185,7 @@ def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=No
 
 
 def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None, normals=False,
-                colors=False):
+                colors=False, min_component_ratio=0.0):
     """``create_mesh`` (pi_GAN/utils.py:42-180) on the device: the sdf of ``create_mesh_sdf`` never leaves the GPU,
     ``ops.marching_cubes`` extracts its level set (the reference's skimage call at level -20: below = sigma > 20, so the
     triangle normals point out of the object), and only the mesh crosses to the host.  Returns ``(verts [V,3] float32,
@@ -194,8 +194,12 @@ def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level
     ``face`` vertex_indices as a uchar-counted list of i4).  Synchronises with the host once to size the mesh.
     ``normals`` / ``colors``: also compute the unit vertex normals (out of the object) and the uint8 colours the conditioned
     generator's rgb head gives each vertex seen along the inward normal; the PLY then carries nx/ny/nz and red/green/blue,
-    and the return value is ``(verts, faces, normals | None, colors | None)``."""
+    and the return value is ``(verts, faces, normals | None, colors | None)``.
+    ``min_component_ratio`` (finite, in [0, 1]) above 0 removes every connected component with fewer triangles than that share
+    of the largest component's (ops.filter_components; 1 keeps the largest and any tied with it), before the colour query; the
+    call then synchronises with the host twice, once for the marching-cubes size and once for the filtered size.  0 (the
+    default) keeps every triangle."""
     sdf = _sdf_device(generator, N, max_batch, z, precision)
     out = _export_mesh(generator.film_siren_nerf, sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1), ply_filename, normals, colors,
-                       precision)
+                       precision, min_component_ratio)
     return out if (normals or colors) else out[:2]

@@ -9,7 +9,13 @@ The NeRF lines time nerf_render.create_mesh stage by stage on the default box [-
 head is scaled by 100 with a zeroed bias (the threshold is the 70th percentile of its sigma): the box-lattice density query
 (bf16 sigma-only kernel) in ms and points/s, marching cubes, the vertex normals (b2r_mc_normals), the colour query at
 x = [vertex, -normal] with to8b, the D2H copy + PLY write with normals and colours, and one whole create_mesh call that writes the
-coloured PLY."""
+coloured PLY.
+
+The "components" entries time the connected-component stages of both meshes (b2r_mesh_cc_label, _select at ratio 0.01 without
+the host read of (V', F'), _compact; device events, median of 20 after warm-up; the pi-GAN mesh without normals, the NeRF one
+with them): ms and triangles/s per stage, the least bytes each stage moves against the copy peak, the number of components,
+(V', F'), and their share of the density query.  For the NeRF mesh also the colour query, the D2H + PLY write and one whole
+create_mesh(min_component_ratio=0.01) call on the filtered mesh, against the unfiltered numbers above."""
 import json
 import os
 import statistics
@@ -100,6 +106,58 @@ def _timed(fn, reps):
     return statistics.median(ts), res
 
 
+CC_RATIO = 0.01
+
+
+def cc_bytes(nv, nf, kv, kf, normals):
+    """Bytes the component stages move at the least, from the mesh's sizes: label writes parent[V], reads the faces (12 B each)
+    and finds every face's three roots, then reads parent[V] and writes labels[V] (16 B/vertex + 12 B/face before any parent
+    traffic of the finds); select clears the counts, reads a label per face for the counts and again for the marks, the counts
+    and labels per vertex, and writes a word per vertex (16 B/vertex + 32 B/face); compact reads the words, the vertices (and
+    normals) and the faces, and writes what is kept."""
+    w = 24 if normals else 12
+    return {"label": 16 * nv + 12 * nf, "select": 16 * nv + 32 * nf, "compact": (4 + w) * nv + w * kv + 12 * nf + 12 * kf}
+
+
+def cc_times(verts, faces, normals, ratio=CC_RATIO):
+    """Device ms (median of REPS after 3 warm-ups) of b2r_mesh_cc_label, b2r_mesh_cc_select and b2r_mesh_cc_compact, plus the
+    number of components (vertices that are their own label), (V', F') and a check against ops.filter_components."""
+    nv, nf = verts.shape[0], faces.shape[0]
+    dev = verts.device
+    st = torch.cuda.current_stream().cuda_stream
+    scratch = torch.empty((lib().b2r_mesh_cc_scratch_bytes(nv, nf),), dtype=torch.uint8, device=dev)
+    labels = torch.empty((nv,), dtype=torch.int32, device=dev)
+    totals = torch.empty((2,), dtype=torch.int64, device=dev)
+    label = lambda: check(lib().b2r_mesh_cc_label(ptr(faces), nf, nv, ptr(labels), ptr(scratch), st), "b2r_mesh_cc_label")  # noqa: E731
+    select = lambda: check(lib().b2r_mesh_cc_select(ptr(faces), nf, nv, ptr(labels), ratio, ptr(scratch), ptr(totals), st),  # noqa: E731
+                           "b2r_mesh_cc_select")
+    ms = {}
+    ms["label"], _ = _timed(label, REPS)
+    ms["select"], _ = _timed(select, REPS)
+    kv, kf = (int(v) for v in totals.tolist())
+    v_out = torch.empty((kv, 3), dtype=torch.float32, device=dev)
+    n_out = None if normals is None else torch.empty((kv, 3), dtype=torch.float32, device=dev)
+    f_out = torch.empty((kf, 3), dtype=torch.int32, device=dev)
+    compact = lambda: check(lib().b2r_mesh_cc_compact(ptr(verts), ptr(normals), ptr(faces), nf, nv, ptr(scratch), ptr(v_out), ptr(n_out),  # noqa: E731
+                                                      ptr(f_out), st), "b2r_mesh_cc_compact")
+    ms["compact"], _ = _timed(compact, REPS)
+    n_comp = int((labels == torch.arange(nv, dtype=torch.int32, device=dev)).sum())
+    ref = ops.filter_components(verts, faces, ratio, normals)
+    same = bool(torch.equal(ref[0], v_out) and torch.equal(ref[1], f_out) and (normals is None or torch.equal(ref[2], n_out)))
+    nb = cc_bytes(nv, nf, kv, kf, normals is not None)
+    out = {"components": n_comp, "ratio": ratio, "V_kept": kv, "F_kept": kf, "equals_ops_filter_components": same}
+    for k in ("label", "select", "compact"):
+        out[f"{k}_ms"] = round(ms[k], 4)
+        out[f"{k}_Gtri_per_s"] = round(nf / (ms[k] * 1e-3) / 1e9, 3)
+        out[f"{k}_min_bytes"] = nb[k]
+        out[f"{k}_frac_of_copy_peak"] = round(nb[k] / (ms[k] * 1e-3) / 1e9 / COPY_PEAK_GBS, 3)
+    out["total_ms"] = round(sum(ms.values()), 4)
+    out["parent_bytes"] = 4 * nv
+    out["parent_fits_l2"] = 4 * nv < 126e6
+    del scratch, labels, v_out, n_out, f_out, ref
+    return out
+
+
 NERF_TRUNK_FLOP = 2 * (60 * 256 + 4 * 256 * 256 + 316 * 256 + 2 * 256 * 256 + 256)    # 8-layer trunk + sigma head, per point
 
 
@@ -140,13 +198,37 @@ def nerf_lines():
             torch.cuda.synchronize()
             whole_ms = (time.perf_counter() - t0) * 1e3
         same = bool(torch.equal(whole[0], verts) and torch.equal(whole[1], faces) and torch.equal(whole[2], nrm) and torch.equal(whole[3], rgb))
+        del whole
+        cc = cc_times(verts, faces, nrm)
+        cc["over_density_query"] = round(cc["total_ms"] / q_ms, 4)
+        fv, ff, fn = ops.filter_components(verts, faces, CC_RATIO, nrm)
+        cc["color_query_filtered_ms"], frgb = _timed(lambda: mesh.vertex_colors(net, fv, fn), 5)
+        cc["color_query_filtered_ms"] = round(cc["color_query_filtered_ms"], 3)
+        with tempfile.TemporaryDirectory() as tmp:
+            path = os.path.join(tmp, "mesh.ply")
+            fts = []
+            for _ in range(2):
+                torch.cuda.synchronize()
+                t0 = time.perf_counter()
+                mesh.write_ply(path, fv.cpu().numpy(), ff.cpu().numpy(), fn.cpu().numpy(), frgb.cpu().numpy())
+                fts.append((time.perf_counter() - t0) * 1e3)
+            cc["d2h_plus_ply_filtered_ms"] = round(statistics.median(fts), 2)
+            cc["ply_bytes_filtered"] = os.path.getsize(path)
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            whole = nerf_render.create_mesh(net, path, n, threshold=thr, min_component_ratio=CC_RATIO)
+            torch.cuda.synchronize()
+            cc["create_mesh_call_filtered_ms"] = round((time.perf_counter() - t0) * 1e3, 1)
+        cc["create_mesh_filtered_equals_stages"] = bool(torch.equal(whole[0], fv) and torch.equal(whole[1], ff) and torch.equal(whole[2], fn)
+                                                        and torch.equal(whole[3], frgb))
+        del fv, ff, fn, frgb
         res[str(n)] = {
             "dims": list(field.shape), "points": pts, "density_query_ms": round(q_ms, 3), "points_per_s": round(pts / (q_ms * 1e-3) / 1e9, 3),
             "points_per_s_unit": "G/s", "trunk_TFLOPs": round(pts * NERF_TRUNK_FLOP / (q_ms * 1e-3) / 1e12, 1), "threshold": thr,
             "marching_cubes_device_ms": round(dev_ms, 4), "host_read_VF_ms": round(host_ms, 4), "normals_ms": round(nrm_ms, 4),
             "color_query_ms": round(col_ms, 3), "V": int(verts.shape[0]), "F": int(faces.shape[0]),
             "d2h_plus_ply_ms": round(statistics.median(ts), 2), "ply_bytes": ply_bytes, "create_mesh_call_ms": round(whole_ms, 1),
-            "create_mesh_equals_stages": same}
+            "create_mesh_equals_stages": same, "components": cc}
         del sigma, field, verts, faces, nrm, rgb, whole, scratch
         torch.cuda.empty_cache()
     return res
@@ -165,7 +247,7 @@ def main():
         net.output_layer_sigma[0].weight.mul_(100.0)
         net.output_layer_sigma[0].bias.zero_()
         gen.set_film_params(gen.get_mapping(z)[0])
-    out = {"metric": "create_mesh on the device: density query, marching cubes, mesh D2H + PLY", "gpu": smi.stdout.strip(),
+    out = {"metric": "create_mesh on the device: density query, marching cubes, connected components, mesh D2H + PLY", "gpu": smi.stdout.strip(),
            "copy_peak_GBs": COPY_PEAK_GBS, "sizes": {}}
     for n in (256, 512):
         q_ms, sdf = density_ms(gen, n)
@@ -190,6 +272,9 @@ def main():
             "GBs": round(nb / (dev_ms * 1e-3) / 1e9, 1), "frac_of_copy_peak": round(nb / (dev_ms * 1e-3) / 1e9 / COPY_PEAK_GBS, 3),
             "mc_over_query": round(dev_ms / q_ms, 4), "d2h_plus_ply_ms": round(statistics.median(ts), 2), "ply_bytes": ply_bytes,
             "repeat_run_identical": same, "field_fits_l2": n ** 3 * 4 < 126e6}
+        cc = cc_times(verts, faces, None)
+        cc["over_density_query"] = round(cc["total_ms"] / q_ms, 4)
+        out["sizes"][str(n)]["components"] = cc
         del sdf, verts, faces, ref_v, ref_f
         torch.cuda.empty_cache()
     out["nerf_sizes"] = nerf_lines()
