@@ -333,6 +333,28 @@ int b2r_mesh_cc_select(const int* faces, long long n_faces, long long n_verts, c
 int b2r_mesh_cc_compact(const float* verts, const float* normals_or_null, const int* faces, long long n_faces, long long n_verts,
                         const void* scratch, float* verts_out, float* normals_out, int* faces_out, void* stream);
 
+/* ---- Taubin smoothing and normals of a triangle mesh (no reference counterpart: clean-up of exported meshes) ---------------
+ * Same mesh conventions and PRECONDITION as the connected components above (faces[F,3] int32 index verts[V,3] fp32, every index
+ * in [0, n_verts), counts in [0, INT32_MAX], NULL allowed only for a count of 0).  A corner of vertex v is (f, c) with
+ * faces[f][c] == v; v's corners are taken in ascending (f, c), a face listing v twice gives two.  scratch:
+ * b2r_mesh_adj_scratch_bytes(V, F) bytes, 16-byte aligned (0 for counts outside [0, INT32_MAX]; with V = 0 the calls do
+ * nothing and scratch may be NULL).
+ *   b2r_mesh_adjacency: builds each vertex's corner list into scratch, exactly ordered whatever the schedule.
+ *   b2r_mesh_smooth:    given that scratch, writes verts_out[V,3] = verts after `iterations` (>= 0) Taubin iterations, each a
+ *                       half-step with w = 0.5f then one with w = -0.53f.  A half-step is Jacobi: for v with k > 0 corners,
+ *                       s = 0, then s += p[faces[f][(c+1)%3]], s += p[faces[f][(c+2)%3]] per corner in order; m = s / (float)(2k);
+ *                       p'[v] = p[v] + w (m - p[v]); a vertex with k = 0 keeps p.  verts_out may equal verts.
+ *   b2r_mesh_normals:   given that scratch, writes normals[V,3], the sum over v's corners in order of the face normal
+ *                       (p[f1]-p[f0]) x (p[f2]-p[f0]) in the face's own corner order, divided by sqrt((x x + y y) + z z), or
+ *                       (0, 0, 0) when that is 0.
+ * Every float operation is rounded separately (no FMA; division and sqrt correctly rounded), so the result is reproducible bit for
+ * bit.  The scratch stays valid for any number of _smooth / _normals calls on the same faces. */
+size_t b2r_mesh_adj_scratch_bytes(long long n_verts, long long n_faces);
+int b2r_mesh_adjacency(const int* faces, long long n_faces, long long n_verts, void* scratch, void* stream);
+int b2r_mesh_smooth(const float* verts, long long n_faces, long long n_verts, int iterations, void* scratch, float* verts_out,
+                    void* stream);
+int b2r_mesh_normals(const float* verts, long long n_faces, long long n_verts, const void* scratch, float* normals, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

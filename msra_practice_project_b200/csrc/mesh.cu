@@ -460,6 +460,251 @@ __global__ void __launch_bounds__(kThreads) cc_compact_kernel(const float* __res
     }
 }
 
+// ---- vertex-face adjacency, Taubin smoothing and mesh normals (b2r_mesh_adjacency / _smooth / _normals) -------------------------
+// A corner is (f, c) with faces[f][c] == v; each vertex's corners are stored contiguously in ascending (f, c), so every sum over
+// them runs in one fixed order and the float path needs no atomics.  Build: count the corners of each vertex (64-bit atomics into
+// ends[]), exclusive 64-bit scan of the counts (tile sums, one-CTA scan of the tile sums, tile scans), fill the corner keys
+// 3f + c with an atomic cursor (ends[v] then holds the END of v's list: begin(v) = ends[v-1], begin(0) = 0), and sort each
+// vertex's keys (insertion sort up to kAdjInsertion keys, heapsort above, so any degree is exact in O(d log d)), replacing each key
+// by its record in place.  The record is the int2 (a, b) = (faces[f][(c+1)%3], faces[f][(c+2)%3]) with c in the two spare high
+// bits (bit 31 of a = c & 1, bit 31 of b = c >> 1): a half-step only gathers positions, and the normals kernel rebuilds the face's
+// own corner order from (v, a, b, c).
+// Scratch: ends[V] (u64), tile sums (u64 per kTile vertices), the records [3F] (int2), and a [V,3] position buffer that the
+// half-steps ping-pong through.
+struct AdjLayout {
+    size_t ends, tile_sums, adj, pos, total;
+};
+
+inline AdjLayout adj_layout(long long n_verts, long long n_faces) {
+    const long long tiles = (n_verts + kTile - 1) / kTile;
+    AdjLayout l;
+    l.ends = 0;
+    l.tile_sums = l.ends + align256((size_t)n_verts * 8);
+    l.adj = l.tile_sums + align256((size_t)tiles * 8);
+    l.pos = l.adj + align256((size_t)n_faces * 24);
+    l.total = l.pos + align256((size_t)n_verts * 12);
+    return l;
+}
+
+constexpr int kAdjInsertion = 16;
+constexpr unsigned kIndexMask = 0x7fffffffu;
+constexpr float kTaubinLambda = 0.5f, kTaubinMu = -0.53f;
+
+__global__ void __launch_bounds__(kThreads) adj_count_kernel(const int* __restrict__ faces, unsigned n_faces,
+                                                             unsigned long long* __restrict__ ends) {
+    const unsigned f = blockIdx.x * kThreads + threadIdx.x;
+    if (f >= n_faces) return;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) atomicAdd(ends + faces[3 * (size_t)f + c], 1ull);
+}
+
+__device__ __forceinline__ unsigned long long warp_inclusive_scan64(unsigned long long x, int lane) {
+#pragma unroll
+    for (int o = 1; o < kWarp; o <<= 1) {
+        const unsigned long long y = __shfl_up_sync(kFull, x, o);
+        if (lane >= o) x += y;
+    }
+    return x;
+}
+
+// Thread t of tile b owns the kPer consecutive counts from b * kTile + t * kPer.
+__global__ void __launch_bounds__(kThreads) adj_tile_sum_kernel(const unsigned long long* __restrict__ cnt, unsigned n,
+                                                                unsigned long long* __restrict__ tile_sums) {
+    __shared__ unsigned long long s_w[kWarps];
+    const unsigned base = blockIdx.x * (unsigned)kTile + threadIdx.x * kPer;
+    unsigned long long t = 0;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q)
+        if (base + q < n) t += cnt[base + q];
+#pragma unroll
+    for (int o = kWarp / 2; o; o >>= 1) t += __shfl_down_sync(kFull, t, o);
+    if ((threadIdx.x & (kWarp - 1)) == 0) s_w[threadIdx.x >> 5] = t;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        unsigned long long s = 0;
+#pragma unroll
+        for (int w = 0; w < kWarps; ++w) s += s_w[w];
+        tile_sums[blockIdx.x] = s;
+    }
+}
+
+// One CTA, in place: tile_sums[b] becomes the sum of the tiles before b.  Thread t owns a contiguous run of tiles.
+__global__ void __launch_bounds__(kScanThreads) adj_scan_tiles_kernel(unsigned long long* __restrict__ tile_sums, int tiles) {
+    __shared__ unsigned long long s_w[kScanThreads / kWarp];
+    const int lane = threadIdx.x & (kWarp - 1), warp = threadIdx.x >> 5;
+    const int per = (tiles + kScanThreads - 1) / kScanThreads;
+    const int beg = min(tiles, (int)threadIdx.x * per), end = min(tiles, beg + per);
+    unsigned long long t = 0;
+    for (int b = beg; b < end; ++b) t += tile_sums[b];
+    const unsigned long long incl = warp_inclusive_scan64(t, lane);
+    if (lane == kWarp - 1) s_w[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        const unsigned long long x = s_w[lane];
+        s_w[lane] = warp_inclusive_scan64(x, lane) - x;
+    }
+    __syncthreads();
+    unsigned long long run = s_w[warp] + incl - t;
+    for (int b = beg; b < end; ++b) {
+        const unsigned long long x = tile_sums[b];
+        tile_sums[b] = run;
+        run += x;
+    }
+}
+
+// In place: cnt[v] becomes the exclusive prefix sum of the counts (the first slot of v's corners).
+__global__ void __launch_bounds__(kThreads) adj_tile_scan_kernel(unsigned long long* __restrict__ cnt, unsigned n,
+                                                                 const unsigned long long* __restrict__ tile_offsets) {
+    __shared__ unsigned long long s_w[kWarps];
+    const int lane = threadIdx.x & (kWarp - 1), warp = threadIdx.x >> 5;
+    const unsigned base = blockIdx.x * (unsigned)kTile + threadIdx.x * kPer;
+    unsigned long long v[kPer], t = 0;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        v[q] = base + q < n ? cnt[base + q] : 0ull;
+        t += v[q];
+    }
+    const unsigned long long incl = warp_inclusive_scan64(t, lane);
+    if (lane == kWarp - 1) s_w[warp] = incl;
+    __syncthreads();
+    if (warp == 0) {
+        const unsigned long long x = lane < kWarps ? s_w[lane] : 0ull;
+        const unsigned long long y = warp_inclusive_scan64(x, lane);
+        __syncwarp();
+        if (lane < kWarps) s_w[lane] = y - x;
+    }
+    __syncthreads();
+    unsigned long long run = tile_offsets[blockIdx.x] + s_w[warp] + incl - t;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        if (base + q < n) cnt[base + q] = run;
+        run += v[q];
+    }
+}
+
+// Corner (f, c) takes the next free slot of its vertex; ends[v] moves from v's first slot to one past its last.
+__global__ void __launch_bounds__(kThreads) adj_fill_kernel(const int* __restrict__ faces, unsigned n_faces,
+                                                            unsigned long long* __restrict__ ends, unsigned long long* __restrict__ keys) {
+    const unsigned f = blockIdx.x * kThreads + threadIdx.x;
+    if (f >= n_faces) return;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) keys[atomicAdd(ends + faces[3 * (size_t)f + c], 1ull)] = 3ull * f + c;
+}
+
+__device__ __forceinline__ unsigned long long adj_begin(const unsigned long long* __restrict__ ends, unsigned v) {
+    return v ? ends[v - 1] : 0ull;
+}
+
+// Sorts the keys of one vertex ascending and replaces each by its record (a, b, c), stored as the int2's little-endian u64.
+__global__ void __launch_bounds__(kThreads) adj_sort_kernel(const int* __restrict__ faces, unsigned n_verts,
+                                                            const unsigned long long* __restrict__ ends, unsigned long long* __restrict__ keys) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n_verts) return;
+    const unsigned long long beg = adj_begin(ends, v);
+    const long long d = (long long)(ends[v] - beg);
+    unsigned long long* a = keys + beg;
+    if (d <= kAdjInsertion) {
+        for (long long i = 1; i < d; ++i) {
+            const unsigned long long k = a[i];
+            long long j = i;
+            for (; j > 0 && a[j - 1] > k; --j) a[j] = a[j - 1];
+            a[j] = k;
+        }
+    } else {
+        auto sift = [a](long long root, long long n) {
+            const unsigned long long k = a[root];
+            for (long long child = 2 * root + 1; child < n; child = 2 * root + 1) {
+                if (child + 1 < n && a[child + 1] > a[child]) ++child;
+                if (a[child] <= k) break;
+                a[root] = a[child];
+                root = child;
+            }
+            a[root] = k;
+        };
+        for (long long i = d / 2 - 1; i >= 0; --i) sift(i, d);
+        for (long long i = d - 1; i > 0; --i) {
+            const unsigned long long top = a[0];
+            a[0] = a[i];
+            a[i] = top;
+            sift(0, i);
+        }
+    }
+    for (long long i = 0; i < d; ++i) {
+        const unsigned long long k = a[i], f = k / 3;
+        const unsigned c = (unsigned)(k - 3 * f);
+        const unsigned ra = (unsigned)faces[3 * f + (c + 1) % 3] | (c & 1u) << 31;
+        const unsigned rb = (unsigned)faces[3 * f + (c + 2) % 3] | (c >> 1) << 31;
+        a[i] = (unsigned long long)ra | (unsigned long long)rb << 32;
+    }
+}
+
+// One umbrella half-step, Jacobi: out[v] = p[v] + w (m - p[v]), m = (sum over v's corners of p[a] + p[b]) / (2k), every
+// operation rounded separately (no FMA).  A vertex without corners keeps its position.
+__global__ void __launch_bounds__(kThreads) smooth_kernel(const float* __restrict__ p, unsigned n_verts,
+                                                          const unsigned long long* __restrict__ ends, const int2* __restrict__ adj,
+                                                          float w, float* __restrict__ out) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n_verts) return;
+    const unsigned long long beg = adj_begin(ends, v), end = ends[v];
+    const float* pv = p + 3 * (size_t)v;
+    float* o = out + 3 * (size_t)v;
+    if (beg == end) {
+#pragma unroll
+        for (int c = 0; c < 3; ++c) o[c] = pv[c];
+        return;
+    }
+    float s[3] = {0.f, 0.f, 0.f};
+    for (unsigned long long i = beg; i < end; ++i) {
+        const int2 r = adj[i];
+        const float* pa = p + 3 * (size_t)((unsigned)r.x & kIndexMask);
+        const float* pb = p + 3 * (size_t)((unsigned)r.y & kIndexMask);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) s[c] = __fadd_rn(__fadd_rn(s[c], pa[c]), pb[c]);
+    }
+    const float k2 = __ull2float_rn(2 * (end - beg));
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const float x = pv[c];
+        o[c] = __fadd_rn(x, __fmul_rn(w, __fsub_rn(__fdiv_rn(s[c], k2), x)));
+    }
+}
+
+// Area-weighted vertex normals: the sum over v's corners of the face normal (p[f1] - p[f0]) x (p[f2] - p[f0]) in the face's
+// own corner order, divided by its length like mc_normals_kernel; (0, 0, 0) when the length is 0.
+__global__ void __launch_bounds__(kThreads) mesh_normals_kernel(const float* __restrict__ p, unsigned n_verts,
+                                                                const unsigned long long* __restrict__ ends,
+                                                                const int2* __restrict__ adj, float* __restrict__ normals) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n_verts) return;
+    const unsigned long long end = ends[v];
+    float n[3] = {0.f, 0.f, 0.f};
+    for (unsigned long long i = adj_begin(ends, v); i < end; ++i) {
+        const int2 r = adj[i];
+        const unsigned a = (unsigned)r.x & kIndexMask, b = (unsigned)r.y & kIndexMask;
+        const unsigned c = (unsigned)r.x >> 31 | ((unsigned)r.y >> 31) << 1;
+        // the cyclic order (v, a, b) starts at corner c of the face
+        const unsigned f0 = c == 0 ? v : c == 1 ? b : a, f1 = c == 0 ? a : c == 1 ? v : b, f2 = c == 0 ? b : c == 1 ? a : v;
+        const float* p0 = p + 3 * (size_t)f0;
+        const float* p1 = p + 3 * (size_t)f1;
+        const float* p2 = p + 3 * (size_t)f2;
+        float e1[3], e2[3];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            e1[k] = __fsub_rn(p1[k], p0[k]);
+            e2[k] = __fsub_rn(p2[k], p0[k]);
+        }
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const int k1 = (k + 1) % 3, k2 = (k + 2) % 3;
+            n[k] = __fadd_rn(n[k], __fsub_rn(__fmul_rn(e1[k1], e2[k2]), __fmul_rn(e1[k2], e2[k1])));
+        }
+    }
+    const float len = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(n[0], n[0]), __fmul_rn(n[1], n[1])), __fmul_rn(n[2], n[2])));
+    float* o = normals + 3 * (size_t)v;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) o[k] = len > 0.f ? __fdiv_rn(n[k], len) : 0.f;
+}
+
 int check_grid(const char* what, int n0, int n1, int n2) {
     B2R_CHECK_ARG(n0 >= 2 && n1 >= 2 && n2 >= 2, "%s: every axis needs n >= 2 (got %d x %d x %d)", what, n0, n1, n2);
     B2R_CHECK_ARG((long long)n0 * n1 * n2 <= INT32_MAX, "%s: n0*n1*n2 = %lld exceeds INT32_MAX", what, (long long)n0 * n1 * n2);
@@ -614,6 +859,83 @@ extern "C" int b2r_mesh_cc_compact(const float* verts, const float* normals_or_n
     cc_compact_kernel<<<tiles, kThreads, 0, (cudaStream_t)stream>>>(verts, normals_or_null, faces, (unsigned)n_faces, (unsigned)n_verts,
                                                                     (const unsigned*)(s + l.vword), (const longlong2*)(s + l.offsets),
                                                                     verts_out, normals_out, faces_out);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" size_t b2r_mesh_adj_scratch_bytes(long long n_verts, long long n_faces) {
+    if (n_verts < 0 || n_verts > INT32_MAX || n_faces < 0 || n_faces > INT32_MAX) return 0;
+    return b2r::mc::adj_layout(n_verts, n_faces).total;
+}
+
+extern "C" int b2r_mesh_adjacency(const int* faces, long long n_faces, long long n_verts, void* scratch, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_adjacency";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG(faces || !n_faces, "%s: NULL faces with n_faces > 0", what);
+    if (!n_verts) return 0;                  // an empty mesh has a 0-byte scratch, which may be NULL
+    if (int rc = check_scratch(what, scratch)) return rc;
+    const AdjLayout l = adj_layout(n_verts, n_faces);
+    const int tiles = (int)((n_verts + kTile - 1) / kTile);
+    char* s = static_cast<char*>(scratch);
+    unsigned long long* ends = (unsigned long long*)(s + l.ends);
+    unsigned long long* tile_sums = (unsigned long long*)(s + l.tile_sums);
+    unsigned long long* keys = (unsigned long long*)(s + l.adj);
+    const unsigned nv = (unsigned)n_verts, nf = (unsigned)n_faces;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = b2r::cuda_result(cudaMemsetAsync(ends, 0, (size_t)n_verts * 8, st), what)) return rc;
+    if (nf) adj_count_kernel<<<blocks_of(nf, kThreads), kThreads, 0, st>>>(faces, nf, ends);
+    adj_tile_sum_kernel<<<tiles, kThreads, 0, st>>>(ends, nv, tile_sums);
+    adj_scan_tiles_kernel<<<1, kScanThreads, 0, st>>>(tile_sums, tiles);
+    adj_tile_scan_kernel<<<tiles, kThreads, 0, st>>>(ends, nv, tile_sums);
+    if (nf) {
+        adj_fill_kernel<<<blocks_of(nf, kThreads), kThreads, 0, st>>>(faces, nf, ends, keys);
+        adj_sort_kernel<<<blocks_of(nv, kThreads), kThreads, 0, st>>>(faces, nv, ends, keys);
+    }
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_smooth(const float* verts, long long n_faces, long long n_verts, int iterations, void* scratch, float* verts_out,
+                               void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_smooth";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG((verts && verts_out) || !n_verts, "%s: NULL verts / verts_out with n_verts > 0", what);
+    B2R_CHECK_ARG(iterations >= 0, "%s: iterations = %d must be >= 0", what, iterations);
+    if (!n_verts) return 0;                  // an empty mesh has a 0-byte scratch, which may be NULL
+    if (int rc = check_scratch(what, scratch)) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (!iterations) {
+        if (verts == verts_out) return 0;
+        return b2r::cuda_result(cudaMemcpyAsync(verts_out, verts, (size_t)n_verts * 12, cudaMemcpyDeviceToDevice, st), what);
+    }
+    const AdjLayout l = adj_layout(n_verts, n_faces);
+    char* s = static_cast<char*>(scratch);
+    const unsigned long long* ends = (const unsigned long long*)(s + l.ends);
+    const int2* adj = (const int2*)(s + l.adj);
+    float* tmp = (float*)(s + l.pos);
+    const unsigned nv = (unsigned)n_verts, blocks = blocks_of(nv, kThreads);
+    for (int it = 0; it < iterations; ++it) {
+        smooth_kernel<<<blocks, kThreads, 0, st>>>(it ? verts_out : verts, nv, ends, adj, kTaubinLambda, tmp);
+        smooth_kernel<<<blocks, kThreads, 0, st>>>(tmp, nv, ends, adj, kTaubinMu, verts_out);
+    }
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_normals(const float* verts, long long n_faces, long long n_verts, const void* scratch, float* normals,
+                                void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_normals";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG((verts && normals) || !n_verts, "%s: NULL verts / normals with n_verts > 0", what);
+    if (!n_verts) return 0;                  // an empty mesh has a 0-byte scratch, which may be NULL
+    if (int rc = check_scratch(what, scratch)) return rc;
+    const AdjLayout l = adj_layout(n_verts, n_faces);
+    const char* s = static_cast<const char*>(scratch);
+    mesh_normals_kernel<<<blocks_of(n_verts, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
+        verts, (unsigned)n_verts, (const unsigned long long*)(s + l.ends), (const int2*)(s + l.adj), normals);
     B2R_LAUNCH_CHECK(what);
     return 0;
 }

@@ -80,15 +80,22 @@ def write_ply(filename, verts, faces, normals=None, colors=None):
         fbody.tofile(fh)
 
 
-def export(model, field, level, spacing, origin, ply_filename, normals, colors, precision, min_component_ratio=0.0):
+def export(model, field, level, spacing, origin, ply_filename, normals, colors, precision, min_component_ratio=0.0,
+           smooth_iterations=0):
     """Extract the level set of ``field`` (vertex normals toward increasing field), colour it with ``model`` and write the PLY.
     Returns (verts, faces, normals | None, colors | None) on the device.  A ``min_component_ratio`` above 0 removes the
     components with fewer triangles than that share of the largest one (ops.filter_components) before the colour query, so
-    dropped vertices cost no MLP rows; it synchronises with the host once more, to size the filtered mesh."""
-    verts, faces, nrm = extract(field, level, spacing, origin, normals or colors)
+    dropped vertices cost no MLP rows; it synchronises with the host once more, to size the filtered mesh.
+    ``smooth_iterations`` above 0 then runs that many Taubin iterations (ops.smooth_mesh) before the colour query, and the
+    normals become the smoothed mesh's own, so colours are sampled on the smoothed surface; the field normals are not computed."""
+    iterations = ops._check_iterations(smooth_iterations)
+    want_normals = normals or colors
+    verts, faces, nrm = extract(field, level, spacing, origin, want_normals and not iterations)
     if min_component_ratio:
-        # marching-cubes faces index their own vertices, so the index check of ops.filter_components is not needed
+        # marching-cubes faces index their own vertices, so the index checks of ops.filter_components / ops.smooth_mesh are not needed
         verts, faces, nrm = ops._filter_components(verts, faces, ops._check_ratio(min_component_ratio), nrm)
+    if iterations:
+        verts, nrm = ops._smooth_mesh(verts, faces, iterations, want_normals)
     rgb = vertex_colors(model, verts, nrm, precision) if colors else None
     if not normals:
         nrm = None

@@ -309,7 +309,7 @@ def density_lattice(model, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), 
 
 
 def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), threshold=50.0,
-                normals=True, colors=True, precision=None, max_batch=256 ** 3, min_component_ratio=0.0):
+                normals=True, colors=True, precision=None, max_batch=256 ** 3, min_component_ratio=0.0, smooth_iterations=0):
     """Mesh of a trained NeRF / SirenNeRF field on the device: the level set ``sigma = threshold`` of ``density_lattice``
     (marching cubes on -sigma at -threshold, so triangle and vertex normals point out of the object, toward lower density),
     the unit vertex normals, and the uint8 colour the model's rgb head gives each vertex seen by a camera looking along the
@@ -319,7 +319,12 @@ def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), 
     ``min_component_ratio`` (finite, in [0, 1]) above 0 removes the floaters: every connected component with fewer triangles
     than that share of the largest component's (ops.filter_components; 1 keeps the largest and any tied with it), before the
     colour query; the call then synchronises with the host twice, once for the marching-cubes size and once for the filtered
-    size.  0 (the default) keeps every triangle."""
+    size.  0 (the default) keeps every triangle.
+    ``smooth_iterations`` (an int >= 0) above 0 runs that many Taubin lambda|mu iterations on the mesh after the component
+    filter and before the colour query (ops.smooth_mesh): the terraces marching cubes leaves where the density rises steeply
+    through ``threshold`` are smoothed out without shrinking the surface, and the topology is unchanged.  The normals are then
+    the smoothed mesh's own area-weighted vertex normals (still out of the object) and the colours are sampled at the smoothed
+    vertices along them; no host synchronisation is added.  0 (the default) leaves the mesh as extracted."""
     sigma, origin, voxel = density_lattice(model, box_min, box_max, N, max_batch=max_batch, precision=precision)
     return mesh.export(model, sigma.neg_(), -float(threshold), voxel, origin, ply_filename, normals, colors, precision,
-                       min_component_ratio)
+                       min_component_ratio, smooth_iterations)

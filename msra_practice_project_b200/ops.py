@@ -918,3 +918,50 @@ def filter_components(verts: torch.Tensor, faces: torch.Tensor, ratio: float, no
     if faces.device != verts.device or (normals is not None and normals.device != verts.device):
         raise RuntimeError("verts, faces and normals must be on the same device")
     return _filter_components(verts, faces, r, normals)
+
+
+def _check_iterations(iterations) -> int:
+    if isinstance(iterations, bool) or not isinstance(iterations, (int, np.integer)) or not 0 <= iterations <= _INT32_MAX:
+        raise ValueError(f"iterations must be an int in [0, 2^31 - 1], got {iterations!r}")
+    return int(iterations)
+
+
+def _smooth_mesh(verts: torch.Tensor, faces: torch.Tensor, iterations: int, normals: bool):
+    """smooth_mesh for faces already known to index [0, V): (verts', normals' | None), no host synchronisation."""
+    dev, n_verts, n_faces = verts.device, verts.shape[0], faces.shape[0]
+    with torch.cuda.device(dev):
+        st = _stream(verts)
+        scratch = torch.empty((lib().b2r_mesh_adj_scratch_bytes(n_verts, n_faces),), dtype=torch.uint8, device=dev)
+        check(lib().b2r_mesh_adjacency(ptr(faces), n_faces, n_verts, ptr(scratch), st), "b2r_mesh_adjacency")
+        out = verts
+        if iterations:
+            out = torch.empty_like(verts)
+            check(lib().b2r_mesh_smooth(ptr(verts), n_faces, n_verts, iterations, ptr(scratch), ptr(out), st), "b2r_mesh_smooth")
+        nrm = None
+        if normals:
+            nrm = torch.empty_like(verts)
+            check(lib().b2r_mesh_normals(ptr(out), n_faces, n_verts, ptr(scratch), ptr(nrm), st), "b2r_mesh_normals")
+    return out, nrm
+
+
+def smooth_mesh(verts: torch.Tensor, faces: torch.Tensor, iterations: int, *, normals: bool = False):
+    """Taubin lambda|mu smoothing of a triangle mesh on the device (b2r_mesh_adjacency / _smooth / _normals).  Each iteration
+    is two umbrella half-steps, p' = p + w (m - p) with w = 0.5 then w = -0.53, where m is the mean over the vertex's corners
+    of the other two vertices of the corner's face (on a closed manifold mesh: the mean of its neighbours); a vertex no face
+    uses stays where it is.  Topology, vertex order and faces are unchanged.  Returns ``verts' [V,3]``, or
+    ``(verts', normals' [V,3])`` with ``normals``: the unit area-weighted vertex normals of the smoothed mesh ((0, 0, 0) where
+    the fan has no area), which point the way the faces are wound.  Equal to ``oracle.mesh_smoothing.smooth`` /
+    ``mesh_normals``.  ``iterations`` must be an int >= 0 (ValueError); 0 without ``normals`` returns ``verts`` without a
+    launch.  Otherwise checks that ``faces`` is [F,3] int32 on the device with every index in [0, V) (RuntimeError otherwise,
+    before any launch; one host synchronisation)."""
+    iterations = _check_iterations(iterations)
+    if not iterations and not normals:
+        return verts
+    verts = _cuda_f32(verts, "verts")
+    if verts.dim() != 2 or verts.shape[1] != 3:
+        raise RuntimeError(f"verts must be [V,3], got {list(verts.shape)}")
+    faces = _mesh_faces(faces, verts.shape[0])
+    if faces.device != verts.device:
+        raise RuntimeError("verts and faces must be on the same device")
+    out, nrm = _smooth_mesh(verts, faces, iterations, normals)
+    return (out, nrm) if normals else out

@@ -185,7 +185,7 @@ def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=No
 
 
 def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None, normals=False,
-                colors=False, min_component_ratio=0.0):
+                colors=False, min_component_ratio=0.0, smooth_iterations=0):
     """``create_mesh`` (pi_GAN/utils.py:42-180) on the device: the sdf of ``create_mesh_sdf`` never leaves the GPU,
     ``ops.marching_cubes`` extracts its level set (the reference's skimage call at level -20: below = sigma > 20, so the
     triangle normals point out of the object), and only the mesh crosses to the host.  Returns ``(verts [V,3] float32,
@@ -198,8 +198,13 @@ def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level
     ``min_component_ratio`` (finite, in [0, 1]) above 0 removes every connected component with fewer triangles than that share
     of the largest component's (ops.filter_components; 1 keeps the largest and any tied with it), before the colour query; the
     call then synchronises with the host twice, once for the marching-cubes size and once for the filtered size.  0 (the
-    default) keeps every triangle."""
+    default) keeps every triangle.
+    ``smooth_iterations`` (an int >= 0) above 0 runs that many Taubin lambda|mu iterations on the mesh after the component
+    filter and before the colour query (ops.smooth_mesh): the terraces marching cubes leaves along the lattice are smoothed
+    out without moving the surface inward, and the topology is unchanged.  The normals are then the smoothed mesh's own
+    area-weighted vertex normals and the colours are sampled at the smoothed vertices; no host synchronisation is added.
+    0 (the default) leaves the mesh as extracted."""
     sdf = _sdf_device(generator, N, max_batch, z, precision)
     out = _export_mesh(generator.film_siren_nerf, sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1), ply_filename, normals, colors,
-                       precision, min_component_ratio)
+                       precision, min_component_ratio, smooth_iterations)
     return out if (normals or colors) else out[:2]

@@ -15,7 +15,14 @@ The "components" entries time the connected-component stages of both meshes (b2r
 the host read of (V', F'), _compact; device events, median of 20 after warm-up; the pi-GAN mesh without normals, the NeRF one
 with them): ms and triangles/s per stage, the least bytes each stage moves against the copy peak, the number of components,
 (V', F'), and their share of the density query.  For the NeRF mesh also the colour query, the D2H + PLY write and one whole
-create_mesh(min_component_ratio=0.01) call on the filtered mesh, against the unfiltered numbers above."""
+create_mesh(min_component_ratio=0.01) call on the filtered mesh, against the unfiltered numbers above.
+
+The "smoothing" entries time Taubin smoothing on the pi-GAN 512^3 mesh and both NeRF meshes (b2r_mesh_adjacency, one
+b2r_mesh_smooth call of SMOOTH_ITERS iterations divided by SMOOTH_ITERS, b2r_mesh_normals; device events, median of 20 after a
+warm-up): ms per stage, the least bytes each stage moves (smooth_bytes) against the copy peak, the scratch bytes and the peak of
+torch's allocator over one ops.smooth_mesh(normals=True) call above what was allocated before it, and a check against that call.
+For the NeRF meshes also one whole create_mesh(smooth_iterations=SMOOTH_ITERS) call against the unsmoothed one above, and whether
+it equals its stages (ops.smooth_mesh, then the colour query)."""
 import json
 import os
 import statistics
@@ -158,6 +165,53 @@ def cc_times(verts, faces, normals, ratio=CC_RATIO):
     return out
 
 
+SMOOTH_ITERS = 10
+
+
+def smooth_bytes(nv, nf):
+    """Bytes the smoothing stages move at the least, from the mesh's sizes (neighbour positions gathered through the corner
+    records are not counted): the adjacency build reads the faces three times (count, fill, the sort's record lookup; 36 B/face),
+    writes the 8-byte corner keys, then reads and rewrites them as records (72 B/face), and touches ends[] five times (40 B/vertex);
+    a half-step reads ends[], the records and its own position and writes one (32 B/vertex + 24 B/face), an iteration is two;
+    the normals read ends[], the records and a position and write a normal (32 B/vertex + 24 B/face)."""
+    return {"adjacency": 40 * nv + 108 * nf, "iteration": 2 * (32 * nv + 24 * nf), "normals": 32 * nv + 24 * nf}
+
+
+def smooth_times(verts, faces):
+    """Device ms of b2r_mesh_adjacency, of one Taubin iteration and of b2r_mesh_normals, their least bytes against the copy
+    peak, the adjacency's memory, and a check against ops.smooth_mesh."""
+    nv, nf = verts.shape[0], faces.shape[0]
+    dev = verts.device
+    st = torch.cuda.current_stream().cuda_stream
+    torch.cuda.synchronize()
+    base = torch.cuda.memory_allocated(dev)
+    torch.cuda.reset_peak_memory_stats(dev)
+    ref_v, ref_n = ops.smooth_mesh(verts, faces, SMOOTH_ITERS, normals=True)
+    torch.cuda.synchronize()
+    peak = torch.cuda.max_memory_allocated(dev) - base
+    nbytes = lib().b2r_mesh_adj_scratch_bytes(nv, nf)
+    scratch = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
+    out_v, out_n = torch.empty_like(verts), torch.empty_like(verts)
+    adj = lambda: check(lib().b2r_mesh_adjacency(ptr(faces), nf, nv, ptr(scratch), st), "b2r_mesh_adjacency")  # noqa: E731
+    ms = {}
+    ms["adjacency"], _ = _timed(adj, REPS)
+    ms["iteration"], _ = _timed(lambda: check(lib().b2r_mesh_smooth(ptr(verts), nf, nv, SMOOTH_ITERS, ptr(scratch), ptr(out_v), st),
+                                              "b2r_mesh_smooth"), REPS)
+    ms["iteration"] /= SMOOTH_ITERS
+    ms["normals"], _ = _timed(lambda: check(lib().b2r_mesh_normals(ptr(out_v), nf, nv, ptr(scratch), ptr(out_n), st), "b2r_mesh_normals"),
+                              REPS)
+    nb = smooth_bytes(nv, nf)
+    out = {"iterations": SMOOTH_ITERS, "equals_ops_smooth_mesh": bool(torch.equal(ref_v, out_v) and torch.equal(ref_n, out_n)),
+           "scratch_bytes": int(nbytes), "peak_alloc_bytes_smooth_mesh_call": int(peak)}
+    for k in ("adjacency", "iteration", "normals"):
+        out[f"{k}_ms"] = round(ms[k], 4)
+        out[f"{k}_min_bytes"] = nb[k]
+        out[f"{k}_frac_of_copy_peak"] = round(nb[k] / (ms[k] * 1e-3) / 1e9 / COPY_PEAK_GBS, 3)
+    out["total_ms"] = round(ms["adjacency"] + SMOOTH_ITERS * ms["iteration"] + ms["normals"], 4)
+    del scratch, out_v, out_n
+    return out, ref_v, ref_n
+
+
 NERF_TRUNK_FLOP = 2 * (60 * 256 + 4 * 256 * 256 + 316 * 256 + 2 * 256 * 256 + 256)    # 8-layer trunk + sigma head, per point
 
 
@@ -222,13 +276,26 @@ def nerf_lines():
         cc["create_mesh_filtered_equals_stages"] = bool(torch.equal(whole[0], fv) and torch.equal(whole[1], ff) and torch.equal(whole[2], fn)
                                                         and torch.equal(whole[3], frgb))
         del fv, ff, fn, frgb
+        sm, sv, sn = smooth_times(verts, faces)
+        sm["over_density_query"] = round(sm["total_ms"] / q_ms, 4)
+        srgb = mesh.vertex_colors(net, sv, sn)
+        with tempfile.TemporaryDirectory() as tmp:
+            path = os.path.join(tmp, "mesh.ply")
+            torch.cuda.synchronize()
+            t0 = time.perf_counter()
+            whole = nerf_render.create_mesh(net, path, n, threshold=thr, smooth_iterations=SMOOTH_ITERS)
+            torch.cuda.synchronize()
+            sm["create_mesh_call_smoothed_ms"] = round((time.perf_counter() - t0) * 1e3, 1)
+        sm["create_mesh_smoothed_equals_stages"] = bool(torch.equal(whole[0], sv) and torch.equal(whole[1], faces)
+                                                        and torch.equal(whole[2], sn) and torch.equal(whole[3], srgb))
+        del sv, sn, srgb
         res[str(n)] = {
             "dims": list(field.shape), "points": pts, "density_query_ms": round(q_ms, 3), "points_per_s": round(pts / (q_ms * 1e-3) / 1e9, 3),
             "points_per_s_unit": "G/s", "trunk_TFLOPs": round(pts * NERF_TRUNK_FLOP / (q_ms * 1e-3) / 1e12, 1), "threshold": thr,
             "marching_cubes_device_ms": round(dev_ms, 4), "host_read_VF_ms": round(host_ms, 4), "normals_ms": round(nrm_ms, 4),
             "color_query_ms": round(col_ms, 3), "V": int(verts.shape[0]), "F": int(faces.shape[0]),
             "d2h_plus_ply_ms": round(statistics.median(ts), 2), "ply_bytes": ply_bytes, "create_mesh_call_ms": round(whole_ms, 1),
-            "create_mesh_equals_stages": same, "components": cc}
+            "create_mesh_equals_stages": same, "components": cc, "smoothing": sm}
         del sigma, field, verts, faces, nrm, rgb, whole, scratch
         torch.cuda.empty_cache()
     return res
@@ -247,7 +314,7 @@ def main():
         net.output_layer_sigma[0].weight.mul_(100.0)
         net.output_layer_sigma[0].bias.zero_()
         gen.set_film_params(gen.get_mapping(z)[0])
-    out = {"metric": "create_mesh on the device: density query, marching cubes, connected components, mesh D2H + PLY", "gpu": smi.stdout.strip(),
+    out = {"metric": "create_mesh on the device: density query, marching cubes, connected components, smoothing, mesh D2H + PLY", "gpu": smi.stdout.strip(),
            "copy_peak_GBs": COPY_PEAK_GBS, "sizes": {}}
     for n in (256, 512):
         q_ms, sdf = density_ms(gen, n)
@@ -275,6 +342,8 @@ def main():
         cc = cc_times(verts, faces, None)
         cc["over_density_query"] = round(cc["total_ms"] / q_ms, 4)
         out["sizes"][str(n)]["components"] = cc
+        if n == 512:
+            out["sizes"][str(n)]["smoothing"] = smooth_times(verts, faces)[0]
         del sdf, verts, faces, ref_v, ref_f
         torch.cuda.empty_cache()
     out["nerf_sizes"] = nerf_lines()
