@@ -355,6 +355,30 @@ int b2r_mesh_smooth(const float* verts, long long n_faces, long long n_verts, in
                     void* stream);
 int b2r_mesh_normals(const float* verts, long long n_faces, long long n_verts, const void* scratch, float* normals, void* stream);
 
+/* ---- quadric edge collapse of a triangle mesh (no reference counterpart: size budget of exported meshes) ------------------
+ * Same mesh conventions and PRECONDITION as above.  The rules (frozen vertices, valid edges, placement, cost, selection) are
+ * those of oracle/mesh_decimation.py; every float64 / float32 operation is rounded separately, so the result is reproducible bit
+ * for bit.  quadrics are [V,10] float64 (the upper triangle of the symmetric 4x4, row by row).  adj_scratch is the scratch of
+ * b2r_mesh_adjacency built on the same (faces, n_faces, n_verts); scratch is b2r_mesh_decimate_scratch_bytes(V, F) bytes,
+ * 16-byte aligned (0 for counts outside [0, INT32_MAX]).  Scratch sized for larger counts serves smaller ones.
+ *   b2r_mesh_quadrics:        quadrics[v] = the sum over v's corners in ascending (f, c) of the area-weighted plane quadric of
+ *                             the corner's face.
+ *   b2r_mesh_decimate_round:  selects a set of independent valid edges.  Writes sel_keys[V] (int64): at the smaller end a of a
+ *                             selected edge the float64 bits of its cost (>= 0, so they order like the cost), INT64_MAX
+ *                             everywhere else; counts_dev[0] = the selected edges S, counts_dev[1] = n_faces - 2 S.
+ *   b2r_mesh_decimate_compact: after _round on the same mesh and scratch, collapses the selected edges, or with cut_or_null
+ *                             (int64 [2] on the device: cost bits, a) only those with (sel_keys[a], a) <= cut, and writes the
+ *                             surviving vertices (collapsed survivors at their placement), their quadrics (Q_a + Q_b on
+ *                             collapse) and the surviving faces, remapped, each in its original order.  verts_out / quadrics_out
+ *                             hold V - k rows and faces_out F - 2k, k the number of collapses. */
+size_t b2r_mesh_decimate_scratch_bytes(long long n_verts, long long n_faces);
+int b2r_mesh_quadrics(const float* verts, long long n_faces, long long n_verts, const void* adj_scratch, double* quadrics, void* stream);
+int b2r_mesh_decimate_round(const float* verts, const double* quadrics, long long n_faces, long long n_verts, const void* adj_scratch,
+                            void* scratch, long long* sel_keys, long long* counts_dev, void* stream);
+int b2r_mesh_decimate_compact(const float* verts, const double* quadrics, const int* faces, long long n_faces, long long n_verts,
+                              const long long* sel_keys, const long long* cut_or_null, void* scratch, float* verts_out,
+                              double* quadrics_out, int* faces_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

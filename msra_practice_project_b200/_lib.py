@@ -96,6 +96,12 @@ SIGNATURES = {
     "b2r_mesh_adjacency": (C.c_int, [C.c_void_p, c_ll, c_ll, C.c_void_p, C.c_void_p]),
     "b2r_mesh_smooth": (C.c_int, [c_float_p, c_ll, c_ll, C.c_int, C.c_void_p, c_float_p, C.c_void_p]),
     "b2r_mesh_normals": (C.c_int, [c_float_p, c_ll, c_ll, C.c_void_p, c_float_p, C.c_void_p]),
+    "b2r_mesh_decimate_scratch_bytes": (C.c_size_t, [c_ll, c_ll]),
+    "b2r_mesh_quadrics": (C.c_int, [c_float_p, c_ll, c_ll, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b2r_mesh_decimate_round": (C.c_int, [c_float_p, C.c_void_p, c_ll, c_ll, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                          C.c_void_p]),
+    "b2r_mesh_decimate_compact": (C.c_int, [c_float_p, C.c_void_p, C.c_void_p, c_ll, c_ll, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            c_float_p, C.c_void_p, C.c_void_p, C.c_void_p]),
 }
 
 _lock = threading.Lock()

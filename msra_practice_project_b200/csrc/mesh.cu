@@ -705,6 +705,399 @@ __global__ void __launch_bounds__(kThreads) mesh_normals_kernel(const float* __r
     for (int k = 0; k < 3; ++k) o[k] = len > 0.f ? __fdiv_rn(n[k], len) : 0.f;
 }
 
+// ---- quadric edge collapse (b2r_mesh_quadrics / _decimate_round / _decimate_compact) ------------------------------------------
+// The rules are oracle/mesh_decimation.py's.  One round over the adjacency of the current faces: dec_flags_kernel marks frozen
+// vertices and counts distinct neighbours; dec_key_kernel gives every vertex the smallest key (cost, a, b) of its valid edges and
+// that edge's placement; dec_min_kernel takes the smallest key over each closed neighbourhood; dec_select_kernel keeps an edge
+// iff both ends agree with its key and with both minima.  Compaction marks the surviving vertices and faces per tile and packs
+// their counts the way mc_scan_kernel scans them (as cc_mark_kernel does), then writes them in order.  One thread per vertex and
+// plain loads of the neighbours' keys: the result does not depend on the schedule, and the float64 / float32 values are formed
+// with separately rounded intrinsics.  An edge's key is the ulonglong2 (float64 bits of the cost, a << 32 | b); the cost is >= 0,
+// so comparing (x, y) as unsigned integers is the lexicographic order.
+// Scratch: info[V] (bit 31 frozen, low bits the valence), key[V], m[V] (ulonglong2), part[V] (the partner of a selected vertex or
+// -1), place[V,3] (the placement of the vertex's key edge), vword[V], tile counts and offsets as in cc_layout, totals and cut.
+struct DecLayout {
+    size_t info, key, m, part, place, vword, counts, offsets, totals, total;
+};
+
+inline DecLayout dec_layout(long long n_verts, long long n_faces) {
+    const long long tiles = cc_tiles(n_verts, n_faces);
+    DecLayout l;
+    l.info = 0;
+    l.key = l.info + align256((size_t)n_verts * 4);
+    l.m = l.key + align256((size_t)n_verts * 16);
+    l.part = l.m + align256((size_t)n_verts * 16);
+    l.place = l.part + align256((size_t)n_verts * 4);
+    l.vword = l.place + align256((size_t)n_verts * 12);
+    l.counts = l.vword + align256((size_t)n_verts * 4);
+    l.offsets = l.counts + align256((size_t)tiles * 4);
+    l.totals = l.offsets + align256((size_t)tiles * sizeof(longlong2));
+    l.total = l.totals + 256;
+    return l;
+}
+
+constexpr unsigned kFrozen = 1u << 31;
+constexpr unsigned long long kNoKey = ~0ull;
+constexpr long long kNotSelected = 0x7fffffffffffffffll;
+
+__device__ __forceinline__ bool key_less(ulonglong2 x, ulonglong2 y) { return x.x < y.x || (x.x == y.x && x.y < y.y); }
+__device__ __forceinline__ bool key_eq(ulonglong2 x, ulonglong2 y) { return x.x == y.x && x.y == y.y; }
+
+__device__ __forceinline__ unsigned rec_a(int2 r) { return (unsigned)r.x & kIndexMask; }
+__device__ __forceinline__ unsigned rec_b(int2 r) { return (unsigned)r.y & kIndexMask; }
+
+// Slot s of v's neighbour list: the a (even s) or b (odd s) of record s / 2.
+__device__ __forceinline__ unsigned nb_slot(const int2* __restrict__ adj, unsigned long long beg, unsigned long long s) {
+    const int2 r = adj[beg + s / 2];
+    return s & 1 ? rec_b(r) : rec_a(r);
+}
+
+// Whether slot s holds the first occurrence of its vertex in the list.
+__device__ __forceinline__ bool nb_first(const int2* __restrict__ adj, unsigned long long beg, unsigned long long s, unsigned u) {
+    for (unsigned long long t = 0; t < s; ++t)
+        if (nb_slot(adj, beg, t) == u) return false;
+    return true;
+}
+
+__device__ __forceinline__ bool nb_has(const int2* __restrict__ adj, unsigned long long beg, unsigned long long end, unsigned u) {
+    for (unsigned long long i = beg; i < end; ++i) {
+        const int2 r = adj[i];
+        if (rec_a(r) == u || rec_b(r) == u) return true;
+    }
+    return false;
+}
+
+// The face of record r of vertex v in its own corner order (as mesh_normals_kernel rebuilds it).
+__device__ __forceinline__ void rec_face(int2 r, unsigned v, unsigned (&f)[3]) {
+    const unsigned a = rec_a(r), b = rec_b(r);
+    const unsigned c = (unsigned)r.x >> 31 | ((unsigned)r.y >> 31) << 1;
+    f[0] = c == 0 ? v : c == 1 ? b : a;
+    f[1] = c == 0 ? a : c == 1 ? v : b;
+    f[2] = c == 0 ? b : c == 1 ? a : v;
+}
+
+__device__ __forceinline__ void cross64(const double (&e1)[3], const double (&e2)[3], double (&n)[3]) {
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        const int k1 = (k + 1) % 3, k2 = (k + 2) % 3;
+        n[k] = __dsub_rn(__dmul_rn(e1[k1], e2[k2]), __dmul_rn(e1[k2], e2[k1]));
+    }
+}
+
+__device__ __forceinline__ double dot64(const double (&n)[3], const double (&m)[3]) {
+    return __dadd_rn(__dadd_rn(__dmul_rn(n[0], m[0]), __dmul_rn(n[1], m[1])), __dmul_rn(n[2], m[2]));
+}
+
+// (p1 - p0) x (p2 - p0) in float64 of three float32 points.
+__device__ __forceinline__ void face_normal64(const float* p0, const float* p1, const float* p2, double (&n)[3]) {
+    double e1[3], e2[3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        e1[k] = __dsub_rn((double)p1[k], (double)p0[k]);
+        e2[k] = __dsub_rn((double)p2[k], (double)p0[k]);
+    }
+    cross64(e1, e2, n);
+}
+
+// Sum over v's corners in order of their faces' area-weighted plane quadrics.
+__global__ void __launch_bounds__(kThreads) dec_quadric_kernel(const float* __restrict__ p, unsigned n_verts,
+                                                               const unsigned long long* __restrict__ ends,
+                                                               const int2* __restrict__ adj, double* __restrict__ q) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n_verts) return;
+    const unsigned long long end = ends[v];
+    double s[10];
+#pragma unroll
+    for (int i = 0; i < 10; ++i) s[i] = 0.0;
+    for (unsigned long long i = adj_begin(ends, v); i < end; ++i) {
+        unsigned f[3];
+        rec_face(adj[i], v, f);
+        const float* p0 = p + 3 * (size_t)f[0];
+        double n[3];
+        face_normal64(p0, p + 3 * (size_t)f[1], p + 3 * (size_t)f[2], n);
+        const double len = __dsqrt_rn(dot64(n, n));
+        if (!(len > 0.0)) continue;                                // adds zeros
+        double e[4];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) e[k] = __ddiv_rn(n[k], len);
+        e[3] = -__dadd_rn(__dadd_rn(__dmul_rn(e[0], (double)p0[0]), __dmul_rn(e[1], (double)p0[1])), __dmul_rn(e[2], (double)p0[2]));
+        const double w = __dmul_rn(len, 0.5);
+        int k = 0;
+#pragma unroll
+        for (int r = 0; r < 4; ++r)
+#pragma unroll
+            for (int c = r; c < 4; ++c, ++k) s[k] = __dadd_rn(s[k], __dmul_rn(w, __dmul_rn(e[r], e[c])));
+    }
+    double* o = q + 10 * (size_t)v;
+#pragma unroll
+    for (int i = 0; i < 10; ++i) o[i] = s[i];
+}
+
+// Frozen (listed twice by a face, or an edge on other than two faces) and the number of distinct neighbours.
+__global__ void __launch_bounds__(kThreads) dec_flags_kernel(unsigned n_verts, const unsigned long long* __restrict__ ends,
+                                                             const int2* __restrict__ adj, unsigned* __restrict__ info) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n_verts) return;
+    const unsigned long long beg = adj_begin(ends, v), end = ends[v];
+    unsigned frozen = 0, valence = 0;
+    for (unsigned long long i = beg; i < end; ++i) {
+        const int2 r = adj[i];
+        if (rec_a(r) == v || rec_b(r) == v) frozen = kFrozen;
+    }
+    for (unsigned long long s = 0; s < 2 * (end - beg); ++s) {
+        const unsigned u = nb_slot(adj, beg, s);
+        if (u == v || !nb_first(adj, beg, s, u)) continue;
+        ++valence;
+        unsigned faces = 0;
+        for (unsigned long long i = beg; i < end; ++i) {
+            const int2 r = adj[i];
+            faces += rec_a(r) == u || rec_b(r) == u;
+        }
+        if (faces != 2) frozen = kFrozen;
+    }
+    info[v] = frozen | valence;
+}
+
+// c(p) = p^T Q p over homogeneous p, as the oracle's fixed expression, clamped to 0 when not > 0.
+__device__ __forceinline__ double quadric_cost(const double (&q)[10], const float* x) {
+    const double X = x[0], Y = x[1], Z = x[2];
+    constexpr int idx[4][4] = {{0, 1, 2, 3}, {1, 4, 5, 6}, {2, 5, 7, 8}, {3, 6, 8, 9}};
+    double r[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        r[i] = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(q[idx[i][0]], X), __dmul_rn(q[idx[i][1]], Y)), __dmul_rn(q[idx[i][2]], Z)),
+                         q[idx[i][3]]);
+    const double c = __dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(r[0], X), __dmul_rn(r[1], Y)), __dmul_rn(r[2], Z)), r[3]);
+    return c > 0.0 ? c : 0.0;
+}
+
+// Whether every face around x that does not hold y keeps dot(n_before, n_after) > 0 with x moved to pos.
+__device__ bool dec_no_flip(const float* __restrict__ p, const unsigned long long* __restrict__ ends, const int2* __restrict__ adj,
+                            unsigned x, unsigned y, const float (&pos)[3]) {
+    const unsigned long long end = ends[x];
+    for (unsigned long long i = adj_begin(ends, x); i < end; ++i) {
+        const int2 r = adj[i];
+        if (rec_a(r) == y || rec_b(r) == y) continue;
+        unsigned f[3];
+        rec_face(r, x, f);
+        const float* q0 = p + 3 * (size_t)f[0];
+        const float* q1 = p + 3 * (size_t)f[1];
+        const float* q2 = p + 3 * (size_t)f[2];
+        double nb[3], na[3];
+        face_normal64(q0, q1, q2, nb);
+        face_normal64(f[0] == x ? pos : q0, f[1] == x ? pos : q1, f[2] == x ? pos : q2, na);
+        if (!(dot64(nb, na) > 0.0)) return false;
+    }
+    return true;
+}
+
+__global__ void __launch_bounds__(kThreads) dec_key_kernel(const float* __restrict__ p, const double* __restrict__ q, unsigned n_verts,
+                                                           const unsigned long long* __restrict__ ends, const int2* __restrict__ adj,
+                                                           const unsigned* __restrict__ info, ulonglong2* __restrict__ key,
+                                                           float* __restrict__ place) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n_verts) return;
+    const unsigned iv = info[v];
+    ulonglong2 best = make_ulonglong2(kNoKey, kNoKey);
+    float best_p[3] = {0.f, 0.f, 0.f};
+    const unsigned long long beg = adj_begin(ends, v), end = ends[v];
+    if (!(iv & kFrozen)) {
+        for (unsigned long long s = 0; s < 2 * (end - beg); ++s) {
+            const unsigned u = nb_slot(adj, beg, s);
+            if (!nb_first(adj, beg, s, u)) continue;
+            const unsigned iu = info[u];
+            if ((iu & kFrozen) || (iv & ~kFrozen) + (iu & ~kFrozen) < 7) continue;
+            const unsigned a = min(u, v), b = max(u, v);
+            double qs[10];
+#pragma unroll
+            for (int i = 0; i < 10; ++i) qs[i] = __dadd_rn(q[10 * (size_t)a + i], q[10 * (size_t)b + i]);
+            const float* pa = p + 3 * (size_t)a;
+            const float* pb = p + 3 * (size_t)b;
+            float mid[3], pos[3];
+#pragma unroll
+            for (int k = 0; k < 3; ++k) mid[k] = __fmul_rn(__fadd_rn(pa[k], pb[k]), 0.5f);
+            double c = quadric_cost(qs, pa);
+            const float* pick = pa;
+            const double cb = quadric_cost(qs, pb);
+            if (cb < c) { c = cb; pick = pb; }
+            const double cm = quadric_cost(qs, mid);
+            if (cm < c) { c = cm; pick = mid; }
+            const ulonglong2 k = make_ulonglong2((unsigned long long)__double_as_longlong(c), (unsigned long long)a << 32 | b);
+            if (!key_less(k, best)) continue;                      // cannot lower key(v): its validity does not matter
+            // link condition: the opposite vertices of the edge's two faces differ, and they are the only common neighbours
+            unsigned o[2] = {~0u, ~0u}, no = 0;
+            for (unsigned long long i = beg; i < end; ++i) {
+                const int2 r = adj[i];
+                if (rec_a(r) == u) o[no++ & 1] = rec_b(r);
+                else if (rec_b(r) == u) o[no++ & 1] = rec_a(r);
+            }
+            if (o[0] == o[1]) continue;
+            const unsigned long long ub = adj_begin(ends, u), ue = ends[u];
+            unsigned common = 0;
+            for (unsigned long long t = 0; t < 2 * (end - beg) && common <= 2; ++t) {
+                const unsigned w = nb_slot(adj, beg, t);
+                if (w != u && nb_first(adj, beg, t, w) && nb_has(adj, ub, ue, w)) ++common;
+            }
+            if (common != 2) continue;
+#pragma unroll
+            for (int i = 0; i < 3; ++i) pos[i] = pick[i];
+            if (!dec_no_flip(p, ends, adj, a, b, pos) || !dec_no_flip(p, ends, adj, b, a, pos)) continue;
+            best = k;
+#pragma unroll
+            for (int i = 0; i < 3; ++i) best_p[i] = pos[i];
+        }
+    }
+    key[v] = best;
+#pragma unroll
+    for (int i = 0; i < 3; ++i) place[3 * (size_t)v + i] = best_p[i];
+}
+
+__global__ void __launch_bounds__(kThreads) dec_min_kernel(unsigned n_verts, const unsigned long long* __restrict__ ends,
+                                                           const int2* __restrict__ adj, const ulonglong2* __restrict__ key,
+                                                           ulonglong2* __restrict__ m) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    if (v >= n_verts) return;
+    ulonglong2 best = key[v];
+    const unsigned long long end = ends[v];
+    for (unsigned long long i = adj_begin(ends, v); i < end; ++i) {
+        const int2 r = adj[i];
+        const ulonglong2 ka = key[rec_a(r)], kb = key[rec_b(r)];
+        if (key_less(ka, best)) best = ka;
+        if (key_less(kb, best)) best = kb;
+    }
+    m[v] = best;
+}
+
+// part[v] = the other end of v's selected edge, or -1; sel_keys[a] = the cost bits of a selected edge at its survivor a, kNotSelected
+// everywhere else; *count += the selected edges (warp-aggregated).
+__global__ void __launch_bounds__(kThreads) dec_select_kernel(unsigned n_verts, const ulonglong2* __restrict__ key,
+                                                              const ulonglong2* __restrict__ m, int* __restrict__ part,
+                                                              long long* __restrict__ sel_keys, long long* __restrict__ count) {
+    const unsigned v = blockIdx.x * kThreads + threadIdx.x;
+    bool survivor = false;
+    if (v < n_verts) {
+        const ulonglong2 k = key[v];
+        int partner = -1;
+        if (k.x != kNoKey && key_eq(m[v], k)) {
+            const unsigned a = (unsigned)(k.y >> 32), b = (unsigned)k.y;
+            const unsigned u = v == a ? b : a;
+            if (key_eq(key[u], k) && key_eq(m[u], k)) partner = (int)u;
+        }
+        part[v] = partner;
+        survivor = partner > (int)v;
+        sel_keys[v] = survivor ? (long long)k.x : kNotSelected;
+    }
+    const unsigned votes = __ballot_sync(kFull, survivor);
+    if ((threadIdx.x & (kWarp - 1)) == 0 && votes) atomicAdd((unsigned long long*)count, (unsigned long long)__popc(votes));
+}
+
+__global__ void dec_count_kernel(long long n_faces, long long* __restrict__ counts) { counts[1] = n_faces - 2 * counts[0]; }
+
+// Whether the selected edge at survivor a collapses: every selected edge, or with a cut (cost bits, a) the ones up to it.
+__device__ __forceinline__ bool dec_kept(const int* __restrict__ part, const long long* __restrict__ sel_keys,
+                                         const long long* __restrict__ cut, unsigned a) {
+    if (part[a] <= (int)a) return false;
+    if (!cut) return true;
+    const long long k = sel_keys[a];
+    return k < cut[0] || (k == cut[0] && (long long)a <= cut[1]);
+}
+
+// The survivor vertex u collapses into, or u itself.
+__device__ __forceinline__ unsigned dec_target(const int* __restrict__ part, const long long* __restrict__ sel_keys,
+                                               const long long* __restrict__ cut, unsigned u) {
+    const int t = part[u];
+    return t >= 0 && t < (int)u && dec_kept(part, sel_keys, cut, (unsigned)t) ? (unsigned)t : u;
+}
+
+// A face is deleted iff it holds both ends of a collapsing edge.
+__device__ __forceinline__ bool dec_face_dies(const int* __restrict__ faces, unsigned f, const int* __restrict__ part,
+                                              const long long* __restrict__ sel_keys, const long long* __restrict__ cut) {
+    unsigned t[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) t[c] = (unsigned)faces[3 * (size_t)f + c];
+    bool dies = false;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const unsigned g = dec_target(part, sel_keys, cut, t[c]);
+        dies |= g != t[c] && (g == t[(c + 1) % 3] || g == t[(c + 2) % 3]);
+    }
+    return dies;
+}
+
+__global__ void __launch_bounds__(kThreads) dec_mark_kernel(const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
+                                                            const int* __restrict__ part, const long long* __restrict__ sel_keys,
+                                                            const long long* __restrict__ cut, unsigned* __restrict__ vword,
+                                                            unsigned* __restrict__ tile_counts) {
+    __shared__ unsigned s_scan[kPer * kWarps + 1];
+    const unsigned base = blockIdx.x * (unsigned)kTile;
+    unsigned cnt[kPer], kept = 0;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned idx = base + q * kThreads + threadIdx.x;
+        const unsigned kv = idx < n_verts && dec_target(part, sel_keys, cut, idx) == idx ? 1u : 0u;
+        const unsigned kf = idx < n_faces && !dec_face_dies(faces, idx, part, sel_keys, cut) ? 1u : 0u;
+        kept |= kv << q;
+        cnt[q] = kv | kf << 16;
+    }
+    const unsigned total = tile_scan(cnt, s_scan);
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned idx = base + q * kThreads + threadIdx.x;
+        if (idx < n_verts) vword[idx] = (kept >> q & 1u ? kKept : 0u) | (cnt[q] & 0xffffu);
+    }
+    if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
+}
+
+// Surviving vertices in order (a collapsing survivor at its placement with Q_a + Q_b), surviving faces in order, remapped.
+__global__ void __launch_bounds__(kThreads) dec_compact_kernel(const float* __restrict__ verts, const double* __restrict__ q,
+                                                               const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
+                                                               const int* __restrict__ part, const long long* __restrict__ sel_keys,
+                                                               const long long* __restrict__ cut, const float* __restrict__ place,
+                                                               const unsigned* __restrict__ vword,
+                                                               const longlong2* __restrict__ offsets, float* __restrict__ verts_out,
+                                                               double* __restrict__ q_out, int* __restrict__ faces_out) {
+    __shared__ unsigned s_scan[kPer * kWarps + 1];
+    const unsigned base = blockIdx.x * (unsigned)kTile;
+    const longlong2 off = offsets[blockIdx.x];
+#pragma unroll 1
+    for (int q8 = 0; q8 < kPer; ++q8) {
+        const unsigned v = base + q8 * kThreads + threadIdx.x;
+        if (v >= n_verts) break;
+        const unsigned w = vword[v];
+        if (!(w & kKept)) continue;
+        const size_t to = (size_t)(off.x + (w & 0xffffu));
+        const bool moves = dec_kept(part, sel_keys, cut, v);
+        const float* from = (moves ? place : verts) + 3 * (size_t)v;
+#pragma unroll
+        for (int c = 0; c < 3; ++c) verts_out[3 * to + c] = from[c];
+        const double* qa = q + 10 * (size_t)v;
+        const double* qb = q + 10 * (size_t)(moves ? part[v] : 0);
+#pragma unroll
+        for (int i = 0; i < 10; ++i) q_out[10 * to + i] = moves ? __dadd_rn(qa[i], qb[i]) : qa[i];
+    }
+    unsigned cnt[kPer];
+#pragma unroll
+    for (int k = 0; k < kPer; ++k) {
+        const unsigned f = base + k * kThreads + threadIdx.x;
+        cnt[k] = f < n_faces && !dec_face_dies(faces, f, part, sel_keys, cut) ? 1u : 0u;
+    }
+    unsigned kept = 0;
+#pragma unroll
+    for (int k = 0; k < kPer; ++k) kept |= cnt[k] << k;
+    tile_scan(cnt, s_scan);
+#pragma unroll
+    for (int k = 0; k < kPer; ++k) {
+        if (!(kept >> k & 1u)) continue;
+        const unsigned f = base + k * kThreads + threadIdx.x;
+        int* out = faces_out + 3 * (off.y + cnt[k]);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const unsigned u = dec_target(part, sel_keys, cut, (unsigned)faces[3 * (size_t)f + c]);
+            out[c] = (int)(offsets[u / kTile].x + (vword[u] & 0xffffu));
+        }
+    }
+}
+
 int check_grid(const char* what, int n0, int n1, int n2) {
     B2R_CHECK_ARG(n0 >= 2 && n1 >= 2 && n2 >= 2, "%s: every axis needs n >= 2 (got %d x %d x %d)", what, n0, n1, n2);
     B2R_CHECK_ARG((long long)n0 * n1 * n2 <= INT32_MAX, "%s: n0*n1*n2 = %lld exceeds INT32_MAX", what, (long long)n0 * n1 * n2);
@@ -936,6 +1329,88 @@ extern "C" int b2r_mesh_normals(const float* verts, long long n_faces, long long
     const char* s = static_cast<const char*>(scratch);
     mesh_normals_kernel<<<blocks_of(n_verts, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
         verts, (unsigned)n_verts, (const unsigned long long*)(s + l.ends), (const int2*)(s + l.adj), normals);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" size_t b2r_mesh_decimate_scratch_bytes(long long n_verts, long long n_faces) {
+    if (n_verts < 0 || n_verts > INT32_MAX || n_faces < 0 || n_faces > INT32_MAX) return 0;
+    return b2r::mc::dec_layout(n_verts, n_faces).total;
+}
+
+extern "C" int b2r_mesh_quadrics(const float* verts, long long n_faces, long long n_verts, const void* adj_scratch, double* quadrics,
+                                 void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_quadrics";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG((verts && quadrics) || !n_verts, "%s: NULL verts / quadrics with n_verts > 0", what);
+    if (!n_verts) return 0;
+    if (int rc = check_scratch(what, adj_scratch)) return rc;
+    const AdjLayout l = adj_layout(n_verts, n_faces);
+    const char* s = static_cast<const char*>(adj_scratch);
+    dec_quadric_kernel<<<blocks_of(n_verts, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
+        verts, (unsigned)n_verts, (const unsigned long long*)(s + l.ends), (const int2*)(s + l.adj), quadrics);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_decimate_round(const float* verts, const double* quadrics, long long n_faces, long long n_verts,
+                                       const void* adj_scratch, void* scratch, long long* sel_keys, long long* counts_dev,
+                                       void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_decimate_round";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG(counts_dev, "%s: NULL counts_dev", what);
+    B2R_CHECK_ARG((verts && quadrics && sel_keys) || !n_verts, "%s: NULL verts / quadrics / sel_keys with n_verts > 0", what);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = b2r::cuda_result(cudaMemsetAsync(counts_dev, 0, 8, st), what)) return rc;
+    if (n_verts) {
+        if (int rc = check_scratch(what, adj_scratch)) return rc;
+        if (int rc = check_scratch(what, scratch)) return rc;
+        const AdjLayout al = adj_layout(n_verts, n_faces);
+        const DecLayout l = dec_layout(n_verts, n_faces);
+        const char* a = static_cast<const char*>(adj_scratch);
+        char* s = static_cast<char*>(scratch);
+        const unsigned long long* ends = (const unsigned long long*)(a + al.ends);
+        const int2* adj = (const int2*)(a + al.adj);
+        unsigned* info = (unsigned*)(s + l.info);
+        ulonglong2* key = (ulonglong2*)(s + l.key);
+        ulonglong2* m = (ulonglong2*)(s + l.m);
+        const unsigned nv = (unsigned)n_verts, blocks = blocks_of(nv, kThreads);
+        dec_flags_kernel<<<blocks, kThreads, 0, st>>>(nv, ends, adj, info);
+        dec_key_kernel<<<blocks, kThreads, 0, st>>>(verts, quadrics, nv, ends, adj, info, key, (float*)(s + l.place));
+        dec_min_kernel<<<blocks, kThreads, 0, st>>>(nv, ends, adj, key, m);
+        dec_select_kernel<<<blocks, kThreads, 0, st>>>(nv, key, m, (int*)(s + l.part), sel_keys, counts_dev);
+    }
+    dec_count_kernel<<<1, 1, 0, st>>>(n_faces, counts_dev);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_decimate_compact(const float* verts, const double* quadrics, const int* faces, long long n_faces,
+                                         long long n_verts, const long long* sel_keys, const long long* cut_or_null, void* scratch,
+                                         float* verts_out, double* quadrics_out, int* faces_out, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_decimate_compact";
+    if (int rc = check_counts(what, n_faces, n_verts)) return rc;
+    B2R_CHECK_ARG((faces && faces_out) || !n_faces, "%s: NULL faces / faces_out with n_faces > 0", what);
+    B2R_CHECK_ARG((verts && quadrics && sel_keys && verts_out && quadrics_out) || !n_verts,
+                  "%s: NULL verts / quadrics / sel_keys / verts_out / quadrics_out with n_verts > 0", what);
+    if (!n_verts) return 0;
+    if (int rc = check_scratch(what, scratch)) return rc;
+    const DecLayout l = dec_layout(n_verts, n_faces);
+    const int tiles = (int)cc_tiles(n_verts, n_faces);
+    char* s = static_cast<char*>(scratch);
+    const int* part = (const int*)(s + l.part);
+    unsigned* vword = (unsigned*)(s + l.vword);
+    longlong2* offsets = (longlong2*)(s + l.offsets);
+    cudaStream_t st = (cudaStream_t)stream;
+    dec_mark_kernel<<<tiles, kThreads, 0, st>>>(faces, (unsigned)n_faces, (unsigned)n_verts, part, sel_keys, cut_or_null, vword,
+                                                (unsigned*)(s + l.counts));
+    mc_scan_kernel<<<1, kScanThreads, 0, st>>>((const unsigned*)(s + l.counts), tiles, offsets, (long long*)(s + l.totals));
+    dec_compact_kernel<<<tiles, kThreads, 0, st>>>(verts, quadrics, faces, (unsigned)n_faces, (unsigned)n_verts, part, sel_keys,
+                                                   cut_or_null, (const float*)(s + l.place), vword, offsets, verts_out, quadrics_out,
+                                                   faces_out);
     B2R_LAUNCH_CHECK(what);
     return 0;
 }

@@ -81,21 +81,29 @@ def write_ply(filename, verts, faces, normals=None, colors=None):
 
 
 def export(model, field, level, spacing, origin, ply_filename, normals, colors, precision, min_component_ratio=0.0,
-           smooth_iterations=0):
+           smooth_iterations=0, max_faces=None):
     """Extract the level set of ``field`` (vertex normals toward increasing field), colour it with ``model`` and write the PLY.
     Returns (verts, faces, normals | None, colors | None) on the device.  A ``min_component_ratio`` above 0 removes the
     components with fewer triangles than that share of the largest one (ops.filter_components) before the colour query, so
     dropped vertices cost no MLP rows; it synchronises with the host once more, to size the filtered mesh.
     ``smooth_iterations`` above 0 then runs that many Taubin iterations (ops.smooth_mesh) before the colour query, and the
-    normals become the smoothed mesh's own, so colours are sampled on the smoothed surface; the field normals are not computed."""
+    normals become the smoothed mesh's own, so colours are sampled on the smoothed surface; the field normals are not computed.
+    ``max_faces`` (an int >= 1) then decimates the mesh to that many triangles (ops.decimate_mesh; one host synchronisation per
+    round) before the colour query, so removed vertices cost no MLP rows, and the normals are the decimated mesh's own."""
     iterations = ops._check_iterations(smooth_iterations)
+    budget = None if max_faces is None else ops._check_max_faces(max_faces)
     want_normals = normals or colors
-    verts, faces, nrm = extract(field, level, spacing, origin, want_normals and not iterations)
+    own_normals = want_normals and (iterations or budget is not None)
+    verts, faces, nrm = extract(field, level, spacing, origin, want_normals and not own_normals)
     if min_component_ratio:
         # marching-cubes faces index their own vertices, so the index checks of ops.filter_components / ops.smooth_mesh are not needed
         verts, faces, nrm = ops._filter_components(verts, faces, ops._check_ratio(min_component_ratio), nrm)
     if iterations:
-        verts, nrm = ops._smooth_mesh(verts, faces, iterations, want_normals)
+        verts, nrm = ops._smooth_mesh(verts, faces, iterations, want_normals and budget is None)
+    if budget is not None:
+        verts, faces = ops._decimate_mesh(verts, faces, budget)
+        if want_normals:
+            verts, nrm = ops._smooth_mesh(verts, faces, 0, True)
     rgb = vertex_colors(model, verts, nrm, precision) if colors else None
     if not normals:
         nrm = None

@@ -309,7 +309,8 @@ def density_lattice(model, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), 
 
 
 def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), threshold=50.0,
-                normals=True, colors=True, precision=None, max_batch=256 ** 3, min_component_ratio=0.0, smooth_iterations=0):
+                normals=True, colors=True, precision=None, max_batch=256 ** 3, min_component_ratio=0.0, smooth_iterations=0,
+                max_faces=None):
     """Mesh of a trained NeRF / SirenNeRF field on the device: the level set ``sigma = threshold`` of ``density_lattice``
     (marching cubes on -sigma at -threshold, so triangle and vertex normals point out of the object, toward lower density),
     the unit vertex normals, and the uint8 colour the model's rgb head gives each vertex seen by a camera looking along the
@@ -324,7 +325,13 @@ def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), 
     filter and before the colour query (ops.smooth_mesh): the terraces marching cubes leaves where the density rises steeply
     through ``threshold`` are smoothed out without shrinking the surface, and the topology is unchanged.  The normals are then
     the smoothed mesh's own area-weighted vertex normals (still out of the object) and the colours are sampled at the smoothed
-    vertices along them; no host synchronisation is added.  0 (the default) leaves the mesh as extracted."""
+    vertices along them; no host synchronisation is added.  0 (the default) leaves the mesh as extracted.
+    ``max_faces`` (an int >= 1) decimates the mesh to that many triangles (or one fewer) after the component filter and the
+    smoothing and before the colour query (ops.decimate_mesh: rounds of quadric edge collapses that keep the topology, leave
+    the open boundary where the surface meets the lattice box in place and never flip a face), so removed vertices cost no MLP
+    rows.  The normals are then the decimated mesh's own area-weighted vertex normals (still out of the object) and the
+    colours are sampled at the decimated vertices along them; the field normals are not computed.  Each round synchronises
+    with the host once, to read its collapse count.  None (the default) leaves the mesh at its extracted size."""
     sigma, origin, voxel = density_lattice(model, box_min, box_max, N, max_batch=max_batch, precision=precision)
     return mesh.export(model, sigma.neg_(), -float(threshold), voxel, origin, ply_filename, normals, colors, precision,
-                       min_component_ratio, smooth_iterations)
+                       min_component_ratio, smooth_iterations, max_faces)

@@ -965,3 +965,77 @@ def smooth_mesh(verts: torch.Tensor, faces: torch.Tensor, iterations: int, *, no
         raise RuntimeError("verts and faces must be on the same device")
     out, nrm = _smooth_mesh(verts, faces, iterations, normals)
     return (out, nrm) if normals else out
+
+
+def _check_max_faces(max_faces) -> int:
+    if isinstance(max_faces, bool) or not isinstance(max_faces, (int, np.integer)) or not 1 <= max_faces:
+        raise ValueError(f"max_faces must be an int >= 1, got {max_faces!r}")
+    return int(max_faces)
+
+
+def _decimate_mesh(verts: torch.Tensor, faces: torch.Tensor, max_faces: int, stats: dict | None = None):
+    """decimate_mesh for faces already known to index [0, V): one host read of the round's counts per round."""
+    dev, n_verts, n_faces = verts.device, verts.shape[0], faces.shape[0]
+    if max_faces >= n_faces:
+        return verts, faces
+    rounds = []
+    with torch.cuda.device(dev):
+        st = _stream(verts)
+        # sized for the input mesh: every round's mesh is smaller and lays its scratch out from the start
+        adj = torch.empty((lib().b2r_mesh_adj_scratch_bytes(n_verts, n_faces),), dtype=torch.uint8, device=dev)
+        scratch = torch.empty((lib().b2r_mesh_decimate_scratch_bytes(n_verts, n_faces),), dtype=torch.uint8, device=dev)
+        sel_keys = torch.empty((n_verts,), dtype=torch.int64, device=dev)
+        counts = torch.empty((2,), dtype=torch.int64, device=dev)
+        check(lib().b2r_mesh_adjacency(ptr(faces), n_faces, n_verts, ptr(adj), st), "b2r_mesh_adjacency")
+        quadrics = torch.empty((n_verts, 10), dtype=torch.float64, device=dev)
+        check(lib().b2r_mesh_quadrics(ptr(verts), n_faces, n_verts, ptr(adj), ptr(quadrics), st), "b2r_mesh_quadrics")
+        while n_faces > max_faces:
+            if rounds:
+                check(lib().b2r_mesh_adjacency(ptr(faces), n_faces, n_verts, ptr(adj), st), "b2r_mesh_adjacency")
+            check(lib().b2r_mesh_decimate_round(ptr(verts), ptr(quadrics), n_faces, n_verts, ptr(adj), ptr(scratch), ptr(sel_keys),
+                                                ptr(counts), st), "b2r_mesh_decimate_round")
+            selected = int(counts[0])
+            if not selected:
+                break
+            cut = None
+            budget = (n_faces - max_faces + 1) // 2
+            if selected > budget:
+                # the budget's cheapest selected edges: (cost bits, a) of the last one, read on the device by the compaction
+                keys = sel_keys[:n_verts]
+                last = torch.sort(keys, stable=True).indices[budget - 1]
+                cut = torch.stack([keys[last], last])
+                selected = budget
+            v_out = torch.empty((n_verts - selected, 3), dtype=torch.float32, device=dev)
+            q_out = torch.empty((n_verts - selected, 10), dtype=torch.float64, device=dev)
+            f_out = torch.empty((n_faces - 2 * selected, 3), dtype=torch.int32, device=dev)
+            check(lib().b2r_mesh_decimate_compact(ptr(verts), ptr(quadrics), ptr(faces), n_faces, n_verts, ptr(sel_keys), ptr(cut),
+                                                  ptr(scratch), ptr(v_out), ptr(q_out), ptr(f_out), st), "b2r_mesh_decimate_compact")
+            verts, quadrics, faces = v_out, q_out, f_out
+            n_verts, n_faces = n_verts - selected, n_faces - 2 * selected
+            rounds.append(selected)
+    if stats is not None:
+        stats["rounds"] = len(rounds)
+        stats["collapses"] = rounds
+    return verts, faces
+
+
+def decimate_mesh(verts: torch.Tensor, faces: torch.Tensor, max_faces: int):
+    """Quadric edge collapse of a triangle mesh on the device down to ``max_faces`` triangles (b2r_mesh_adjacency / _quadrics /
+    _decimate_round / _decimate_compact).  Rounds of independent collapses preserve the topology: closed stays closed, genus
+    and components do not change, no non-manifold edge appears and no face flips.  Vertices on an open boundary (an edge on one
+    face) or on non-manifold input never move.  Each round collapses the edges that are the cheapest (area-weighted plane
+    quadrics, placement at either end or the midpoint) within both ends' neighbourhoods; the round that would pass the budget
+    collapses only its cheapest ones, so the result has ``max_faces`` or ``max_faces - 1`` triangles unless no edge can
+    collapse first.  Surviving vertices and faces keep their order.  Returns ``(verts' [V',3] float32, faces' [F',3] int32)``,
+    equal to ``oracle.mesh_decimation.decimate``.  ``max_faces`` must be an int >= 1 (ValueError).  Checks that ``faces`` is
+    [F,3] int32 on the device with every index in [0, V) (RuntimeError otherwise, before any launch; one host
+    synchronisation); ``max_faces >= F`` then returns the inputs without a launch.  Every round synchronises once more to read
+    its collapse count."""
+    max_faces = _check_max_faces(max_faces)
+    verts = _cuda_f32(verts, "verts")
+    if verts.dim() != 2 or verts.shape[1] != 3:
+        raise RuntimeError(f"verts must be [V,3], got {list(verts.shape)}")
+    faces = _mesh_faces(faces, verts.shape[0])
+    if faces.device != verts.device:
+        raise RuntimeError("verts and faces must be on the same device")
+    return _decimate_mesh(verts, faces, max_faces)

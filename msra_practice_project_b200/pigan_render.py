@@ -185,7 +185,7 @@ def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=No
 
 
 def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None, normals=False,
-                colors=False, min_component_ratio=0.0, smooth_iterations=0):
+                colors=False, min_component_ratio=0.0, smooth_iterations=0, max_faces=None):
     """``create_mesh`` (pi_GAN/utils.py:42-180) on the device: the sdf of ``create_mesh_sdf`` never leaves the GPU,
     ``ops.marching_cubes`` extracts its level set (the reference's skimage call at level -20: below = sigma > 20, so the
     triangle normals point out of the object), and only the mesh crosses to the host.  Returns ``(verts [V,3] float32,
@@ -203,8 +203,14 @@ def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level
     filter and before the colour query (ops.smooth_mesh): the terraces marching cubes leaves along the lattice are smoothed
     out without moving the surface inward, and the topology is unchanged.  The normals are then the smoothed mesh's own
     area-weighted vertex normals and the colours are sampled at the smoothed vertices; no host synchronisation is added.
-    0 (the default) leaves the mesh as extracted."""
+    0 (the default) leaves the mesh as extracted.
+    ``max_faces`` (an int >= 1) decimates the mesh to that many triangles (or one fewer) after the component filter and the
+    smoothing and before the colour query (ops.decimate_mesh: rounds of quadric edge collapses that keep the topology, leave
+    the open boundary where the surface meets the lattice box in place and never flip a face), so removed vertices cost no MLP
+    rows.  The normals are then the decimated mesh's own area-weighted vertex normals (still out of the object) and the
+    colours are sampled at the decimated vertices along them; the field normals are not computed.  Each round synchronises
+    with the host once, to read its collapse count.  None (the default) leaves the mesh at its extracted size."""
     sdf = _sdf_device(generator, N, max_batch, z, precision)
     out = _export_mesh(generator.film_siren_nerf, sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1), ply_filename, normals, colors,
-                       precision, min_component_ratio, smooth_iterations)
+                       precision, min_component_ratio, smooth_iterations, max_faces)
     return out if (normals or colors) else out[:2]

@@ -22,7 +22,15 @@ b2r_mesh_smooth call of SMOOTH_ITERS iterations divided by SMOOTH_ITERS, b2r_mes
 warm-up): ms per stage, the least bytes each stage moves (smooth_bytes) against the copy peak, the scratch bytes and the peak of
 torch's allocator over one ops.smooth_mesh(normals=True) call above what was allocated before it, and a check against that call.
 For the NeRF meshes also one whole create_mesh(smooth_iterations=SMOOTH_ITERS) call against the unsmoothed one above, and whether
-it equals its stages (ops.smooth_mesh, then the colour query)."""
+it equals its stages (ops.smooth_mesh, then the colour query).
+
+The "decimation" entries (``--decimation`` runs only these) time ops.decimate_mesh on the pi-GAN 512^3 mesh down to 25,000 faces
+and on the NeRF 512^3 mesh down to 1,000,000: the number of rounds and the collapses of each, the wall time of the whole call
+(host clock around a call that ends in a device synchronise; it includes the one host read per round) and its mean per round,
+and the peak of torch's allocator over the call above what was allocated before it.  For the NeRF mesh also one whole
+create_mesh(max_faces=1_000_000) call against create_mesh() on the same field, each split into the call without a PLY (device
+work and the host reads) and the D2H copy + PLY write of its outputs, and whether the decimated call equals its stages
+(ops.decimate_mesh, the mesh normals, the colour query)."""
 import json
 import os
 import statistics
@@ -301,6 +309,76 @@ def nerf_lines():
     return res
 
 
+DEC_PIGAN, DEC_NERF = 25_000, 1_000_000
+
+
+def decimate_times(verts, faces, max_faces):
+    """Rounds, wall ms of one ops.decimate_mesh call (and per round), allocator peak above the inputs, (V', F')."""
+    dev = verts.device
+    ops._decimate_mesh(verts, faces, max_faces)                  # warm-up
+    torch.cuda.synchronize()
+    base = torch.cuda.memory_allocated(dev)
+    torch.cuda.reset_peak_memory_stats(dev)
+    stats = {}
+    t0 = time.perf_counter()
+    dv, df = ops._decimate_mesh(verts, faces, max_faces, stats)
+    torch.cuda.synchronize()
+    ms = (time.perf_counter() - t0) * 1e3
+    peak = torch.cuda.max_memory_allocated(dev) - base
+    again = ops._decimate_mesh(verts, faces, max_faces)
+    return {"V": int(verts.shape[0]), "F": int(faces.shape[0]), "max_faces": max_faces, "V_out": int(dv.shape[0]), "F_out": int(df.shape[0]),
+            "rounds": stats["rounds"], "collapses_per_round": stats["collapses"], "call_ms": round(ms, 2),
+            "mean_ms_per_round": round(ms / max(1, stats["rounds"]), 3), "peak_alloc_bytes": int(peak),
+            "repeat_run_identical": bool(torch.equal(again[0], dv) and torch.equal(again[1], df))}, dv, df
+
+
+def _call_split(fn, path):
+    """(ms of fn(None) ended by a device synchronise, ms of the D2H copy + PLY write of its outputs, the outputs)."""
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    out = fn(None)
+    torch.cuda.synchronize()
+    dev_ms = (time.perf_counter() - t0) * 1e3
+    t0 = time.perf_counter()
+    mesh.write_ply(path, *(t.cpu().numpy() for t in out))
+    return dev_ms, (time.perf_counter() - t0) * 1e3, out
+
+
+def decimation_lines(gen):
+    res = {}
+    sdf = pigan_render.density_grid(gen.film_siren_nerf, N=512).reshape(512, 512, 512)
+    verts, faces = ops.marching_cubes(sdf, -20.0, 0.2 / 511, (-0.1, -0.1, -0.1))
+    res["pigan_512"] = decimate_times(verts, faces, DEC_PIGAN)[0]
+    del sdf, verts, faces
+    torch.manual_seed(0)
+    net = models.NeRF().cuda()
+    with torch.no_grad():
+        net.output_layer_sigma.weight.mul_(100.0)
+        net.output_layer_sigma.bias.zero_()
+    sigma, origin, voxel = nerf_render.density_lattice(net, N=512)
+    thr = float(torch.quantile(sigma.flatten()[::97].float(), 0.7))
+    verts, faces = ops.marching_cubes(-sigma, -thr, voxel, origin)
+    del sigma
+    torch.cuda.empty_cache()
+    d, dv, df = decimate_times(verts, faces, DEC_NERF)
+    del verts, faces
+    with tempfile.TemporaryDirectory() as tmp:
+        path = os.path.join(tmp, "mesh.ply")
+        for name, kw in (("none", {}), ("max_faces", {"max_faces": DEC_NERF})):
+            dev_ms, ply_ms, out = _call_split(lambda p: nerf_render.create_mesh(net, p, 512, threshold=thr, **kw), path)
+            d[f"create_mesh_{name}_no_ply_ms"] = round(dev_ms, 1)
+            d[f"create_mesh_{name}_d2h_plus_ply_ms"] = round(ply_ms, 1)
+            d[f"create_mesh_{name}_ply_bytes"] = os.path.getsize(path)
+            if name == "max_faces":
+                _, dn = ops.smooth_mesh(dv, df, 0, normals=True)
+                rgb = mesh.vertex_colors(net, dv, dn)
+                d["create_mesh_max_faces_equals_stages"] = bool(all(torch.equal(a, b) for a, b in zip(out, (dv, df, dn, rgb))))
+            del out
+            torch.cuda.empty_cache()
+    res["nerf_512"] = d
+    return res
+
+
 def main():
     smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
     print("gpu:", smi.stdout.strip().splitlines()[0] if smi.returncode == 0 and smi.stdout.strip() else "unknown")
@@ -314,6 +392,9 @@ def main():
         net.output_layer_sigma[0].weight.mul_(100.0)
         net.output_layer_sigma[0].bias.zero_()
         gen.set_film_params(gen.get_mapping(z)[0])
+    if "--decimation" in sys.argv[1:]:
+        print(json.dumps({"metric": "mesh decimation on the device", "gpu": smi.stdout.strip(), "decimation": decimation_lines(gen)}))
+        return
     out = {"metric": "create_mesh on the device: density query, marching cubes, connected components, smoothing, mesh D2H + PLY", "gpu": smi.stdout.strip(),
            "copy_peak_GBs": COPY_PEAK_GBS, "sizes": {}}
     for n in (256, 512):
@@ -347,6 +428,7 @@ def main():
         del sdf, verts, faces, ref_v, ref_f
         torch.cuda.empty_cache()
     out["nerf_sizes"] = nerf_lines()
+    out["decimation"] = decimation_lines(gen)
     # the numpy oracle at 128^3, host only, for scale
     sdf = pigan_render.density_grid(gen.film_siren_nerf, N=128).reshape(128, 128, 128).cpu().numpy()
     t0 = time.perf_counter()
