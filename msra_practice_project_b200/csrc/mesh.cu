@@ -286,31 +286,123 @@ __global__ void __launch_bounds__(kThreads) mc_faces_kernel(int n0, int n1, int 
 // its only root once every union is done, and the labels (root of each vertex) are the minimum-index labels whatever the
 // schedule.  Selection counts the faces per label (warp-aggregated: faces arrive in lattice order, so one dominant component
 // would otherwise serialise nearly every atomic on one address), takes their integer maximum and marks what is kept.
-// Compaction writes the kept vertices and faces in their relative order, no sort and no atomics.
+// Compaction (mark_kernel, compact_kernel, shared with the edge collapse) writes the kept vertices and faces in their relative
+// order, no sort and no atomics.
 //
-// Scratch: a[V] (the parent array while labelling, triangle counts per label while selecting), vword[V] (bit 31 = kept, bits
-// 0..15 = rank of the vertex among the kept ones of its tile), tile counts and offsets as in marching cubes, and the maximum.
-// Tile b covers vertices AND faces [b*kTile, +kTile): its kept-vertex and kept-face counts are the two 16-bit fields
-// mc_scan_kernel expects, so the scan writes (V', F') and every tile's (first vertex, first face).
-struct CcLayout {
-    size_t a, vword, counts, offsets, max, total;
+// Scratch: a[V] (the parent array while labelling, triangle counts per label while selecting), then the compaction tail, whose
+// last 256 bytes hold the maximum.
+
+// The end of every compaction scratch, from byte `at`: vword[V], tile counts and offsets as in marching cubes, and 256 bytes
+// that the caller uses for its own device scalars.
+struct CompactTail {
+    size_t vword, counts, offsets, last, total;
 };
 
-inline long long cc_tiles(long long n_verts, long long n_faces) { return ((n_verts > n_faces ? n_verts : n_faces) + kTile - 1) / kTile; }
+inline long long compact_tiles(long long n_verts, long long n_faces) {
+    return ((n_verts > n_faces ? n_verts : n_faces) + kTile - 1) / kTile;
+}
+
+inline CompactTail compact_tail(size_t at, long long n_verts, long long n_faces) {
+    const long long tiles = compact_tiles(n_verts, n_faces);
+    CompactTail t;
+    t.vword = at;
+    t.counts = t.vword + align256((size_t)n_verts * 4);
+    t.offsets = t.counts + align256((size_t)tiles * 4);
+    t.last = t.offsets + align256((size_t)tiles * sizeof(longlong2));
+    t.total = t.last + 256;
+    return t;
+}
+
+struct CcLayout {
+    size_t a;
+    CompactTail tail;
+};
 
 inline CcLayout cc_layout(long long n_verts, long long n_faces) {
-    const long long tiles = cc_tiles(n_verts, n_faces);
     CcLayout l;
     l.a = 0;
-    l.vword = l.a + align256((size_t)n_verts * 4);
-    l.counts = l.vword + align256((size_t)n_verts * 4);
-    l.offsets = l.counts + align256((size_t)tiles * 4);
-    l.max = l.offsets + align256((size_t)tiles * sizeof(longlong2));
-    l.total = l.max + 256;
+    l.tail = compact_tail(l.a + align256((size_t)n_verts * 4), n_verts, n_faces);
     return l;
 }
 
+// vword per vertex: bit 31 = kept, bits 0..15 = rank of the vertex among the kept ones of its tile.  Tile b covers vertices AND
+// faces [b*kTile, +kTile): its kept-vertex and kept-face counts are the two 16-bit fields mc_scan_kernel expects, so the scan
+// writes (V', F') and every tile's (first vertex, first face).
 constexpr unsigned kKept = 1u << 31;
+
+// Keep: __device__ bool vert(unsigned v) const and bool face(unsigned f) const, whether vertex v / face f survives.
+// Keep and Emit carry their pointers as struct members, where __restrict__ has no effect, so their read-only loads use __ldg: that
+// keeps them on the read-only path and lets them be issued ahead of the stores of compact_kernel.
+template <class Keep>
+__global__ void __launch_bounds__(kThreads) mark_kernel(Keep keep, unsigned n_faces, unsigned n_verts, unsigned* __restrict__ vword,
+                                                        unsigned* __restrict__ tile_counts) {
+    __shared__ unsigned s_scan[kPer * kWarps + 1];
+    const unsigned base = blockIdx.x * (unsigned)kTile;
+    unsigned cnt[kPer], kept = 0;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned idx = base + q * kThreads + threadIdx.x;
+        const unsigned kv = idx < n_verts && keep.vert(idx) ? 1u : 0u;
+        const unsigned kf = idx < n_faces && keep.face(idx) ? 1u : 0u;
+        kept |= kv << q;
+        cnt[q] = kv | kf << 16;
+    }
+    const unsigned total = tile_scan(cnt, s_scan);
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned idx = base + q * kThreads + threadIdx.x;
+        if (idx < n_verts) vword[idx] = (kept >> q & 1u ? kKept : 0u) | (cnt[q] & 0xffffu);
+    }
+    if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
+}
+
+// Kept vertex v goes to offsets[v / kTile].x + its rank; a kept face goes to its tile's first face + its rank among the tile's
+// kept faces, each index u replaced by the kept vertex it maps to.  Emit: __device__ void vert(unsigned v, size_t to) const writes
+// kept vertex v's payload as output vertex `to`; bool face(unsigned f, const unsigned (&t)[3]) const, whether face f with indices t
+// survives; unsigned target(unsigned u) const, the kept vertex index u maps to.
+template <class Emit>
+__global__ void __launch_bounds__(kThreads) compact_kernel(Emit emit, const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
+                                                           const unsigned* __restrict__ vword, const longlong2* __restrict__ offsets,
+                                                           int* __restrict__ faces_out) {
+    __shared__ unsigned s_scan[kPer * kWarps + 1];
+    const unsigned base = blockIdx.x * (unsigned)kTile;
+    const longlong2 off = offsets[blockIdx.x];
+#pragma unroll 2
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned v = base + q * kThreads + threadIdx.x;
+        if (v >= n_verts) break;
+        const unsigned w = vword[v];
+        if (w & kKept) emit.vert(v, (size_t)(off.x + (w & 0xffffu)));
+    }
+    // The face indices are read again for the remap rather than held across tile_scan: holding all kPer * 3 of them takes
+    // both instantiations to 64 registers (48 for DecEmit this way), one resident CTA per SM fewer.
+    unsigned cnt[kPer];
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        const unsigned f = base + q * kThreads + threadIdx.x;
+        cnt[q] = 0;
+        if (f >= n_faces) continue;
+        unsigned t[3];
+#pragma unroll
+        for (int c = 0; c < 3; ++c) t[c] = (unsigned)faces[3 * (size_t)f + c];
+        cnt[q] = emit.face(f, t) ? 1u : 0u;
+    }
+    unsigned kept = 0;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) kept |= cnt[q] << q;
+    tile_scan(cnt, s_scan);
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) {
+        if (!(kept >> q & 1u)) continue;
+        const unsigned f = base + q * kThreads + threadIdx.x;
+        int* out = faces_out + 3 * (off.y + cnt[q]);
+#pragma unroll
+        for (int c = 0; c < 3; ++c) {
+            const unsigned u = emit.target((unsigned)faces[3 * (size_t)f + c]);
+            out[c] = (int)(offsets[u / kTile].x + (vword[u] & 0xffffu));
+        }
+    }
+}
 
 __global__ void cc_init_kernel(unsigned* __restrict__ parent, unsigned n_verts) {
     const unsigned v = blockIdx.x * blockDim.x + threadIdx.x;
@@ -384,81 +476,35 @@ __device__ __forceinline__ unsigned cc_keep(unsigned t, float ratio, unsigned t_
     return ratio == 0.f || (t > 0 && (double)t >= __dmul_rn((double)ratio, (double)t_max)) ? 1u : 0u;
 }
 
-__global__ void __launch_bounds__(kThreads) cc_mark_kernel(const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
-                                                           const int* __restrict__ labels, const unsigned* __restrict__ tri,
-                                                           const unsigned* __restrict__ t_max_p, float ratio,
-                                                           unsigned* __restrict__ vword, unsigned* __restrict__ tile_counts) {
-    __shared__ unsigned s_scan[kPer * kWarps + 1];
-    const unsigned t_max = *t_max_p;
-    const unsigned base = blockIdx.x * (unsigned)kTile;
-    unsigned cnt[kPer], kept = 0;
-#pragma unroll
-    for (int q = 0; q < kPer; ++q) {
-        const unsigned idx = base + q * kThreads + threadIdx.x;
-        const unsigned kv = idx < n_verts ? cc_keep(tri[labels[idx]], ratio, t_max) : 0u;
-        const unsigned kf = idx < n_faces ? cc_keep(tri[labels[faces[3 * (size_t)idx]]], ratio, t_max) : 0u;
-        kept |= kv << q;
-        cnt[q] = kv | kf << 16;
-    }
-    const unsigned total = tile_scan(cnt, s_scan);
-#pragma unroll
-    for (int q = 0; q < kPer; ++q) {
-        const unsigned idx = base + q * kThreads + threadIdx.x;
-        if (idx < n_verts) vword[idx] = (kept >> q & 1u ? kKept : 0u) | (cnt[q] & 0xffffu);
-    }
-    if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
-}
+// A vertex is kept iff its component is; a face iff its first vertex is (its three vertices share one component).
+struct CcKeep {
+    const int* faces;
+    const int* labels;
+    const unsigned* tri;
+    const unsigned* t_max;
+    float ratio;
+    __device__ bool vert(unsigned v) const { return cc_keep(__ldg(tri + __ldg(labels + v)), ratio, __ldg(t_max)); }
+    __device__ bool face(unsigned f) const { return vert((unsigned)__ldg(faces + 3 * (size_t)f)); }
+};
 
-// Kept vertex v goes to offsets[v / kTile].x + its rank; a face is kept iff its first vertex is (its three vertices share one
-// component), and goes to its tile's first face + its rank among the tile's kept faces, with its indices remapped.
-__global__ void __launch_bounds__(kThreads) cc_compact_kernel(const float* __restrict__ verts, const float* __restrict__ normals,
-                                                              const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
-                                                              const unsigned* __restrict__ vword,
-                                                              const longlong2* __restrict__ offsets, float* __restrict__ verts_out,
-                                                              float* __restrict__ normals_out, int* __restrict__ faces_out) {
-    __shared__ unsigned s_scan[kPer * kWarps + 1];
-    const unsigned base = blockIdx.x * (unsigned)kTile;
-    const longlong2 off = offsets[blockIdx.x];
-#pragma unroll 2
-    for (int q = 0; q < kPer; ++q) {
-        const unsigned v = base + q * kThreads + threadIdx.x;
-        if (v >= n_verts) break;
-        const unsigned w = vword[v];
-        if (!(w & kKept)) continue;
-        const size_t to = 3 * (size_t)(off.x + (w & 0xffffu)), from = 3 * (size_t)v;
+// Kept vertices keep their position (and normal, when normals is given) and index; a face is kept iff its first vertex is.
+struct CcEmit {
+    const float* verts;
+    const float* normals;
+    const unsigned* vword;
+    float* verts_out;
+    float* normals_out;
+    __device__ void vert(unsigned v, size_t to) const {
 #pragma unroll
-        for (int c = 0; c < 3; ++c) verts_out[to + c] = verts[from + c];
+        for (int c = 0; c < 3; ++c) verts_out[3 * to + c] = __ldg(verts + 3 * (size_t)v + c);
         if (normals) {
 #pragma unroll
-            for (int c = 0; c < 3; ++c) normals_out[to + c] = normals[from + c];
+            for (int c = 0; c < 3; ++c) normals_out[3 * to + c] = __ldg(normals + 3 * (size_t)v + c);
         }
     }
-    unsigned cnt[kPer];
-    int tri[kPer][3];
-#pragma unroll
-    for (int q = 0; q < kPer; ++q) {
-        const unsigned f = base + q * kThreads + threadIdx.x;
-        cnt[q] = 0;
-        if (f >= n_faces) continue;
-#pragma unroll
-        for (int c = 0; c < 3; ++c) tri[q][c] = faces[3 * (size_t)f + c];
-        cnt[q] = vword[tri[q][0]] >> 31;
-    }
-    unsigned kept = 0;
-#pragma unroll
-    for (int q = 0; q < kPer; ++q) kept |= cnt[q] << q;
-    tile_scan(cnt, s_scan);
-#pragma unroll
-    for (int q = 0; q < kPer; ++q) {
-        if (!(kept >> q & 1u)) continue;
-        int* out = faces_out + 3 * (off.y + cnt[q]);
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            const unsigned u = (unsigned)tri[q][c];
-            out[c] = (int)(offsets[u / kTile].x + (vword[u] & 0xffffu));
-        }
-    }
-}
+    __device__ bool face(unsigned, const unsigned (&t)[3]) const { return __ldg(vword + t[0]) >> 31; }
+    __device__ unsigned target(unsigned u) const { return u; }
+};
 
 // ---- vertex-face adjacency, Taubin smoothing and mesh normals (b2r_mesh_adjacency / _smooth / _normals) -------------------------
 // A corner is (f, c) with faces[f][c] == v; each vertex's corners are stored contiguously in ascending (f, c), so every sum over
@@ -489,6 +535,18 @@ inline AdjLayout adj_layout(long long n_verts, long long n_faces) {
 constexpr int kAdjInsertion = 16;
 constexpr unsigned kIndexMask = 0x7fffffffu;
 constexpr float kTaubinLambda = 0.5f, kTaubinMu = -0.53f;
+
+__device__ __forceinline__ unsigned rec_a(int2 r) { return (unsigned)r.x & kIndexMask; }
+__device__ __forceinline__ unsigned rec_b(int2 r) { return (unsigned)r.y & kIndexMask; }
+
+// The face of record r of vertex v in its own corner order: the cyclic order (v, a, b) starts at corner c of the face.
+__device__ __forceinline__ void rec_face(int2 r, unsigned v, unsigned (&f)[3]) {
+    const unsigned a = rec_a(r), b = rec_b(r);
+    const unsigned c = (unsigned)r.x >> 31 | ((unsigned)r.y >> 31) << 1;
+    f[0] = c == 0 ? v : c == 1 ? b : a;
+    f[1] = c == 0 ? a : c == 1 ? v : b;
+    f[2] = c == 0 ? b : c == 1 ? a : v;
+}
 
 __global__ void __launch_bounds__(kThreads) adj_count_kernel(const int* __restrict__ faces, unsigned n_faces,
                                                              unsigned long long* __restrict__ ends) {
@@ -656,8 +714,8 @@ __global__ void __launch_bounds__(kThreads) smooth_kernel(const float* __restric
     float s[3] = {0.f, 0.f, 0.f};
     for (unsigned long long i = beg; i < end; ++i) {
         const int2 r = adj[i];
-        const float* pa = p + 3 * (size_t)((unsigned)r.x & kIndexMask);
-        const float* pb = p + 3 * (size_t)((unsigned)r.y & kIndexMask);
+        const float* pa = p + 3 * (size_t)rec_a(r);
+        const float* pb = p + 3 * (size_t)rec_b(r);
 #pragma unroll
         for (int c = 0; c < 3; ++c) s[c] = __fadd_rn(__fadd_rn(s[c], pa[c]), pb[c]);
     }
@@ -679,14 +737,11 @@ __global__ void __launch_bounds__(kThreads) mesh_normals_kernel(const float* __r
     const unsigned long long end = ends[v];
     float n[3] = {0.f, 0.f, 0.f};
     for (unsigned long long i = adj_begin(ends, v); i < end; ++i) {
-        const int2 r = adj[i];
-        const unsigned a = (unsigned)r.x & kIndexMask, b = (unsigned)r.y & kIndexMask;
-        const unsigned c = (unsigned)r.x >> 31 | ((unsigned)r.y >> 31) << 1;
-        // the cyclic order (v, a, b) starts at corner c of the face
-        const unsigned f0 = c == 0 ? v : c == 1 ? b : a, f1 = c == 0 ? a : c == 1 ? v : b, f2 = c == 0 ? b : c == 1 ? a : v;
-        const float* p0 = p + 3 * (size_t)f0;
-        const float* p1 = p + 3 * (size_t)f1;
-        const float* p2 = p + 3 * (size_t)f2;
+        unsigned f[3];
+        rec_face(adj[i], v, f);
+        const float* p0 = p + 3 * (size_t)f[0];
+        const float* p1 = p + 3 * (size_t)f[1];
+        const float* p2 = p + 3 * (size_t)f[2];
         float e1[3], e2[3];
 #pragma unroll
         for (int k = 0; k < 3; ++k) {
@@ -709,30 +764,26 @@ __global__ void __launch_bounds__(kThreads) mesh_normals_kernel(const float* __r
 // The rules are oracle/mesh_decimation.py's.  One round over the adjacency of the current faces: dec_flags_kernel marks frozen
 // vertices and counts distinct neighbours; dec_key_kernel gives every vertex the smallest key (cost, a, b) of its valid edges and
 // that edge's placement; dec_min_kernel takes the smallest key over each closed neighbourhood; dec_select_kernel keeps an edge
-// iff both ends agree with its key and with both minima.  Compaction marks the surviving vertices and faces per tile and packs
-// their counts the way mc_scan_kernel scans them (as cc_mark_kernel does), then writes them in order.  One thread per vertex and
-// plain loads of the neighbours' keys: the result does not depend on the schedule, and the float64 / float32 values are formed
-// with separately rounded intrinsics.  An edge's key is the ulonglong2 (float64 bits of the cost, a << 32 | b); the cost is >= 0,
-// so comparing (x, y) as unsigned integers is the lexicographic order.
+// iff both ends agree with its key and with both minima.  Compaction (mark_kernel, compact_kernel with DecKeep / DecEmit) writes
+// the surviving vertices and faces in order.  One thread per vertex and plain loads of the neighbours' keys: the result does not
+// depend on the schedule, and the float64 / float32 values are formed with separately rounded intrinsics.  An edge's key is the
+// ulonglong2 (float64 bits of the cost, a << 32 | b); the cost is >= 0, so comparing (x, y) as unsigned integers is the
+// lexicographic order.
 // Scratch: info[V] (bit 31 frozen, low bits the valence), key[V], m[V] (ulonglong2), part[V] (the partner of a selected vertex or
-// -1), place[V,3] (the placement of the vertex's key edge), vword[V], tile counts and offsets as in cc_layout, totals and cut.
+// -1), place[V,3] (the placement of the vertex's key edge), then the compaction tail, whose last 256 bytes hold the totals.
 struct DecLayout {
-    size_t info, key, m, part, place, vword, counts, offsets, totals, total;
+    size_t info, key, m, part, place;
+    CompactTail tail;
 };
 
 inline DecLayout dec_layout(long long n_verts, long long n_faces) {
-    const long long tiles = cc_tiles(n_verts, n_faces);
     DecLayout l;
     l.info = 0;
     l.key = l.info + align256((size_t)n_verts * 4);
     l.m = l.key + align256((size_t)n_verts * 16);
     l.part = l.m + align256((size_t)n_verts * 16);
     l.place = l.part + align256((size_t)n_verts * 4);
-    l.vword = l.place + align256((size_t)n_verts * 12);
-    l.counts = l.vword + align256((size_t)n_verts * 4);
-    l.offsets = l.counts + align256((size_t)tiles * 4);
-    l.totals = l.offsets + align256((size_t)tiles * sizeof(longlong2));
-    l.total = l.totals + 256;
+    l.tail = compact_tail(l.place + align256((size_t)n_verts * 12), n_verts, n_faces);
     return l;
 }
 
@@ -742,9 +793,6 @@ constexpr long long kNotSelected = 0x7fffffffffffffffll;
 
 __device__ __forceinline__ bool key_less(ulonglong2 x, ulonglong2 y) { return x.x < y.x || (x.x == y.x && x.y < y.y); }
 __device__ __forceinline__ bool key_eq(ulonglong2 x, ulonglong2 y) { return x.x == y.x && x.y == y.y; }
-
-__device__ __forceinline__ unsigned rec_a(int2 r) { return (unsigned)r.x & kIndexMask; }
-__device__ __forceinline__ unsigned rec_b(int2 r) { return (unsigned)r.y & kIndexMask; }
 
 // Slot s of v's neighbour list: the a (even s) or b (odd s) of record s / 2.
 __device__ __forceinline__ unsigned nb_slot(const int2* __restrict__ adj, unsigned long long beg, unsigned long long s) {
@@ -765,15 +813,6 @@ __device__ __forceinline__ bool nb_has(const int2* __restrict__ adj, unsigned lo
         if (rec_a(r) == u || rec_b(r) == u) return true;
     }
     return false;
-}
-
-// The face of record r of vertex v in its own corner order (as mesh_normals_kernel rebuilds it).
-__device__ __forceinline__ void rec_face(int2 r, unsigned v, unsigned (&f)[3]) {
-    const unsigned a = rec_a(r), b = rec_b(r);
-    const unsigned c = (unsigned)r.x >> 31 | ((unsigned)r.y >> 31) << 1;
-    f[0] = c == 0 ? v : c == 1 ? b : a;
-    f[1] = c == 0 ? a : c == 1 ? v : b;
-    f[2] = c == 0 ? b : c == 1 ? a : v;
 }
 
 __device__ __forceinline__ void cross64(const double (&e1)[3], const double (&e2)[3], double (&n)[3]) {
@@ -996,25 +1035,22 @@ __global__ void dec_count_kernel(long long n_faces, long long* __restrict__ coun
 // Whether the selected edge at survivor a collapses: every selected edge, or with a cut (cost bits, a) the ones up to it.
 __device__ __forceinline__ bool dec_kept(const int* __restrict__ part, const long long* __restrict__ sel_keys,
                                          const long long* __restrict__ cut, unsigned a) {
-    if (part[a] <= (int)a) return false;
+    if (__ldg(part + a) <= (int)a) return false;
     if (!cut) return true;
-    const long long k = sel_keys[a];
-    return k < cut[0] || (k == cut[0] && (long long)a <= cut[1]);
+    const long long k = __ldg(sel_keys + a), c0 = __ldg(cut);
+    return k < c0 || (k == c0 && (long long)a <= __ldg(cut + 1));
 }
 
 // The survivor vertex u collapses into, or u itself.
 __device__ __forceinline__ unsigned dec_target(const int* __restrict__ part, const long long* __restrict__ sel_keys,
                                                const long long* __restrict__ cut, unsigned u) {
-    const int t = part[u];
+    const int t = __ldg(part + u);
     return t >= 0 && t < (int)u && dec_kept(part, sel_keys, cut, (unsigned)t) ? (unsigned)t : u;
 }
 
-// A face is deleted iff it holds both ends of a collapsing edge.
-__device__ __forceinline__ bool dec_face_dies(const int* __restrict__ faces, unsigned f, const int* __restrict__ part,
-                                              const long long* __restrict__ sel_keys, const long long* __restrict__ cut) {
-    unsigned t[3];
-#pragma unroll
-    for (int c = 0; c < 3; ++c) t[c] = (unsigned)faces[3 * (size_t)f + c];
+// A face with indices t is deleted iff it holds both ends of a collapsing edge.
+__device__ __forceinline__ bool dec_face_dies(const unsigned (&t)[3], const int* __restrict__ part, const long long* __restrict__ sel_keys,
+                                              const long long* __restrict__ cut) {
     bool dies = false;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
@@ -1024,84 +1060,61 @@ __device__ __forceinline__ bool dec_face_dies(const int* __restrict__ faces, uns
     return dies;
 }
 
-__global__ void __launch_bounds__(kThreads) dec_mark_kernel(const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
-                                                            const int* __restrict__ part, const long long* __restrict__ sel_keys,
-                                                            const long long* __restrict__ cut, unsigned* __restrict__ vword,
-                                                            unsigned* __restrict__ tile_counts) {
-    __shared__ unsigned s_scan[kPer * kWarps + 1];
-    const unsigned base = blockIdx.x * (unsigned)kTile;
-    unsigned cnt[kPer], kept = 0;
+// A vertex survives iff it does not collapse into another; a face iff it does not hold both ends of a collapsing edge.
+struct DecKeep {
+    const int* faces;
+    const int* part;
+    const long long* sel_keys;
+    const long long* cut;
+    __device__ bool vert(unsigned v) const { return dec_target(part, sel_keys, cut, v) == v; }
+    __device__ bool face(unsigned f) const {
+        unsigned t[3];
 #pragma unroll
-    for (int q = 0; q < kPer; ++q) {
-        const unsigned idx = base + q * kThreads + threadIdx.x;
-        const unsigned kv = idx < n_verts && dec_target(part, sel_keys, cut, idx) == idx ? 1u : 0u;
-        const unsigned kf = idx < n_faces && !dec_face_dies(faces, idx, part, sel_keys, cut) ? 1u : 0u;
-        kept |= kv << q;
-        cnt[q] = kv | kf << 16;
+        for (int c = 0; c < 3; ++c) t[c] = (unsigned)__ldg(faces + 3 * (size_t)f + c);
+        return !dec_face_dies(t, part, sel_keys, cut);
     }
-    const unsigned total = tile_scan(cnt, s_scan);
-#pragma unroll
-    for (int q = 0; q < kPer; ++q) {
-        const unsigned idx = base + q * kThreads + threadIdx.x;
-        if (idx < n_verts) vword[idx] = (kept >> q & 1u ? kKept : 0u) | (cnt[q] & 0xffffu);
-    }
-    if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
-}
+};
 
-// Surviving vertices in order (a collapsing survivor at its placement with Q_a + Q_b), surviving faces in order, remapped.
-__global__ void __launch_bounds__(kThreads) dec_compact_kernel(const float* __restrict__ verts, const double* __restrict__ q,
-                                                               const int* __restrict__ faces, unsigned n_faces, unsigned n_verts,
-                                                               const int* __restrict__ part, const long long* __restrict__ sel_keys,
-                                                               const long long* __restrict__ cut, const float* __restrict__ place,
-                                                               const unsigned* __restrict__ vword,
-                                                               const longlong2* __restrict__ offsets, float* __restrict__ verts_out,
-                                                               double* __restrict__ q_out, int* __restrict__ faces_out) {
-    __shared__ unsigned s_scan[kPer * kWarps + 1];
-    const unsigned base = blockIdx.x * (unsigned)kTile;
-    const longlong2 off = offsets[blockIdx.x];
-#pragma unroll 1
-    for (int q8 = 0; q8 < kPer; ++q8) {
-        const unsigned v = base + q8 * kThreads + threadIdx.x;
-        if (v >= n_verts) break;
-        const unsigned w = vword[v];
-        if (!(w & kKept)) continue;
-        const size_t to = (size_t)(off.x + (w & 0xffffu));
+// A collapsing survivor moves to its placement with Q_a + Q_b, any other survivor keeps its position and Q; face indices map
+// through the collapses.
+struct DecEmit {
+    const float* verts;
+    const double* q;
+    const int* part;
+    const long long* sel_keys;
+    const long long* cut;
+    const float* place;
+    float* verts_out;
+    double* q_out;
+    __device__ void vert(unsigned v, size_t to) const {
         const bool moves = dec_kept(part, sel_keys, cut, v);
         const float* from = (moves ? place : verts) + 3 * (size_t)v;
 #pragma unroll
-        for (int c = 0; c < 3; ++c) verts_out[3 * to + c] = from[c];
+        for (int c = 0; c < 3; ++c) verts_out[3 * to + c] = __ldg(from + c);
         const double* qa = q + 10 * (size_t)v;
-        const double* qb = q + 10 * (size_t)(moves ? part[v] : 0);
+        const double* qb = q + 10 * (size_t)(moves ? __ldg(part + v) : 0);
 #pragma unroll
-        for (int i = 0; i < 10; ++i) q_out[10 * to + i] = moves ? __dadd_rn(qa[i], qb[i]) : qa[i];
+        for (int i = 0; i < 10; ++i) q_out[10 * to + i] = moves ? __dadd_rn(__ldg(qa + i), __ldg(qb + i)) : __ldg(qa + i);
     }
-    unsigned cnt[kPer];
-#pragma unroll
-    for (int k = 0; k < kPer; ++k) {
-        const unsigned f = base + k * kThreads + threadIdx.x;
-        cnt[k] = f < n_faces && !dec_face_dies(faces, f, part, sel_keys, cut) ? 1u : 0u;
-    }
-    unsigned kept = 0;
-#pragma unroll
-    for (int k = 0; k < kPer; ++k) kept |= cnt[k] << k;
-    tile_scan(cnt, s_scan);
-#pragma unroll
-    for (int k = 0; k < kPer; ++k) {
-        if (!(kept >> k & 1u)) continue;
-        const unsigned f = base + k * kThreads + threadIdx.x;
-        int* out = faces_out + 3 * (off.y + cnt[k]);
-#pragma unroll
-        for (int c = 0; c < 3; ++c) {
-            const unsigned u = dec_target(part, sel_keys, cut, (unsigned)faces[3 * (size_t)f + c]);
-            out[c] = (int)(offsets[u / kTile].x + (vword[u] & 0xffffu));
-        }
-    }
-}
+    __device__ bool face(unsigned, const unsigned (&t)[3]) const { return !dec_face_dies(t, part, sel_keys, cut); }
+    __device__ unsigned target(unsigned u) const { return dec_target(part, sel_keys, cut, u); }
+};
 
 int check_grid(const char* what, int n0, int n1, int n2) {
     B2R_CHECK_ARG(n0 >= 2 && n1 >= 2 && n2 >= 2, "%s: every axis needs n >= 2 (got %d x %d x %d)", what, n0, n1, n2);
     B2R_CHECK_ARG((long long)n0 * n1 * n2 <= INT32_MAX, "%s: n0*n1*n2 = %lld exceeds INT32_MAX", what, (long long)n0 * n1 * n2);
     return 0;
+}
+
+// mark_kernel, then mc_scan_kernel over its tile counts: vword, every tile's (first vertex, first face) and the totals (V', F').
+template <class Keep>
+static void mark_and_scan(Keep keep, long long n_faces, long long n_verts, char* s, const CompactTail& t, long long* totals,
+                          cudaStream_t st) {
+    const int tiles = (int)compact_tiles(n_verts, n_faces);
+    if (tiles)
+        mark_kernel<<<tiles, kThreads, 0, st>>>(keep, (unsigned)n_faces, (unsigned)n_verts, (unsigned*)(s + t.vword),
+                                                (unsigned*)(s + t.counts));
+    mc_scan_kernel<<<1, kScanThreads, 0, st>>>((const unsigned*)(s + t.counts), tiles, (longlong2*)(s + t.offsets), totals);
 }
 
 }  // namespace mc
@@ -1186,7 +1199,7 @@ constexpr unsigned kMaxBlocks = 8 * 148;      // cc_max_kernel: grid-stride, a f
 
 extern "C" size_t b2r_mesh_cc_scratch_bytes(long long n_verts, long long n_faces) {
     if (n_verts < 0 || n_verts > INT32_MAX || n_faces < 0 || n_faces > INT32_MAX) return 0;
-    return b2r::mc::cc_layout(n_verts, n_faces).total;
+    return b2r::mc::cc_layout(n_verts, n_faces).tail.total;
 }
 
 extern "C" int b2r_mesh_cc_label(const int* faces, long long n_faces, long long n_verts, int* labels, void* scratch, void* stream) {
@@ -1216,10 +1229,9 @@ extern "C" int b2r_mesh_cc_select(const int* faces, long long n_faces, long long
     B2R_CHECK_ARG(std::isfinite(ratio) && ratio >= 0.f && ratio <= 1.f, "%s: ratio = %g must be finite and in [0, 1]", what, (double)ratio);
     if (int rc = check_scratch(what, scratch)) return rc;
     const CcLayout l = cc_layout(n_verts, n_faces);
-    const int tiles = (int)cc_tiles(n_verts, n_faces);
     char* s = static_cast<char*>(scratch);
     unsigned* tri = (unsigned*)(s + l.a);
-    unsigned* t_max = (unsigned*)(s + l.max);
+    unsigned* t_max = (unsigned*)(s + l.tail.last);
     cudaStream_t st = (cudaStream_t)stream;
     if (int rc = b2r::cuda_result(cudaMemsetAsync(tri, 0, (size_t)n_verts * 4, st), what)) return rc;
     if (int rc = b2r::cuda_result(cudaMemsetAsync(t_max, 0, 4, st), what)) return rc;
@@ -1228,10 +1240,7 @@ extern "C" int b2r_mesh_cc_select(const int* faces, long long n_faces, long long
         const unsigned blocks = blocks_of(n_verts, kThreads);
         cc_max_kernel<<<blocks < kMaxBlocks ? blocks : kMaxBlocks, kThreads, 0, st>>>(tri, (unsigned)n_verts, t_max);
     }
-    if (tiles)
-        cc_mark_kernel<<<tiles, kThreads, 0, st>>>(faces, (unsigned)n_faces, (unsigned)n_verts, labels, tri, t_max, ratio,
-                                                   (unsigned*)(s + l.vword), (unsigned*)(s + l.counts));
-    mc_scan_kernel<<<1, kScanThreads, 0, st>>>((const unsigned*)(s + l.counts), tiles, (longlong2*)(s + l.offsets), totals_dev);
+    mark_and_scan(CcKeep{faces, labels, tri, t_max, ratio}, n_faces, n_verts, s, l.tail, totals_dev, st);
     B2R_LAUNCH_CHECK(what);
     return 0;
 }
@@ -1245,13 +1254,14 @@ extern "C" int b2r_mesh_cc_compact(const float* verts, const float* normals_or_n
     B2R_CHECK_ARG((verts && verts_out && (!normals_or_null || normals_out)) || !n_verts,
                   "%s: NULL verts / verts_out, or normals given and NULL normals_out, with n_verts > 0", what);
     if (int rc = check_scratch(what, scratch)) return rc;
-    const CcLayout l = cc_layout(n_verts, n_faces);
-    const int tiles = (int)cc_tiles(n_verts, n_faces);
+    const CompactTail t = cc_layout(n_verts, n_faces).tail;
+    const int tiles = (int)compact_tiles(n_verts, n_faces);
     if (!tiles) return 0;
     const char* s = static_cast<const char*>(scratch);
-    cc_compact_kernel<<<tiles, kThreads, 0, (cudaStream_t)stream>>>(verts, normals_or_null, faces, (unsigned)n_faces, (unsigned)n_verts,
-                                                                    (const unsigned*)(s + l.vword), (const longlong2*)(s + l.offsets),
-                                                                    verts_out, normals_out, faces_out);
+    const unsigned* vword = (const unsigned*)(s + t.vword);
+    compact_kernel<<<tiles, kThreads, 0, (cudaStream_t)stream>>>(CcEmit{verts, normals_or_null, vword, verts_out, normals_out}, faces,
+                                                                 (unsigned)n_faces, (unsigned)n_verts, vword,
+                                                                 (const longlong2*)(s + t.offsets), faces_out);
     B2R_LAUNCH_CHECK(what);
     return 0;
 }
@@ -1335,7 +1345,7 @@ extern "C" int b2r_mesh_normals(const float* verts, long long n_faces, long long
 
 extern "C" size_t b2r_mesh_decimate_scratch_bytes(long long n_verts, long long n_faces) {
     if (n_verts < 0 || n_verts > INT32_MAX || n_faces < 0 || n_faces > INT32_MAX) return 0;
-    return b2r::mc::dec_layout(n_verts, n_faces).total;
+    return b2r::mc::dec_layout(n_verts, n_faces).tail.total;
 }
 
 extern "C" int b2r_mesh_quadrics(const float* verts, long long n_faces, long long n_verts, const void* adj_scratch, double* quadrics,
@@ -1399,18 +1409,14 @@ extern "C" int b2r_mesh_decimate_compact(const float* verts, const double* quadr
     if (!n_verts) return 0;
     if (int rc = check_scratch(what, scratch)) return rc;
     const DecLayout l = dec_layout(n_verts, n_faces);
-    const int tiles = (int)cc_tiles(n_verts, n_faces);
+    const int tiles = (int)compact_tiles(n_verts, n_faces);
     char* s = static_cast<char*>(scratch);
     const int* part = (const int*)(s + l.part);
-    unsigned* vword = (unsigned*)(s + l.vword);
-    longlong2* offsets = (longlong2*)(s + l.offsets);
     cudaStream_t st = (cudaStream_t)stream;
-    dec_mark_kernel<<<tiles, kThreads, 0, st>>>(faces, (unsigned)n_faces, (unsigned)n_verts, part, sel_keys, cut_or_null, vword,
-                                                (unsigned*)(s + l.counts));
-    mc_scan_kernel<<<1, kScanThreads, 0, st>>>((const unsigned*)(s + l.counts), tiles, offsets, (long long*)(s + l.totals));
-    dec_compact_kernel<<<tiles, kThreads, 0, st>>>(verts, quadrics, faces, (unsigned)n_faces, (unsigned)n_verts, part, sel_keys,
-                                                   cut_or_null, (const float*)(s + l.place), vword, offsets, verts_out, quadrics_out,
-                                                   faces_out);
+    mark_and_scan(DecKeep{faces, part, sel_keys, cut_or_null}, n_faces, n_verts, s, l.tail, (long long*)(s + l.tail.last), st);
+    compact_kernel<<<tiles, kThreads, 0, st>>>(
+        DecEmit{verts, quadrics, part, sel_keys, cut_or_null, (const float*)(s + l.place), verts_out, quadrics_out}, faces,
+        (unsigned)n_faces, (unsigned)n_verts, (const unsigned*)(s + l.tail.vword), (const longlong2*)(s + l.tail.offsets), faces_out);
     B2R_LAUNCH_CHECK(what);
     return 0;
 }

@@ -25,14 +25,6 @@ def box_lattice(box_min, box_max, n):
     return dims, tuple(float(np.float32(v)) for v in lo), float(np.float32(step))
 
 
-def extract(field, level, spacing, origin, want_normals):
-    """(verts, faces, normals | None) of the level set of ``field`` on the device (ops.marching_cubes)."""
-    if want_normals:
-        return ops.marching_cubes(field, level, spacing, origin, normals=True)
-    verts, faces = ops.marching_cubes(field, level, spacing, origin)
-    return verts, faces, None
-
-
 def vertex_colors(model, verts, normals, precision=None):
     """uint8 [V,3] colours of the model's rgb head at each vertex, seen by a camera looking along ``-normals``
     (rows x = [vertex, -normal]), quantised on the device by ops.to8b."""
@@ -90,11 +82,14 @@ def export(model, field, level, spacing, origin, ply_filename, normals, colors, 
     normals become the smoothed mesh's own, so colours are sampled on the smoothed surface; the field normals are not computed.
     ``max_faces`` (an int >= 1) then decimates the mesh to that many triangles (ops.decimate_mesh; one host synchronisation per
     round) before the colour query, so removed vertices cost no MLP rows, and the normals are the decimated mesh's own."""
-    iterations = ops._check_iterations(smooth_iterations)
-    budget = None if max_faces is None else ops._check_max_faces(max_faces)
+    iterations = ops._check_int("iterations", smooth_iterations, 0, ops._INT32_MAX)
+    budget = None if max_faces is None else ops._check_int("max_faces", max_faces, 1)
     want_normals = normals or colors
     own_normals = want_normals and (iterations or budget is not None)
-    verts, faces, nrm = extract(field, level, spacing, origin, want_normals and not own_normals)
+    if want_normals and not own_normals:
+        verts, faces, nrm = ops.marching_cubes(field, level, spacing, origin, normals=True)
+    else:
+        (verts, faces), nrm = ops.marching_cubes(field, level, spacing, origin), None
     if min_component_ratio:
         # marching-cubes faces index their own vertices, so the index checks of ops.filter_components / ops.smooth_mesh are not needed
         verts, faces, nrm = ops._filter_components(verts, faces, ops._check_ratio(min_component_ratio), nrm)

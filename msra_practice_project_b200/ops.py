@@ -850,6 +850,31 @@ def _mesh_faces(faces: torch.Tensor, n_verts: int) -> torch.Tensor:
     return faces.contiguous()
 
 
+def _mesh_args(verts: torch.Tensor, faces: torch.Tensor, normals: torch.Tensor | None = None):
+    """The checked ``(verts, faces, normals)`` of a mesh op: ``verts`` and ``normals`` (when given) contiguous [V,3] float32
+    CUDA tensors, ``faces`` as ``_mesh_faces`` leaves it, all on one device; raises RuntimeError otherwise, before any launch."""
+    verts = _cuda_f32(verts, "verts")
+    if verts.dim() != 2 or verts.shape[1] != 3:
+        raise RuntimeError(f"verts must be [V,3], got {list(verts.shape)}")
+    if normals is not None:
+        normals = _cuda_f32(normals, "normals")
+        if normals.shape != verts.shape:
+            raise RuntimeError(f"normals must have the shape of verts {list(verts.shape)}, got {list(normals.shape)}")
+    faces = _mesh_faces(faces, verts.shape[0])
+    if faces.device != verts.device or (normals is not None and normals.device != verts.device):
+        names = "verts and faces" if normals is None else "verts, faces and normals"
+        raise RuntimeError(f"{names} must be on the same device")
+    return verts, faces, normals
+
+
+def _check_int(name: str, value, lo: int, hi: int | None = None) -> int:
+    """``value`` as an int in [lo, hi] (no upper bound when ``hi`` is None); ValueError for anything else, bools included."""
+    if isinstance(value, bool) or not isinstance(value, (int, np.integer)) or value < lo or (hi is not None and value > hi):
+        bound = f">= {lo}" if hi is None else f"in [{lo}, {'2^31 - 1' if hi == _INT32_MAX else hi}]"
+        raise ValueError(f"{name} must be an int {bound}, got {value!r}")
+    return int(value)
+
+
 def _cc_label(faces: torch.Tensor, n_verts: int, scratch: torch.Tensor) -> torch.Tensor:
     labels = torch.empty((n_verts,), dtype=torch.int32, device=faces.device)
     check(lib().b2r_mesh_cc_label(ptr(faces), faces.shape[0], n_verts, ptr(labels), ptr(scratch), _stream(faces)), "b2r_mesh_cc_label")
@@ -907,23 +932,8 @@ def filter_components(verts: torch.Tensor, faces: torch.Tensor, ratio: float, no
     r = _check_ratio(ratio)
     if r == 0.0:
         return verts, faces, normals
-    verts = _cuda_f32(verts, "verts")
-    if verts.dim() != 2 or verts.shape[1] != 3:
-        raise RuntimeError(f"verts must be [V,3], got {list(verts.shape)}")
-    if normals is not None:
-        normals = _cuda_f32(normals, "normals")
-        if normals.shape != verts.shape:
-            raise RuntimeError(f"normals must have the shape of verts {list(verts.shape)}, got {list(normals.shape)}")
-    faces = _mesh_faces(faces, verts.shape[0])
-    if faces.device != verts.device or (normals is not None and normals.device != verts.device):
-        raise RuntimeError("verts, faces and normals must be on the same device")
+    verts, faces, normals = _mesh_args(verts, faces, normals)
     return _filter_components(verts, faces, r, normals)
-
-
-def _check_iterations(iterations) -> int:
-    if isinstance(iterations, bool) or not isinstance(iterations, (int, np.integer)) or not 0 <= iterations <= _INT32_MAX:
-        raise ValueError(f"iterations must be an int in [0, 2^31 - 1], got {iterations!r}")
-    return int(iterations)
 
 
 def _smooth_mesh(verts: torch.Tensor, faces: torch.Tensor, iterations: int, normals: bool):
@@ -954,23 +964,12 @@ def smooth_mesh(verts: torch.Tensor, faces: torch.Tensor, iterations: int, *, no
     ``mesh_normals``.  ``iterations`` must be an int >= 0 (ValueError); 0 without ``normals`` returns ``verts`` without a
     launch.  Otherwise checks that ``faces`` is [F,3] int32 on the device with every index in [0, V) (RuntimeError otherwise,
     before any launch; one host synchronisation)."""
-    iterations = _check_iterations(iterations)
+    iterations = _check_int("iterations", iterations, 0, _INT32_MAX)
     if not iterations and not normals:
         return verts
-    verts = _cuda_f32(verts, "verts")
-    if verts.dim() != 2 or verts.shape[1] != 3:
-        raise RuntimeError(f"verts must be [V,3], got {list(verts.shape)}")
-    faces = _mesh_faces(faces, verts.shape[0])
-    if faces.device != verts.device:
-        raise RuntimeError("verts and faces must be on the same device")
+    verts, faces, _ = _mesh_args(verts, faces)
     out, nrm = _smooth_mesh(verts, faces, iterations, normals)
     return (out, nrm) if normals else out
-
-
-def _check_max_faces(max_faces) -> int:
-    if isinstance(max_faces, bool) or not isinstance(max_faces, (int, np.integer)) or not 1 <= max_faces:
-        raise ValueError(f"max_faces must be an int >= 1, got {max_faces!r}")
-    return int(max_faces)
 
 
 def _decimate_mesh(verts: torch.Tensor, faces: torch.Tensor, max_faces: int, stats: dict | None = None):
@@ -1031,11 +1030,6 @@ def decimate_mesh(verts: torch.Tensor, faces: torch.Tensor, max_faces: int):
     [F,3] int32 on the device with every index in [0, V) (RuntimeError otherwise, before any launch; one host
     synchronisation); ``max_faces >= F`` then returns the inputs without a launch.  Every round synchronises once more to read
     its collapse count."""
-    max_faces = _check_max_faces(max_faces)
-    verts = _cuda_f32(verts, "verts")
-    if verts.dim() != 2 or verts.shape[1] != 3:
-        raise RuntimeError(f"verts must be [V,3], got {list(verts.shape)}")
-    faces = _mesh_faces(faces, verts.shape[0])
-    if faces.device != verts.device:
-        raise RuntimeError("verts and faces must be on the same device")
+    max_faces = _check_int("max_faces", max_faces, 1)
+    verts, faces, _ = _mesh_args(verts, faces)
     return _decimate_mesh(verts, faces, max_faces)
