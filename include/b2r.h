@@ -311,6 +311,31 @@ int b2r_mc_emit(const float* field, int n0, int n1, int n2, float level, float s
  * the triangle normals face.  A zero-length n (a flat field there) gives (0, 0, 0). */
 int b2r_mc_normals(const float* field, int n0, int n1, int n2, float level, const void* scratch, float* normals, void* stream);
 
+/* ---- narrow-band marching cubes (no reference counterpart: the density query of create_mesh limited to the surface's bricks) --
+ * Bricks of `stride` (>= 2) cells per axis: an axis of n points has nb = ceil((n - 1) / stride) bricks; brick b covers the cells
+ * [b stride, min((b + 1) stride, n - 1)) and its coarse corners are the points min(b stride, n - 1), min((b + 1) stride, n - 1).
+ * Flags are one byte per brick, [nb0, nb1, nb2], axis 0 slowest.  "Below" is field < level, NaN not below (b2r_mc_count).
+ *   b2r_band_select:   given a field whose values are valid at every coarse corner (+inf elsewhere keeps the rest above the
+ *                      level), flags[b] = 1 for every brick within one brick (26-neighbourhood, clamped at the box) of a brick
+ *                      whose 8 coarse corners are not all on the same side of the level, 0 otherwise; index[] = the linear indices,
+ *                      ascending, of the needed points: every point of the closure of a flagged brick and every point one step
+ *                      along one axis from such a point (the differences of b2r_mc_normals read them); count_dev[0] = their number
+ *                      M, one long long in DEVICE memory.  index must hold n0*n1*n2 ints.  scratch: b2r_band_scratch_bytes(n0, n1,
+ *                      n2, stride) bytes, 16-byte aligned (0 for a shape b2r_mc_scratch_bytes rejects or stride < 2).
+ *   b2r_lattice_rows:  x[r] = (point, direction) of row index[r] of the grid_n or lattice_dims description `in`, for r < m, with
+ *                      the point formula of those rows (so an MLP on x equals the MLP on the description at those rows).
+ *                      PRECONDITION: every index[r] lies in [0, in->n_rays) (not checked: the indices are in device memory).
+ *   b2r_mc_count_band: b2r_mc_count limited to the flagged bricks: a cell outside a flagged brick gets configuration 0, and a
+ *                      crossing edge is counted only when it is an edge of a cell in a flagged brick.  b2r_mc_emit and
+ *                      b2r_mc_normals then give the mesh of b2r_mc_count with the faces of the other cells and the vertices on
+ *                      no counted edge removed, in the same relative order.  scratch as for b2r_mc_count. */
+size_t b2r_band_scratch_bytes(int n0, int n1, int n2, int stride);
+int b2r_band_select(const float* field, int n0, int n1, int n2, float level, int stride, void* scratch, unsigned char* flags,
+                    int* index, long long* count_dev, void* stream);
+int b2r_lattice_rows(const b2r_mlp_input* in, const int* index, long long m, float* x, void* stream);
+int b2r_mc_count_band(const float* field, int n0, int n1, int n2, float level, const unsigned char* flags, int stride,
+                      void* scratch, long long* totals_dev, void* stream);
+
 /* ---- connected components of a triangle mesh (no reference counterpart: clean-up of exported meshes) ----------------------
  * faces[F,3] (int32) index verts[V,3]; two vertices are connected when a face has them as (v0,v1) or (v1,v2).  PRECONDITION:
  * every face index lies in [0, n_verts) (not checked: the indices are in device memory; ops.py checks them first).  Counts are

@@ -87,6 +87,12 @@ SIGNATURES = {
     "b2r_mc_emit": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                               C.c_void_p, c_float_p, C.c_void_p, C.c_void_p]),
     "b2r_mc_normals": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, c_float_p, C.c_void_p]),
+    "b2r_band_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    "b2r_band_select": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                  C.c_void_p, C.c_void_p]),
+    "b2r_lattice_rows": (C.c_int, [C.POINTER(MlpInput), C.c_void_p, c_ll, c_float_p, C.c_void_p]),
+    "b2r_mc_count_band": (C.c_int, [c_float_p, C.c_int, C.c_int, C.c_int, C.c_float, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                    C.c_void_p]),
     "b2r_mesh_cc_scratch_bytes": (C.c_size_t, [c_ll, c_ll]),
     "b2r_mesh_cc_label": (C.c_int, [C.c_void_p, c_ll, c_ll, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b2r_mesh_cc_select": (C.c_int, [C.c_void_p, c_ll, c_ll, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),

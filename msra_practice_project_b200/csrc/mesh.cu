@@ -5,7 +5,8 @@
 // consecutive linear indices per CTA:
 //   mc_count_kernel     reads the field; writes one 32-bit word per point (crossing bits of the point's 3 owned edges,
 //                       the configuration of the cell it is the minimum corner of, the point's first vertex index within
-//                       its tile) and the tile's vertex / triangle counts
+//                       its tile) and the tile's vertex / triangle counts; its Band instantiation (b2r_mc_count_band) keeps
+//                       only the cells of flagged bricks and their edges
 //   mc_scan_kernel      exclusive scan of the tile counts (one CTA) + the totals (V, F)
 //   mc_vertices_kernel  reads the words, and the field at crossing points only; writes the vertices
 //   mc_faces_kernel     reads the words of the cell corners; writes the triangles
@@ -82,8 +83,13 @@ __device__ __forceinline__ unsigned tile_scan(unsigned (&v)[kPer], unsigned* s /
     return s[kPer * kWarps];
 }
 
+// Mask: __device__ unsigned edges(i, j, k, bits) const and unsigned cell(i, j, k, cfg) const return the crossing bits and the
+// configuration of point (i, j, k) that are counted.  DenseMask counts everything; Band (below) limits the mesh to flagged bricks,
+// and the other passes, which only read the words, follow.
+template <class Mask>
 __global__ void __launch_bounds__(kThreads) mc_count_kernel(const float* __restrict__ f, int n0, int n1, int n2, float level,
-                                                            unsigned* __restrict__ words, unsigned* __restrict__ tile_counts) {
+                                                            unsigned* __restrict__ words, unsigned* __restrict__ tile_counts,
+                                                            Mask mask) {
     __shared__ unsigned s_ntri[256];
     __shared__ unsigned s_scan[kPer * kWarps + 1];
     static_assert(kThreads == 256, "one configuration per thread");
@@ -112,9 +118,9 @@ __global__ void __launch_bounds__(kThreads) mc_count_kernel(const float* __restr
             b |= below(idx + s0 + s1) << 6;
             b |= below(idx + s0 + s1 + 1) << 7;
         }
-        const unsigned bits = (ci ? ((b ^ (b >> 4)) & 1) : 0) | (cj ? ((b ^ (b >> 2)) & 1) << 1 : 0) |
-                              (ck ? ((b ^ (b >> 1)) & 1) << 2 : 0);
-        const unsigned cfg = cell ? b : 0;
+        const unsigned bits = mask.edges(i, j, k, (ci ? ((b ^ (b >> 4)) & 1) : 0) | (cj ? ((b ^ (b >> 2)) & 1) << 1 : 0) |
+                                                  (ck ? ((b ^ (b >> 1)) & 1) << 2 : 0));
+        const unsigned cfg = mask.cell(i, j, k, cell ? b : 0);
         word[q] = bits | cfg << kCfgShift;
         cnt[q] = __popc(bits) | s_ntri[cfg] << 16;
     }
@@ -125,6 +131,147 @@ __global__ void __launch_bounds__(kThreads) mc_count_kernel(const float* __restr
         if (idx < n) words[idx] = word[q] | (cnt[q] & 0xffffu) << kVertShift;
     }
     if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
+}
+
+struct DenseMask {
+    __device__ __forceinline__ unsigned edges(unsigned, unsigned, unsigned, unsigned bits) const { return bits; }
+    __device__ __forceinline__ unsigned cell(unsigned, unsigned, unsigned, unsigned cfg) const { return cfg; }
+};
+
+// ---- narrow band (b2r_band_select, b2r_mc_count_band) -------------------------------------------------------------------------
+// Bricks of `stride` cells per axis: an axis of n points has nb = ceil((n - 1) / stride) bricks, brick b covers cells
+// [b stride, min((b + 1) stride, n - 1)) and its closure the points [b stride, min((b + 1) stride, n - 1)].  Flags are one byte
+// per brick, axis 0 slowest.  The bricks whose closure holds coordinate c are those of the cells c - 1 and c that exist, so one
+// span serves the needed-point test and the edge mask of the count pass.
+struct Band {
+    const unsigned char* flags;
+    unsigned n0, n1, n2, nb1, nb2, stride;
+
+    __device__ __forceinline__ bool flag(unsigned b0, unsigned b1, unsigned b2) const { return __ldg(flags + (b0 * nb1 + b1) * nb2 + b2) != 0; }
+    // [lo, hi]: the bricks of the cells next to coordinate c of an axis of n points
+    __device__ __forceinline__ void span(unsigned c, unsigned n, unsigned& lo, unsigned& hi) const {
+        lo = (c ? c - 1 : 0) / stride;
+        hi = (c + 1 < n ? c : c - 1) / stride;
+    }
+    __device__ __forceinline__ bool any(const unsigned (&lo)[3], const unsigned (&hi)[3]) const {
+        for (unsigned b0 = lo[0]; b0 <= hi[0]; ++b0)
+            for (unsigned b1 = lo[1]; b1 <= hi[1]; ++b1)
+                for (unsigned b2 = lo[2]; b2 <= hi[2]; ++b2)
+                    if (flag(b0, b1, b2)) return true;
+        return false;
+    }
+    // point (i, j, k) lies in the closure of a flagged brick, or one step along one axis from such a point
+    __device__ __forceinline__ bool needed(unsigned i, unsigned j, unsigned k) const {
+        const unsigned p[3] = {i, j, k}, n[3] = {n0, n1, n2};
+        unsigned lo[3], hi[3], wlo[3], whi[3], t;
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            span(p[a], n[a], lo[a], hi[a]);
+            span(p[a] ? p[a] - 1 : 0, n[a], wlo[a], t);
+            span(p[a] + 1 < n[a] ? p[a] + 1 : p[a], n[a], t, whi[a]);
+        }
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            unsigned l[3] = {lo[0], lo[1], lo[2]}, h[3] = {hi[0], hi[1], hi[2]};
+            l[a] = wlo[a];
+            h[a] = whi[a];
+            if (any(l, h)) return true;
+        }
+        return false;
+    }
+    // the count pass keeps the configuration of a cell in a flagged brick and an edge of such a cell, and clears the rest
+    __device__ __forceinline__ unsigned cell(unsigned i, unsigned j, unsigned k, unsigned cfg) const {
+        return cfg && flag(i / stride, j / stride, k / stride) ? cfg : 0u;
+    }
+    __device__ __forceinline__ unsigned edges(unsigned i, unsigned j, unsigned k, unsigned bits) const {
+        if (!bits) return 0u;
+        const unsigned p[3] = {i, j, k}, n[3] = {n0, n1, n2};
+        unsigned lo[3], hi[3];
+#pragma unroll
+        for (int a = 0; a < 3; ++a) span(p[a], n[a], lo[a], hi[a]);
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            if (!(bits >> a & 1u)) continue;
+            unsigned l[3] = {lo[0], lo[1], lo[2]}, h[3] = {hi[0], hi[1], hi[2]};
+            l[a] = h[a] = p[a] / stride;           // the edge p -> p + e_a lies in the cells whose axis-a coordinate is p[a]
+            if (!any(l, h)) bits &= ~(1u << a);
+        }
+        return bits;
+    }
+};
+
+// One thread per brick: flagged (raw[b] = 1) when its 8 coarse corners are not all on the same side of the level.
+__global__ void band_flag_kernel(const float* __restrict__ f, Band band, unsigned nb0, float level, unsigned char* __restrict__ raw) {
+    const unsigned nb = nb0 * band.nb1 * band.nb2, b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nb) return;
+    const unsigned bb[3] = {b / (band.nb1 * band.nb2), b / band.nb2 % band.nb1, b % band.nb2}, n[3] = {band.n0, band.n1, band.n2};
+    unsigned lo[3], hi[3];
+#pragma unroll
+    for (int a = 0; a < 3; ++a) {
+        lo[a] = min(bb[a] * band.stride, n[a] - 1);
+        hi[a] = min((bb[a] + 1) * band.stride, n[a] - 1);     // the last brick may be partial
+    }
+    unsigned below = 0;
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+        const unsigned i = c & 4 ? hi[0] : lo[0], j = c & 2 ? hi[1] : lo[1], k = c & 1 ? hi[2] : lo[2];
+        below += f[((size_t)i * band.n1 + j) * band.n2 + k] < level ? 1u : 0u;     // NaN is not below
+    }
+    raw[b] = below != 0 && below != 8;
+}
+
+// flags[b] = any raw flag in the 26-neighbourhood of b, clamped at the box.
+__global__ void band_dilate_kernel(const unsigned char* __restrict__ raw, unsigned nb0, unsigned nb1, unsigned nb2,
+                                   unsigned char* __restrict__ flags) {
+    const unsigned b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= nb0 * nb1 * nb2) return;
+    const unsigned b0 = b / (nb1 * nb2), b1 = b / nb2 % nb1, b2 = b % nb2;
+    unsigned char any = 0;
+    for (unsigned i = b0 ? b0 - 1 : 0; i <= min(b0 + 1, nb0 - 1); ++i)
+        for (unsigned j = b1 ? b1 - 1 : 0; j <= min(b1 + 1, nb1 - 1); ++j)
+            for (unsigned k = b2 ? b2 - 1 : 0; k <= min(b2 + 1, nb2 - 1); ++k) any |= raw[((size_t)i * nb1 + j) * nb2 + k];
+    flags[b] = any;
+}
+
+// The needed points in ascending linear index, in two passes over the lattice that evaluate Band::needed alike and keep no per-point
+// state: kEmit = false writes each tile's needed count (the low 16-bit field mc_scan_kernel scans); kEmit = true writes the points
+// to index[offsets[tile].x + rank].
+template <bool kEmit>
+__global__ void __launch_bounds__(kThreads) band_points_kernel(Band band, unsigned* __restrict__ tile_counts,
+                                                               const longlong2* __restrict__ offsets, int* __restrict__ index) {
+    __shared__ unsigned s_scan[kPer * kWarps + 1];
+    const unsigned n = band.n0 * band.n1 * band.n2, base = blockIdx.x * (unsigned)kTile;
+    unsigned cnt[kPer], kept = 0;
+#pragma unroll 1
+    for (int q = 0; q < kPer; ++q) {            // one copy of the test: unrolled, it spills
+        const unsigned idx = base + q * kThreads + threadIdx.x, r = idx / band.n2;
+        kept |= (idx < n && band.needed(r / band.n1, r % band.n1, idx % band.n2) ? 1u : 0u) << q;
+    }
+#pragma unroll
+    for (int q = 0; q < kPer; ++q) cnt[q] = kept >> q & 1u;
+    const unsigned total = tile_scan(cnt, s_scan);
+    if (!kEmit) {
+        if (threadIdx.x == 0) tile_counts[blockIdx.x] = total;
+        return;
+    }
+    const long long first = offsets[blockIdx.x].x;
+#pragma unroll
+    for (int q = 0; q < kPer; ++q)
+        if (kept >> q & 1u) index[first + cnt[q]] = (int)(base + q * kThreads + threadIdx.x);
+}
+
+// x[r] = (point, direction) of row index[r] of the lattice description (load_row: the points of the dense lattice query).
+__global__ void lattice_rows_kernel(RowSource src, const int* __restrict__ index, unsigned m, float* __restrict__ x) {
+    const unsigned r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= m) return;
+    float p[3], v[3];
+    load_row(src, index[r], p, v);
+    float* out = x + 6 * (size_t)r;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        out[c] = p[c];
+        out[3 + c] = v[c];
+    }
 }
 
 // One CTA: thread t owns a contiguous run of tiles.  offsets[b] = (first vertex, first triangle) of tile b.
@@ -1136,7 +1283,8 @@ extern "C" int b2r_mc_count(const float* field, int n0, int n1, int n2, float le
     const int tiles = (int)((n + kTile - 1) / kTile);
     char* s = static_cast<char*>(scratch);
     cudaStream_t st = (cudaStream_t)stream;
-    mc_count_kernel<<<tiles, kThreads, 0, st>>>(field, n0, n1, n2, level, (unsigned*)(s + l.words), (unsigned*)(s + l.counts));
+    mc_count_kernel<<<tiles, kThreads, 0, st>>>(field, n0, n1, n2, level, (unsigned*)(s + l.words), (unsigned*)(s + l.counts),
+                                                DenseMask{});
     mc_scan_kernel<<<1, kScanThreads, 0, st>>>((const unsigned*)(s + l.counts), tiles, (longlong2*)(s + l.offsets), totals_dev);
     B2R_LAUNCH_CHECK("b2r_mc_count");
     return 0;
@@ -1174,6 +1322,98 @@ extern "C" int b2r_mc_normals(const float* field, int n0, int n1, int n2, float 
     mc_normals_kernel<<<tiles, kThreads, 0, (cudaStream_t)stream>>>(field, n0, n1, n2, level, (const unsigned*)(s + l.words),
                                                                     (const longlong2*)(s + l.offsets), normals);
     B2R_LAUNCH_CHECK("b2r_mc_normals");
+    return 0;
+}
+
+namespace b2r {
+namespace mc {
+
+unsigned bricks(int n, int stride) { return (unsigned)(((long long)n - 2) / stride + 1); }      // ceil((n - 1) / stride), n >= 2
+
+Band make_band(int n0, int n1, int n2, int stride, const unsigned char* flags) {
+    return Band{flags, (unsigned)n0, (unsigned)n1, (unsigned)n2, bricks(n1, stride), bricks(n2, stride), (unsigned)stride};
+}
+
+// band_select scratch: the raw (undilated) flags, the tile counts and offsets of the needed points, and the totals
+struct BandLayout {
+    size_t raw, counts, offsets, totals, total;
+};
+
+BandLayout band_layout(int n0, int n1, int n2, int stride) {
+    const long long n = (long long)n0 * n1 * n2, tiles = (n + kTile - 1) / kTile;
+    BandLayout l;
+    l.raw = 0;
+    l.counts = l.raw + align256((size_t)bricks(n0, stride) * bricks(n1, stride) * bricks(n2, stride));
+    l.offsets = l.counts + align256((size_t)tiles * 4);
+    l.totals = l.offsets + align256((size_t)tiles * sizeof(longlong2));
+    l.total = l.totals + 256;
+    return l;
+}
+
+}  // namespace mc
+}  // namespace b2r
+
+extern "C" size_t b2r_band_scratch_bytes(int n0, int n1, int n2, int stride) {
+    if (n0 < 2 || n1 < 2 || n2 < 2 || (long long)n0 * n1 * n2 > INT32_MAX || stride < 2) return 0;
+    return b2r::mc::band_layout(n0, n1, n2, stride).total;
+}
+
+extern "C" int b2r_band_select(const float* field, int n0, int n1, int n2, float level, int stride, void* scratch,
+                               unsigned char* flags, int* index, long long* count_dev, void* stream) {
+    using namespace b2r::mc;
+    if (int rc = check_grid("b2r_band_select", n0, n1, n2)) return rc;
+    B2R_CHECK_ARG(stride >= 2, "b2r_band_select: stride = %d must be >= 2", stride);
+    B2R_CHECK_ARG(field && scratch && flags && index && count_dev, "b2r_band_select: NULL pointer");
+    B2R_CHECK_ARG(((uintptr_t)scratch & 15) == 0, "b2r_band_select: scratch must be 16-byte aligned");
+    const long long n = (long long)n0 * n1 * n2;
+    const BandLayout l = band_layout(n0, n1, n2, stride);
+    const unsigned nb0 = bricks(n0, stride), nb = nb0 * bricks(n1, stride) * bricks(n2, stride);
+    const int tiles = (int)((n + kTile - 1) / kTile);
+    char* s = static_cast<char*>(scratch);
+    unsigned char* raw = (unsigned char*)(s + l.raw);
+    cudaStream_t st = (cudaStream_t)stream;
+    const Band band = make_band(n0, n1, n2, stride, flags);
+    band_flag_kernel<<<(nb + 255) / 256, 256, 0, st>>>(field, band, nb0, level, raw);
+    band_dilate_kernel<<<(nb + 255) / 256, 256, 0, st>>>(raw, nb0, band.nb1, band.nb2, flags);
+    unsigned* counts = (unsigned*)(s + l.counts);
+    longlong2* offsets = (longlong2*)(s + l.offsets);
+    long long* totals = (long long*)(s + l.totals);
+    band_points_kernel<false><<<tiles, kThreads, 0, st>>>(band, counts, offsets, index);
+    mc_scan_kernel<<<1, kScanThreads, 0, st>>>(counts, tiles, offsets, totals);
+    band_points_kernel<true><<<tiles, kThreads, 0, st>>>(band, counts, offsets, index);
+    B2R_LAUNCH_CHECK("b2r_band_select");
+    return b2r::cuda_result(cudaMemcpyAsync(count_dev, totals, sizeof(long long), cudaMemcpyDeviceToDevice, st), "b2r_band_select");
+}
+
+extern "C" int b2r_lattice_rows(const b2r_mlp_input* in, const int* index, long long m, float* x, void* stream) {
+    using namespace b2r;
+    B2R_CHECK_ARG(in, "b2r_lattice_rows: NULL input description");
+    if (int rc = check_mlp_input(in)) return rc;
+    B2R_CHECK_ARG(in->grid_n > 0 || lattice_mode(in), "b2r_lattice_rows: the description must be grid_n or lattice_dims rows");
+    B2R_CHECK_ARG(m >= 0 && m <= INT32_MAX, "b2r_lattice_rows: m = %lld must be in [0, INT32_MAX]", m);
+    if (m == 0) return 0;
+    B2R_CHECK_ARG(index && x, "b2r_lattice_rows: NULL pointer");
+    mc::lattice_rows_kernel<<<(unsigned)((m + 255) / 256), 256, 0, (cudaStream_t)stream>>>(make_row_source(in), index, (unsigned)m, x);
+    B2R_LAUNCH_CHECK("b2r_lattice_rows");
+    return 0;
+}
+
+extern "C" int b2r_mc_count_band(const float* field, int n0, int n1, int n2, float level, const unsigned char* flags, int stride,
+                                 void* scratch, long long* totals_dev, void* stream) {
+    using namespace b2r::mc;
+    if (int rc = check_grid("b2r_mc_count_band", n0, n1, n2)) return rc;
+    B2R_CHECK_ARG(stride >= 2, "b2r_mc_count_band: stride = %d must be >= 2", stride);
+    B2R_CHECK_ARG(field && flags && scratch && totals_dev, "b2r_mc_count_band: NULL pointer");
+    B2R_CHECK_ARG(((uintptr_t)scratch & 15) == 0, "b2r_mc_count_band: scratch must be 16-byte aligned");
+    const long long n = (long long)n0 * n1 * n2;
+    const Layout l = layout(n);
+    const int tiles = (int)((n + kTile - 1) / kTile);
+    char* s = static_cast<char*>(scratch);
+    cudaStream_t st = (cudaStream_t)stream;
+    mc_count_kernel<<<tiles, kThreads, 0, st>>>(field, n0, n1, n2, level, (unsigned*)(s + l.words), (unsigned*)(s + l.counts),
+                                                make_band(n0, n1, n2, stride, flags));
+    mc_scan_kernel<<<1, kScanThreads, 0, st>>>((const unsigned*)(s + l.counts), tiles, (longlong2*)(s + l.offsets), totals_dev);
+    B2R_LAUNCH_CHECK("b2r_mc_count_band");
     return 0;
 }
 

@@ -25,6 +25,50 @@ def box_lattice(box_min, box_max, n):
     return dims, tuple(float(np.float32(v)) for v in lo), float(np.float32(step))
 
 
+def check_band_lattice(dims) -> None:
+    """RuntimeError unless a lattice of ``dims`` points fits the narrow-band export: its int32 point indices and marching cubes
+    take at most 2^31 - 1 points.  Runs on the host, so create_mesh raises it before any launch."""
+    points = math.prod(int(d) for d in dims)
+    if points > ops._INT32_MAX:
+        raise RuntimeError(f"lattice of {points} points; the narrow-band export and marching_cubes take at most 2^31 - 1")
+
+
+def coarse_index(dims, stride, device) -> torch.Tensor:
+    """int32 linear indices (ascending) of the coarse corners of bricks of ``stride`` cells: the points ``min(b * stride, n - 1)``
+    on every axis."""
+    axes = [torch.clamp(torch.arange(nb + 1, device=device) * stride, max=n - 1) for n, nb in zip(dims, ops.brick_dims(dims, stride))]
+    return ((axes[0][:, None, None] * dims[1] + axes[1][None, :, None]) * dims[2] + axes[2][None, None, :]).reshape(-1).to(torch.int32)
+
+
+def query_rows(model, field, index, *, grid=None, lattice=None, max_batch, precision=None) -> None:
+    """field.view(-1)[index] = -sigma of ``model`` at rows ``index`` of the ``grid`` or ``lattice`` description (the sigma-only MLP
+    on ``ops.lattice_rows`` x rows, ``max_batch`` rows per launch), so each value is the dense query's."""
+    flat = field.view(-1)
+    for b in range(0, index.shape[0], max_batch):
+        rows = index[b:b + max_batch]
+        raw = ops.mlp(model, x=ops._lattice_rows(rows, grid, lattice), precision=precision, sigma_only=True)
+        flat.index_copy_(0, rows.long(), -raw[:, 3])
+
+
+def band_field(model, dims, level, stride, *, grid=None, lattice=None, max_batch, precision=None):
+    """-sigma of ``model`` on the lattice of ``dims`` points queried only near the level set: at the coarse corners of bricks of
+    ``stride`` cells, then at the points ``ops.band_select`` lists for them; every other point holds +inf.  The lattice is one
+    ``grid = (N, 0, N^3)`` or ``lattice = (dims, origin, voxel, 0, count)`` description as ``ops.mlp`` takes it (query_rows).
+    Returns ``(field [n0,n1,n2], flags)``; synchronises with the host once, in ``ops.band_select``.  Besides the field, the
+    index list of ``ops.band_select`` (4 B per lattice point) is held until the band query ends."""
+    check_band_lattice(dims)
+    dev = next(model.parameters()).device
+    if dev.type != "cuda":
+        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    field = torch.full(tuple(dims), math.inf, dtype=torch.float32, device=dev)
+    with torch.no_grad():
+        query_rows(model, field, coarse_index(dims, stride, dev), grid=grid, lattice=lattice, max_batch=max_batch,
+                   precision=precision)
+        flags, index = ops.band_select(field, level, stride)
+        query_rows(model, field, index, grid=grid, lattice=lattice, max_batch=max_batch, precision=precision)
+    return field, flags
+
+
 def vertex_colors(model, verts, normals, precision=None):
     """uint8 [V,3] colours of the model's rgb head at each vertex, seen by a camera looking along ``-normals``
     (rows x = [vertex, -normal]), quantised on the device by ops.to8b."""
@@ -73,7 +117,7 @@ def write_ply(filename, verts, faces, normals=None, colors=None):
 
 
 def export(model, field, level, spacing, origin, ply_filename, normals, colors, precision, min_component_ratio=0.0,
-           smooth_iterations=0, max_faces=None):
+           smooth_iterations=0, max_faces=None, bricks=None):
     """Extract the level set of ``field`` (vertex normals toward increasing field), colour it with ``model`` and write the PLY.
     Returns (verts, faces, normals | None, colors | None) on the device.  A ``min_component_ratio`` above 0 removes the
     components with fewer triangles than that share of the largest one (ops.filter_components) before the colour query, so
@@ -81,15 +125,17 @@ def export(model, field, level, spacing, origin, ply_filename, normals, colors, 
     ``smooth_iterations`` above 0 then runs that many Taubin iterations (ops.smooth_mesh) before the colour query, and the
     normals become the smoothed mesh's own, so colours are sampled on the smoothed surface; the field normals are not computed.
     ``max_faces`` (an int >= 1) then decimates the mesh to that many triangles (ops.decimate_mesh; one host synchronisation per
-    round) before the colour query, so removed vertices cost no MLP rows, and the normals are the decimated mesh's own."""
+    round) before the colour query, so removed vertices cost no MLP rows, and the normals are the decimated mesh's own.
+    ``bricks = (stride, flags)`` limits the extraction to the flagged bricks (``ops.marching_cubes(bricks=...)``; the field of
+    ``band_field``)."""
     iterations = ops._check_int("iterations", smooth_iterations, 0, ops._INT32_MAX)
     budget = None if max_faces is None else ops._check_int("max_faces", max_faces, 1)
     want_normals = normals or colors
     own_normals = want_normals and (iterations or budget is not None)
     if want_normals and not own_normals:
-        verts, faces, nrm = ops.marching_cubes(field, level, spacing, origin, normals=True)
+        verts, faces, nrm = ops.marching_cubes(field, level, spacing, origin, normals=True, bricks=bricks)
     else:
-        (verts, faces), nrm = ops.marching_cubes(field, level, spacing, origin), None
+        (verts, faces), nrm = ops.marching_cubes(field, level, spacing, origin, bricks=bricks), None
     if min_component_ratio:
         # marching-cubes faces index their own vertices, so the index checks of ops.filter_components / ops.smooth_mesh are not needed
         verts, faces, nrm = ops._filter_components(verts, faces, ops._check_ratio(min_component_ratio), nrm)

@@ -16,6 +16,8 @@ There is no CPU path: tensors and models must live on a CUDA device.
 """
 from __future__ import annotations
 
+import math
+
 import numpy as np
 import torch
 from tqdm import tqdm
@@ -310,7 +312,7 @@ def density_lattice(model, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), 
 
 def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), threshold=50.0,
                 normals=True, colors=True, precision=None, max_batch=256 ** 3, min_component_ratio=0.0, smooth_iterations=0,
-                max_faces=None):
+                max_faces=None, narrow_band=None):
     """Mesh of a trained NeRF / SirenNeRF field on the device: the level set ``sigma = threshold`` of ``density_lattice``
     (marching cubes on -sigma at -threshold, so triangle and vertex normals point out of the object, toward lower density),
     the unit vertex normals, and the uint8 colour the model's rgb head gives each vertex seen by a camera looking along the
@@ -331,7 +333,24 @@ def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), 
     the open boundary where the surface meets the lattice box in place and never flip a face), so removed vertices cost no MLP
     rows.  The normals are then the decimated mesh's own area-weighted vertex normals (still out of the object) and the
     colours are sampled at the decimated vertices along them; the field normals are not computed.  Each round synchronises
-    with the host once, to read its collapse count.  None (the default) leaves the mesh at its extracted size."""
-    sigma, origin, voxel = density_lattice(model, box_min, box_max, N, max_batch=max_batch, precision=precision)
-    return mesh.export(model, sigma.neg_(), -float(threshold), voxel, origin, ply_filename, normals, colors, precision,
-                       min_component_ratio, smooth_iterations, max_faces)
+    with the host once, to read its collapse count.  None (the default) leaves the mesh at its extracted size.
+    ``narrow_band`` (an int B >= 2) queries the density only near the surface (mesh.band_field): at the corners of bricks of B
+    cells, then in the bricks whose corners are not all on one side of ``threshold`` and their 26 neighbours, and marching cubes
+    runs on those bricks only.  The mesh, normals and colours are the dense ones less the triangles outside those bricks, bit
+    for bit, so a surface the brick corners cannot see -- a piece that lies within a brick and its neighbours without changing
+    which side of the threshold any brick corner is on, such as a blob smaller than a brick -- is missed.  It adds one host
+    synchronisation, to size the band.  The lattice may hold at most 2^31 - 1 points (RuntimeError before any launch
+    otherwise), and the band's index list takes 4 B per lattice point beside the field.  None (the default) queries every
+    lattice point."""
+    stride = None if narrow_band is None else ops._check_int("narrow_band", narrow_band, 2, ops._INT32_MAX)
+    if stride is None:
+        sigma, origin, voxel = density_lattice(model, box_min, box_max, N, max_batch=max_batch, precision=precision)
+        field, bricks = sigma.neg_(), None
+    else:
+        dims, origin, voxel = mesh.box_lattice(box_min, box_max, N)
+        mesh.check_band_lattice(dims)
+        field, flags = mesh.band_field(model, dims, -float(threshold), stride, lattice=(dims, origin, voxel, 0, math.prod(dims)),
+                                       max_batch=int(max_batch), precision=precision)
+        bricks = (stride, flags)
+    return mesh.export(model, field, -float(threshold), voxel, origin, ply_filename, normals, colors, precision,
+                       min_component_ratio, smooth_iterations, max_faces, bricks)

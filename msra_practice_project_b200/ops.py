@@ -799,19 +799,95 @@ def to8b(x: torch.Tensor) -> torch.Tensor:
 _INT32_MAX = 2 ** 31 - 1
 
 
-def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, origin=(0.0, 0.0, 0.0), *, normals: bool = False):
+def _mc_field(field: torch.Tensor) -> torch.Tensor:
+    """``field`` as a contiguous [n0,n1,n2] float32 CUDA tensor with every n >= 2 and at most 2^31 - 1 points; RuntimeError
+    otherwise."""
+    field = _cuda_f32(field, "field")
+    if field.dim() != 3 or min(field.shape) < 2:
+        raise RuntimeError(f"field must be [n0,n1,n2] with every n >= 2, got {list(field.shape)}")
+    if field.numel() > _INT32_MAX:
+        raise RuntimeError(f"field has {field.numel()} points; marching_cubes takes at most 2^31 - 1")
+    return field
+
+
+def brick_dims(shape, stride: int) -> tuple:
+    """Bricks per axis of a lattice of ``shape`` points for bricks of ``stride`` cells: ``ceil((n - 1) / stride)`` each."""
+    return tuple((int(n) - 2) // stride + 1 for n in shape)
+
+
+def band_select(field: torch.Tensor, level: float, stride: int):
+    """Flagged bricks and needed points of a narrow-band query (b2r_band_select) on ``field`` [n0,n1,n2], whose values must be
+    valid at every coarse corner (the points ``min(b * stride, n - 1)`` on every axis) and may be +inf elsewhere.  Returns
+    ``(flags uint8 [nb0,nb1,nb2], index int32 [M])`` on the field's device: a brick is flagged when its 8 coarse corners are
+    not all on the same side of ``level`` (``field < level``, NaN not below), dilated by one brick over the 26-neighbourhood;
+    ``index`` lists, ascending, every point of the closure of a flagged brick and every point one step along one axis from
+    one.  Synchronises once with the host to read M.  The list is allocated for every lattice point (4 B each) before M is known;
+    ``index`` is a view of that allocation."""
+    field = _mc_field(field)
+    stride = _check_int("stride", stride, 2, _INT32_MAX)
+    n0, n1, n2 = (int(s) for s in field.shape)
+    dev = field.device
+    flags = torch.empty(brick_dims(field.shape, stride), dtype=torch.uint8, device=dev)
+    index = torch.empty((field.numel(),), dtype=torch.int32, device=dev)
+    count = torch.empty((1,), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        scratch = torch.empty((lib().b2r_band_scratch_bytes(n0, n1, n2, stride),), dtype=torch.uint8, device=dev)
+        check(lib().b2r_band_select(ptr(field), n0, n1, n2, float(level), stride, ptr(scratch), ptr(flags), ptr(index), ptr(count),
+                                    _stream(field)), "b2r_band_select")
+        return flags, index[:int(count.item())]
+
+
+def _lattice_rows(index: torch.Tensor, grid=None, lattice=None) -> torch.Tensor:
+    """lattice_rows for an index already known to lie in range."""
+    inp, _, _ = _make_input(None, None, None, grid, lattice)
+    x = torch.empty((index.shape[0], 6), dtype=torch.float32, device=index.device)
+    with torch.cuda.device(index.device):
+        check(lib().b2r_lattice_rows(C.byref(inp), ptr(index), index.shape[0], ptr(x), _stream(index)), "b2r_lattice_rows")
+    return x
+
+
+def lattice_rows(index: torch.Tensor, grid: tuple | None = None, lattice: tuple | None = None) -> torch.Tensor:
+    """x rows [M,6] = (point, zero direction) of rows ``index`` (int32 [M], on the device) of one ``grid`` or ``lattice``
+    description as ``mlp`` takes it (b2r_lattice_rows), so ``mlp(model, x=lattice_rows(index, ...))`` evaluates those rows'
+    points.  Checks that every index lies in [0, count) first (RuntimeError otherwise; one host synchronisation)."""
+    if (grid is None) == (lattice is None):
+        raise ValueError("give exactly one of grid / lattice")
+    if not isinstance(index, torch.Tensor) or not index.is_cuda or index.dtype != torch.int32 or index.dim() != 1:
+        raise RuntimeError("index must be a 1-d int32 CUDA tensor")
+    count = int((grid or lattice)[-1])
+    if index.numel():
+        lo, hi = (int(v) for v in torch.aminmax(index))
+        if lo < 0 or hi >= count:
+            raise RuntimeError(f"row indices span [{lo}, {hi}], outside [0, {count})")
+    return _lattice_rows(index.contiguous(), grid, lattice)
+
+
+def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, origin=(0.0, 0.0, 0.0), *, normals: bool = False,
+                   bricks: tuple | None = None):
     """Marching cubes of ``field`` [n0,n1,n2] (axis 0 slowest) at ``level`` on the device (b2r_mc_count / b2r_mc_emit; the
     table and its rule: oracle/marching_cubes.py).  Returns ``(verts [V,3] float32, faces [F,3] int32)`` on the field's
     device; vertex ``origin + (p + t e_a) * spacing`` lies on the lattice edge from point ``p`` along axis ``a``, and the
     triangle normals point from ``field < level`` to ``field >= level``.  Synchronises once with the host to read the
     mesh size (V, F), as ``torch.nonzero`` does.  Empty meshes are ``[0,3]`` tensors.
     ``normals=True`` also returns the unit vertex normals [V,3] (b2r_mc_normals: the field's central-difference gradient
-    interpolated along the vertex's edge, pointing toward increasing field; (0, 0, 0) where it vanishes)."""
-    field = _cuda_f32(field, "field")
-    if field.dim() != 3 or min(field.shape) < 2:
-        raise RuntimeError(f"field must be [n0,n1,n2] with every n >= 2, got {list(field.shape)}")
-    if field.numel() > _INT32_MAX:
-        raise RuntimeError(f"field has {field.numel()} points; marching_cubes takes at most 2^31 - 1")
+    interpolated along the vertex's edge, pointing toward increasing field; (0, 0, 0) where it vanishes).
+    ``bricks=(stride, flags)`` (flags uint8 [nb0,nb1,nb2] on the field's device, as ``band_select`` returns them) limits the
+    mesh to the flagged bricks (b2r_mc_count_band): the faces of cells in other bricks and the vertices on no edge of a cell
+    in a flagged brick are removed, and the rest keeps its order."""
+    field = _mc_field(field)
+    if bricks is not None:
+        if not isinstance(bricks, tuple) or len(bricks) != 2:
+            raise ValueError("bricks must be a tuple (stride, flags)")
+        stride = _check_int("stride", bricks[0], 2, _INT32_MAX)
+        flags = bricks[1]
+        if not isinstance(flags, torch.Tensor) or flags.dtype != torch.uint8 or not flags.is_cuda:
+            raise RuntimeError("brick flags must be a uint8 CUDA tensor")
+        if tuple(flags.shape) != brick_dims(field.shape, stride):
+            raise RuntimeError(f"brick flags must be {list(brick_dims(field.shape, stride))} for stride {stride}, "
+                               f"got {list(flags.shape)}")
+        if flags.device != field.device:
+            raise RuntimeError("field and brick flags must be on the same device")
+        flags = flags.contiguous()
     n0, n1, n2 = (int(s) for s in field.shape)
     level, spacing = float(level), float(spacing)
     ox, oy, oz = (float(o) for o in origin)
@@ -819,7 +895,11 @@ def marching_cubes(field: torch.Tensor, level: float, spacing: float = 1.0, orig
     scratch = torch.empty((lib().b2r_mc_scratch_bytes(n0, n1, n2),), dtype=torch.uint8, device=dev)
     totals = torch.empty((2,), dtype=torch.int64, device=dev)
     with torch.cuda.device(dev):
-        check(lib().b2r_mc_count(ptr(field), n0, n1, n2, level, ptr(scratch), ptr(totals), _stream(field)), "b2r_mc_count")
+        if bricks is None:
+            check(lib().b2r_mc_count(ptr(field), n0, n1, n2, level, ptr(scratch), ptr(totals), _stream(field)), "b2r_mc_count")
+        else:
+            check(lib().b2r_mc_count_band(ptr(field), n0, n1, n2, level, ptr(flags), stride, ptr(scratch), ptr(totals),
+                                          _stream(field)), "b2r_mc_count_band")
         n_verts, n_faces = (int(v) for v in totals.tolist())
         if n_verts > _INT32_MAX or n_faces > _INT32_MAX:
             raise RuntimeError(f"mesh of {n_verts} vertices / {n_faces} triangles: int32 vertex indices hold at most 2^31 - 1")

@@ -12,7 +12,7 @@ import torch
 from tqdm import tqdm
 
 from . import ops
-from .mesh import export as _export_mesh, write_ply  # noqa: F401  (pigan_render.write_ply is public)
+from .mesh import band_field, check_band_lattice, export as _export_mesh, write_ply  # noqa: F401  (pigan_render.write_ply is public)
 from .nerf_render import (REFERENCE_RAY_CHUNK, _draw_t_rand, get_rays, maps_to_numpy, raw_to_outputs, render_image_device, render_rays,
                           run_network, sample_pdf, to8b)
 
@@ -161,8 +161,9 @@ def density_grid(model, N=256, max_batch=64 ** 3, *, begin=0, count=None, precis
     return out[0] if len(out) == 1 else torch.cat(out)
 
 
-def _sdf_device(generator, N, max_batch, z, precision):
-    """-sigma of the generator conditioned on z (drawn when None) on the N^3 lattice, as a CUDA tensor [N,N,N] (x slowest)."""
+def _sdf_device(generator, N, max_batch, z, precision, band=None):
+    """-sigma of the generator conditioned on z (drawn when None) on the N^3 lattice, as a CUDA tensor [N,N,N] (x slowest).
+    With ``band = (level, stride)`` the narrow-band query of mesh.band_field instead: ``(sdf, flags)``."""
     dev = next(generator.parameters()).device
     if dev.type != "cuda":
         raise RuntimeError("generator parameters must live on a CUDA device: the B200 render path has no CPU fallback")
@@ -171,6 +172,9 @@ def _sdf_device(generator, N, max_batch, z, precision):
     with torch.no_grad():
         film_params = generator.get_mapping(z.to(dev))
         generator.set_film_params(film_params[0])
+        if band is not None:
+            return band_field(generator.film_siren_nerf, (N, N, N), band[0], band[1], grid=(N, 0, N ** 3), max_batch=max_batch,
+                              precision=precision)
         sdf = density_grid(generator.film_siren_nerf, N=N, max_batch=max_batch, precision=precision)
     return sdf.reshape(N, N, N)
 
@@ -185,7 +189,7 @@ def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=No
 
 
 def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None, normals=False,
-                colors=False, min_component_ratio=0.0, smooth_iterations=0, max_faces=None):
+                colors=False, min_component_ratio=0.0, smooth_iterations=0, max_faces=None, narrow_band=None):
     """``create_mesh`` (pi_GAN/utils.py:42-180) on the device: the sdf of ``create_mesh_sdf`` never leaves the GPU,
     ``ops.marching_cubes`` extracts its level set (the reference's skimage call at level -20: below = sigma > 20, so the
     triangle normals point out of the object), and only the mesh crosses to the host.  Returns ``(verts [V,3] float32,
@@ -209,8 +213,22 @@ def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level
     the open boundary where the surface meets the lattice box in place and never flip a face), so removed vertices cost no MLP
     rows.  The normals are then the decimated mesh's own area-weighted vertex normals (still out of the object) and the
     colours are sampled at the decimated vertices along them; the field normals are not computed.  Each round synchronises
-    with the host once, to read its collapse count.  None (the default) leaves the mesh at its extracted size."""
-    sdf = _sdf_device(generator, N, max_batch, z, precision)
+    with the host once, to read its collapse count.  None (the default) leaves the mesh at its extracted size.
+    ``narrow_band`` (an int B >= 2) queries the density only near the surface (mesh.band_field): at the corners of bricks of B
+    cells, then in the bricks whose corners are not all on one side of ``level`` and their 26 neighbours, and marching cubes
+    runs on those bricks only.  The mesh, normals and colours are the dense ones less the triangles outside those bricks, bit
+    for bit, so a surface the brick corners cannot see -- a piece that lies within a brick and its neighbours without changing
+    which side of the level any brick corner is on, such as a blob smaller than a brick -- is missed.  It adds one host
+    synchronisation, to size the band.  The lattice may hold at most 2^31 - 1 points (RuntimeError before any launch
+    otherwise), and the band's index list takes 4 B per lattice point beside the field.  None (the default) queries every
+    lattice point; ``create_mesh_sdf`` and ``density_grid`` always do."""
+    stride = None if narrow_band is None else ops._check_int("narrow_band", narrow_band, 2, ops._INT32_MAX)
+    if stride is None:
+        sdf, bricks = _sdf_device(generator, N, max_batch, z, precision), None
+    else:
+        check_band_lattice((N, N, N))
+        sdf, flags = _sdf_device(generator, N, max_batch, z, precision, (float(level), stride))
+        bricks = (stride, flags)
     out = _export_mesh(generator.film_siren_nerf, sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1), ply_filename, normals, colors,
-                       precision, min_component_ratio, smooth_iterations, max_faces)
+                       precision, min_component_ratio, smooth_iterations, max_faces, bricks)
     return out if (normals or colors) else out[:2]
