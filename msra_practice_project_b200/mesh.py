@@ -57,9 +57,7 @@ def band_field(model, dims, level, stride, *, grid=None, lattice=None, max_batch
     Returns ``(field [n0,n1,n2], flags)``; synchronises with the host once, in ``ops.band_select``.  Besides the field, the
     index list of ``ops.band_select`` (4 B per lattice point) is held until the band query ends."""
     check_band_lattice(dims)
-    dev = next(model.parameters()).device
-    if dev.type != "cuda":
-        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    dev = ops._model_args(model)[4]
     field = torch.full(tuple(dims), math.inf, dtype=torch.float32, device=dev)
     with torch.no_grad():
         query_rows(model, field, coarse_index(dims, stride, dev), grid=grid, lattice=lattice, max_batch=max_batch,

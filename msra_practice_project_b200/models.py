@@ -136,7 +136,7 @@ class NeRF(torch.nn.Module):
 
     def forward(self, x):
         from . import ops
-        return ops.mlp_points(self, x)
+        return ops.mlp(self, x=x)
 
 
 class _Siren(torch.nn.Linear):
@@ -162,7 +162,7 @@ class SirenNeRF(torch.nn.Module):
 
     def forward(self, x):
         from . import ops
-        return ops.mlp_points(self, x)
+        return ops.mlp(self, x=x)
 
 
 class _FilmSiren(torch.nn.Module):
@@ -202,7 +202,7 @@ class FilmSirenNeRF(torch.nn.Module):
         elif self.film_params is None:
             raise ValueError
         from . import ops
-        return ops.mlp_points(self, x)
+        return ops.mlp(self, x=x)
 
 
 class MappingNetwork(torch.nn.Module):

@@ -297,9 +297,7 @@ def density_lattice(model, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), 
     edge (mesh.box_lattice): ``(sigma [n0,n1,n2] on the device, origin, voxel)``, axis 0 slowest.  The points are made on the
     device from the lattice index with zero view direction; the bf16 NeRF path stops after the sigma head.  ``max_batch``
     bounds the points per launch."""
-    dev = _model_device(model)
-    if dev.type != "cuda":
-        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    dev = ops._model_args(model)[4]
     dims, origin, voxel = mesh.box_lattice(box_min, box_max, N)
     total = dims[0] * dims[1] * dims[2]
     sigma = torch.empty((total,), dtype=torch.float32, device=dev)

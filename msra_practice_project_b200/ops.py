@@ -108,22 +108,28 @@ def _last_sample_begin(kind: int, rows: int, spr: int, dev):
     return ls, (count, ids)
 
 
-def _last_sample_finish(kind: int, flat, film, use_dir, n_latents, rows_per_latent, inp, spr: int, keep, raw) -> int:
-    """Reads the number of flagged rays (the one host sync of the pass) and re-evaluates their last samples in fp32."""
-    count, ids = keep
+def _with_last_sample(want: bool, launch, kind: int, inp, spr: int, raw, weights, n_latents: int = 1,
+                      rows_per_latent: int = 0) -> None:
+    """``launch(ls)`` of a bf16 forward into ``raw`` (ls: a LastSample pointer, or None).  With ``want`` the forward lists the
+    rays whose last sample is in the bf16 error band; their count is read (the one host sync of the pass) and those last
+    samples are re-evaluated in fp32 with ``weights = (flat, film | None, use_dir)``."""
+    if not want:
+        launch(None)
+        return
+    flat, film, use_dir = weights
+    ls, (count, ids) = _last_sample_begin(kind, raw.shape[0], spr, raw.device)
+    launch(C.byref(ls))
     n_rays = ids.shape[0]
     n = min(int(count.item()), n_rays)
     last_sample_stats["calls"] += 1
     last_sample_stats["rays"] += int(n_rays)
     last_sample_stats["flagged"] += n
     if n == 0:
-        return 0
-    dev = raw.device
+        return
     ws_bytes = lib().b2r_mlp_f32_workspace_bytes(kind, n, 0) + ((n * 4 + 15) & ~15)
-    ws = torch.empty((ws_bytes // 4,), dtype=torch.float32, device=dev)
+    ws = torch.empty((ws_bytes // 4,), dtype=torch.float32, device=raw.device)
     check(lib().b2r_mlp_f32_last_sigma(kind, ptr(flat), ptr(film), int(use_dir), int(n_latents), int(rows_per_latent), C.byref(inp), int(spr),
                                        ids.data_ptr(), n, ptr(raw), ptr(ws), ws_bytes, _stream(raw)), "b2r_mlp_f32_last_sigma")
-    return n
 
 
 def _cuda_f32(t: torch.Tensor, name: str) -> torch.Tensor:
@@ -136,6 +142,17 @@ def _cuda_f32(t: torch.Tensor, name: str) -> torch.Tensor:
 
 def _stream(t: torch.Tensor) -> int:
     return torch.cuda.current_stream(t.device).cuda_stream
+
+
+def _model_args(model):
+    """``(net, kind, use_dir, params, device)`` of a radiance-field model: ``net`` unwrapped from DataParallel, ``params`` in
+    flat order (models.param_list); TypeError for an unknown model, RuntimeError unless its parameters are on a CUDA device."""
+    kind = models.model_kind(model)
+    net = model.module if isinstance(model, torch.nn.DataParallel) else model
+    ps = models.param_list(net, kind)
+    if ps[0].device.type != "cuda":
+        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    return net, kind, bool(getattr(net, "use_dir", True)), ps, ps[0].device
 
 
 # ---- K1 / K2 ---------------------------------------------------------------------------------------
@@ -288,17 +305,9 @@ class _Composite(torch.autograd.Function):
     @staticmethod
     def backward(ctx, g_rgb, g_depth, g_acc, _g_w):
         raw, z, keep = ctx.saved_tensors
-        n, s = z.shape
-        g_rgb = torch.zeros((n, 3), device=z.device) if g_rgb is None else _cuda_f32(g_rgb, "g_rgb")
-        g_depth = None if g_depth is None else _cuda_f32(g_depth, "g_depth")
-        g_acc = None if g_acc is None else _cuda_f32(g_acc, "g_acc")
-        d_raw = torch.empty(raw.shape, dtype=torch.float32, device=raw.device)
-        if n == 0:
-            return d_raw, None, None, None
-        with torch.cuda.device(z.device):
-            check(lib().b2r_composite_bwd(ptr(raw), ptr(z), keep.data_ptr(), ctx.dstride, n, s, ptr(g_rgb), ptr(g_depth),
-                                          ptr(g_acc), ptr(d_raw), _stream(z)), "b2r_composite_bwd")
-        return d_raw, None, None, None
+        if g_rgb is None:
+            g_rgb = torch.zeros((z.shape[0], 3), device=z.device)
+        return composite_backward((raw, z, keep, ctx.dstride), g_rgb, g_depth, g_acc), None, None, None
 
 
 def composite(raw, z_vals, rays_d, want_weights: bool = True, packed_out: torch.Tensor | None = None):
@@ -386,12 +395,7 @@ def _packed_weights(model, kind: int, flat: torch.Tensor, film: torch.Tensor | N
         hit = _pack_cache.get(model) if film is None else None
     if hit is not None and hit[0] == key:
         return hit[1]
-    nbytes = lib().b2r_mlp_tc_packed_bytes(kind)
-    if nbytes == 0:
-        raise RuntimeError(f"model kind {kind} has no tensor-core path in this build")
-    packed = torch.empty((nbytes,), dtype=torch.uint8, device=flat.device)
-    with torch.cuda.device(flat.device):
-        check(lib().b2r_mlp_tc_pack(kind, ptr(flat), ptr(film), int(use_dir), ptr(packed), _stream(flat)), "b2r_mlp_tc_pack")
+    packed = pack_tc(flat, kind, film, use_dir)
     if film is None:
         with _pack_lock:
             _pack_cache[model] = (key, packed)
@@ -425,22 +429,28 @@ def _make_input(rays, z, x, grid, lattice=None):
     return inp, int(count), ()
 
 
+def _mlp_f32_forward(kind: int, flat, film, use_dir, inp, raw, keep: int, gemm_mode: int) -> torch.Tensor:
+    """b2r_mlp_f32_fwd of the rows ``inp`` describes into ``raw``; returns the workspace, which with ``keep`` = 1 holds every
+    layer's output for b2r_mlp_f32_bwd.  ``gemm_mode`` 1 runs the GEMMs in tf32, 0 in fp32."""
+    dev = raw.device
+    ws_bytes = lib().b2r_mlp_f32_workspace_bytes(kind, raw.shape[0], keep)
+    ws = torch.empty((max(ws_bytes, 16) // 4,), dtype=torch.float32, device=dev)
+    with torch.cuda.device(dev):
+        check(lib().b2r_mlp_f32_fwd(kind, ptr(flat), ptr(film), int(use_dir), C.byref(inp), ptr(raw), ptr(ws), ws_bytes, keep,
+                                    gemm_mode, _stream(flat)), "b2r_mlp_f32_fwd")
+    return ws
+
+
 class _MlpF32(torch.autograd.Function):
     """fp32 forward that keeps every layer's output, and its reverse mode (K8)."""
 
     @staticmethod
     def forward(ctx, flat, film, kind, use_dir, rays, z, x, gemm_mode):
         inp, rows, keep = _make_input(rays, z, x, None)
-        ctx.gemm_mode = gemm_mode
-        dev = flat.device
-        raw = torch.empty((rows, 4), dtype=torch.float32, device=dev)
-        ws_bytes = lib().b2r_mlp_f32_workspace_bytes(kind, rows, 1)
-        ws = torch.empty((max(ws_bytes, 16) // 4,), dtype=torch.float32, device=dev)
-        with torch.cuda.device(dev):
-            check(lib().b2r_mlp_f32_fwd(kind, ptr(flat), ptr(film), int(use_dir), C.byref(inp), ptr(raw), ptr(ws), ws_bytes, 1,
-                                        gemm_mode, _stream(flat)), "b2r_mlp_f32_fwd")
-        ctx.kind, ctx.use_dir, ctx.rows = kind, use_dir, rows
-        ctx.keep = keep
+        raw = torch.empty((rows, 4), dtype=torch.float32, device=flat.device)
+        ws = _mlp_f32_forward(kind, flat, film, use_dir, inp, raw, 1, gemm_mode)
+        ctx.kind, ctx.use_dir, ctx.gemm_mode = kind, use_dir, gemm_mode
+        ctx.inp, ctx.keep = inp, keep          # the rows' description and the tensors it points into
         ctx.has_film = film is not None
         ctx.save_for_backward(flat, film if film is not None else flat.new_empty(0), raw, ws)
         return raw
@@ -449,10 +459,7 @@ class _MlpF32(torch.autograd.Function):
     def backward(ctx, d_raw):
         flat, film, raw, ws = ctx.saved_tensors
         film = film if ctx.has_film else None
-        rays = ctx.keep[0] if len(ctx.keep) == 2 else None
-        z = ctx.keep[1] if len(ctx.keep) == 2 else None
-        x = ctx.keep[0] if len(ctx.keep) == 1 else None
-        inp, rows, _ = _make_input(rays, z, x, None)
+        rows = raw.shape[0]
         dev = flat.device
         d_raw = _cuda_f32(d_raw, "d_raw")
         need_w = ctx.needs_input_grad[0]
@@ -464,7 +471,7 @@ class _MlpF32(torch.autograd.Function):
         sc_bytes = lib().b2r_mlp_f32_bwd_scratch_bytes(ctx.kind, rows)
         scratch = torch.empty((max(sc_bytes, 16) // 4,), dtype=torch.float32, device=dev)
         with torch.cuda.device(dev):
-            check(lib().b2r_mlp_f32_bwd(ctx.kind, ptr(flat), ptr(film), int(ctx.use_dir), C.byref(inp), ptr(raw), ptr(d_raw),
+            check(lib().b2r_mlp_f32_bwd(ctx.kind, ptr(flat), ptr(film), int(ctx.use_dir), C.byref(ctx.inp), ptr(raw), ptr(d_raw),
                                         ptr(ws), ptr(scratch), sc_bytes, ptr(d_flat), ptr(d_film), ctx.gemm_mode, _stream(flat)),
                   "b2r_mlp_f32_bwd")
         return d_flat, d_film, None, None, None, None, None, None
@@ -478,10 +485,7 @@ def _packed_bwd_weights(model, kind: int, flat: torch.Tensor) -> torch.Tensor:
         hit = _pack_bwd_cache.get(model)
     if hit is not None and hit[0] == key:
         return hit[1]
-    nbytes = lib().b2r_mlp_tc_bwd_packed_bytes(kind)
-    packed = torch.empty((nbytes,), dtype=torch.uint8, device=flat.device)
-    with torch.cuda.device(flat.device):
-        check(lib().b2r_mlp_tc_pack_bwd(kind, ptr(flat), ptr(packed), _stream(flat)), "b2r_mlp_tc_pack_bwd")
+    packed = pack_tc_bwd(flat, kind)
     with _pack_lock:
         _pack_bwd_cache[model] = (key, packed)
     return packed
@@ -489,7 +493,10 @@ def _packed_bwd_weights(model, kind: int, flat: torch.Tensor) -> torch.Tensor:
 
 def pack_tc(flat: torch.Tensor, kind: int, film=None, use_dir: bool = True) -> torch.Tensor:
     """b2r_mlp_tc_pack of a flat fp32 parameter tensor (no cache)."""
-    packed = torch.empty((lib().b2r_mlp_tc_packed_bytes(kind),), dtype=torch.uint8, device=flat.device)
+    nbytes = lib().b2r_mlp_tc_packed_bytes(kind)
+    if nbytes == 0:
+        raise RuntimeError(f"model kind {kind} has no tensor-core path in this build")
+    packed = torch.empty((nbytes,), dtype=torch.uint8, device=flat.device)
     with torch.cuda.device(flat.device):
         check(lib().b2r_mlp_tc_pack(kind, ptr(flat), ptr(film), int(use_dir), ptr(packed), _stream(flat)), "b2r_mlp_tc_pack")
     return packed
@@ -503,17 +510,41 @@ def pack_tc_bwd(flat: torch.Tensor, kind: int) -> torch.Tensor:
     return packed
 
 
-def tc_train_forward(packed: torch.Tensor, kind: int, rays: torch.Tensor, z: torch.Tensor):
-    """b2r_mlp_tc_train_fwd on (rays, z): (raw[rows,4], saved activation buffer)."""
-    inp, rows, keep = _make_input(rays, z, None, None)
+def _pack_film_batched(flat: torch.Tensor, film: torch.Tensor, use_dir, n_latents: int) -> torch.Tensor:
+    """b2r_mlp_tc_pack_film_batched: the FiLM-SIREN weights folded with each of the ``n_latents`` latents of ``film``,
+    [n_latents, packed bytes] (no cache)."""
+    packed = torch.empty((n_latents, lib().b2r_mlp_tc_packed_bytes(models.KIND_FILM)), dtype=torch.uint8, device=flat.device)
+    with torch.cuda.device(flat.device):
+        check(lib().b2r_mlp_tc_pack_film_batched(ptr(flat), ptr(film), int(use_dir), n_latents, ptr(packed), _stream(flat)),
+              "b2r_mlp_tc_pack_film_batched")
+    return packed
+
+
+def tc_train_forward(packed: torch.Tensor, kind: int, rays: torch.Tensor | None = None, z: torch.Tensor | None = None, *,
+                     x: torch.Tensor | None = None, n_latents: int = 1, rows_per_latent: int = 0, last_sample: tuple | None = None):
+    """Fused bf16 training forward on the rows of (rays, z) or x: (raw[rows,4], saved activation buffer).  One latent:
+    b2r_mlp_tc_train_fwd; FiLM-SIREN with ``n_latents`` > 1 (``packed`` [n_latents, bytes] from _pack_film_batched):
+    b2r_mlp_tc_train_fwd_film_batched, rows [b * rows_per_latent, (b+1) * rows_per_latent) on latent b.
+    ``last_sample = (flat, film | None, use_dir)``: on (rays, z) rows, the render's last-sample sign check, whose flagged rays
+    are re-evaluated in fp32 with those weights (_with_last_sample); None gives the raw bf16 forward."""
+    inp, rows, keep = _make_input(rays, z, x, None)
     dev = packed.device
     raw = torch.empty((rows, 4), dtype=torch.float32, device=dev)
     nbytes = lib().b2r_mlp_tc_train_saved_bytes(kind, rows)
     saved = torch.empty((max(nbytes, 16),), dtype=torch.uint8, device=dev)
-    if rows > 0:
-        with torch.cuda.device(dev):
-            check(lib().b2r_mlp_tc_train_fwd(kind, ptr(packed), C.byref(inp), ptr(raw), ptr(saved), nbytes, None, _stream(packed)),
+    if rows == 0:
+        return raw, saved
+
+    def launch(ls):
+        if n_latents == 1:
+            check(lib().b2r_mlp_tc_train_fwd(kind, ptr(packed), C.byref(inp), ptr(raw), ptr(saved), nbytes, ls, _stream(packed)),
                   "b2r_mlp_tc_train_fwd")
+        else:
+            check(lib().b2r_mlp_tc_train_fwd_film_batched(ptr(packed), n_latents, int(rows_per_latent), C.byref(inp), ptr(raw),
+                                                          ptr(saved), nbytes, ls, _stream(packed)), "b2r_mlp_tc_train_fwd_film_batched")
+    spr = z.shape[1] if rays is not None else 0
+    with torch.cuda.device(dev):
+        _with_last_sample(last_sample is not None and spr > 0, launch, kind, inp, spr, raw, last_sample, n_latents, rows_per_latent)
     del keep
     return raw, saved
 
@@ -560,26 +591,13 @@ class _MlpTcTrain(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, flat, model, kind, rays, z, x):
-        inp, rows, keep = _make_input(rays, z, x, None)
-        dev = flat.device
-        raw = torch.empty((rows, 4), dtype=torch.float32, device=dev)
         fd = flat.detach()
         packed = _packed_weights(model, kind, fd, None, True)
-        nbytes = lib().b2r_mlp_tc_train_saved_bytes(kind, rows)
-        saved = torch.empty((max(nbytes, 16),), dtype=torch.uint8, device=dev)
-        if rows > 0:
-            with torch.cuda.device(dev):
-                # opt-in (_EXACT_LAST_TRAIN): the same last-sample sign check as the render, so that autograd callers see the render's
-                # raw values; d sigma_last is zero on either side of the step, so the reverse mode is unaffected
-                spr = z.shape[1] if rays is not None else 0
-                ls, ls_keep = _last_sample_begin(kind, rows, spr, dev) if (_EXACT_LAST_TRAIN and spr > 0) else (None, None)
-                check(lib().b2r_mlp_tc_train_fwd(kind, ptr(packed), C.byref(inp), ptr(raw), ptr(saved), nbytes,
-                                                 C.byref(ls) if ls is not None else None, _stream(flat)), "b2r_mlp_tc_train_fwd")
-                if ls is not None:
-                    _last_sample_finish(kind, fd, None, True, 1, 0, inp, spr, ls_keep, raw)
-        ctx.model, ctx.kind, ctx.rows = model, kind, rows
+        # opt-in (_EXACT_LAST_TRAIN): the same last-sample sign check as the render, so that autograd callers see the render's raw
+        # values; d sigma_last is zero on either side of the step, so the reverse mode is unaffected
+        raw, saved = tc_train_forward(packed, kind, rays, z, x=x, last_sample=(fd, None, True) if _EXACT_LAST_TRAIN else None)
+        ctx.model, ctx.kind = model, kind
         ctx.save_for_backward(flat, raw, saved)
-        del keep
         return raw
 
     @staticmethod
@@ -587,17 +605,9 @@ class _MlpTcTrain(torch.autograd.Function):
         flat, raw, saved = ctx.saved_tensors
         if not ctx.needs_input_grad[0]:
             return (None,) * 6
-        dev = flat.device
         d_flat = torch.zeros_like(flat)
-        if ctx.rows == 0:
-            return d_flat, None, None, None, None, None
-        d_raw = _cuda_f32(d_raw, "d_raw")
-        packed_bwd = _packed_bwd_weights(ctx.model, ctx.kind, flat.detach())
-        sbytes = lib().b2r_mlp_tc_train_scratch_bytes(ctx.kind, ctx.rows)
-        scratch = torch.empty((sbytes,), dtype=torch.uint8, device=dev)
-        with torch.cuda.device(dev):
-            check(lib().b2r_mlp_tc_train_bwd(ctx.kind, ptr(packed_bwd), ctx.rows, ptr(raw), ptr(d_raw), ptr(saved), ptr(scratch),
-                                             sbytes, ptr(d_flat), _stream(flat)), "b2r_mlp_tc_train_bwd")
+        if raw.shape[0]:
+            tc_train_backward(_packed_bwd_weights(ctx.model, ctx.kind, flat.detach()), ctx.kind, raw, d_raw, saved, d_flat)
         return d_flat, None, None, None, None, None
 
 
@@ -611,32 +621,13 @@ class _MlpTcTrainFilm(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, flat, film, rays, z, x, rows_per_latent, use_dir=True):
-        kind = models.KIND_FILM
-        inp, rows, keep = _make_input(rays, z, x, None)
-        dev = flat.device
-        n_lat = 1 if film.dim() == 2 else film.shape[0]
-        raw = torch.empty((rows, 4), dtype=torch.float32, device=dev)
         fd, fl = flat.detach(), film.detach().contiguous()
-        packed = torch.empty((n_lat, lib().b2r_mlp_tc_packed_bytes(kind)), dtype=torch.uint8, device=dev)
-        nbytes = lib().b2r_mlp_tc_train_saved_bytes(kind, rows)
-        saved = torch.empty((max(nbytes, 16),), dtype=torch.uint8, device=dev)
-        if rows > 0:
-            with torch.cuda.device(dev):
-                check(lib().b2r_mlp_tc_pack_film_batched(ptr(fd), ptr(fl), int(use_dir), n_lat, ptr(packed), _stream(flat)), "b2r_mlp_tc_pack_film_batched")
-                spr = z.shape[1] if rays is not None else 0
-                ls, ls_keep = _last_sample_begin(kind, rows, spr, dev) if (_EXACT_LAST_TRAIN and spr > 0) else (None, None)
-                lsp = C.byref(ls) if ls is not None else None
-                if n_lat == 1:
-                    check(lib().b2r_mlp_tc_train_fwd(kind, ptr(packed), C.byref(inp), ptr(raw), ptr(saved), nbytes, lsp, _stream(flat)),
-                          "b2r_mlp_tc_train_fwd")
-                else:
-                    check(lib().b2r_mlp_tc_train_fwd_film_batched(ptr(packed), n_lat, int(rows_per_latent), C.byref(inp), ptr(raw), ptr(saved),
-                                                                  nbytes, lsp, _stream(flat)), "b2r_mlp_tc_train_fwd_film_batched")
-                if ls is not None:
-                    _last_sample_finish(kind, fd, fl, use_dir, n_lat, int(rows_per_latent), inp, spr, ls_keep, raw)
-        ctx.rows, ctx.n_lat, ctx.rows_per_latent, ctx.use_dir = rows, n_lat, int(rows_per_latent), int(bool(use_dir))
+        n_lat = 1 if film.dim() == 2 else film.shape[0]
+        raw, saved = tc_train_forward(_pack_film_batched(fd, fl, use_dir, n_lat), models.KIND_FILM, rays, z, x=x, n_latents=n_lat,
+                                      rows_per_latent=int(rows_per_latent),
+                                      last_sample=(fd, fl, use_dir) if _EXACT_LAST_TRAIN else None)
+        ctx.rows, ctx.n_lat, ctx.rows_per_latent, ctx.use_dir = raw.shape[0], n_lat, int(rows_per_latent), int(bool(use_dir))
         ctx.save_for_backward(flat, film, raw, saved)
-        del keep
         return raw
 
     @staticmethod
@@ -667,16 +658,11 @@ class _MlpTcTrainFilm(torch.autograd.Function):
 def mlp_film_batched_train(model, film: torch.Tensor, rays: torch.Tensor, z: torch.Tensor, rows_per_latent: int) -> torch.Tensor:
     """Differentiable counterpart of mlp_film_batched: FiLM-SIREN on (rays, z) rows for B latents in one launch sequence with the
     autograd graph to the model's parameters and to film[B,9,512] (fused tensor-core training path, bf16 arithmetic)."""
-    kind = models.model_kind(model)
-    net = model.module if isinstance(model, torch.nn.DataParallel) else model
-    if kind != models.KIND_FILM:
+    if models.model_kind(model) != models.KIND_FILM:
         raise TypeError("mlp_film_batched_train needs a FilmSirenNeRF model")
-    use_dir = bool(getattr(net, "use_dir", True))
     if rows_per_latent <= 0 or rows_per_latent % 512 != 0:
         raise RuntimeError("rows_per_latent must be a positive multiple of 512")
-    ps = models.param_list(net, kind)
-    if ps[0].device.type != "cuda":
-        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    net, kind, use_dir, _, _ = _model_args(model)
     if film.dim() != 3 or tuple(film.shape[1:]) != (9, 512) or not film.is_cuda:
         raise RuntimeError(f"film must be a CUDA tensor [B,9,512], got {tuple(film.shape)}")
     return _MlpTcTrainFilm.apply(models.flat_params(net, kind), film.float(), rays, z, None, int(rows_per_latent), use_dir)
@@ -694,15 +680,9 @@ def mlp(model, rays: torch.Tensor | None = None, z: torch.Tensor | None = None, 
 
     bf16 inference on ray samples -- (rays, z), or x with ``samples_per_ray`` given -- also runs the last-sample sign check
     (see _EXACT_LAST above) unless ``exact_last_sample`` is False."""
-    kind = models.model_kind(model)
+    net, kind, use_dir, ps, dev = _model_args(model)
     if kind == models.KIND_SIREN:
         sigma_only = False                       # no such kernel for SirenNeRF: the full evaluation is a superset
-    net = model.module if isinstance(model, torch.nn.DataParallel) else model
-    use_dir = bool(getattr(net, "use_dir", True))
-    ps = models.param_list(net, kind)
-    dev = ps[0].device
-    if dev.type != "cuda":
-        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
     film = None
     if kind == models.KIND_FILM:
         film = models.film_tensor(net)
@@ -725,44 +705,30 @@ def mlp(model, rays: torch.Tensor | None = None, z: torch.Tensor | None = None, 
     raw = torch.empty((rows, 4), dtype=torch.float32, device=dev)
     if rows == 0:
         return raw
+    if precision != "bf16":
+        _mlp_f32_forward(kind, flat, film, use_dir, inp, raw, 0, 1 if precision == "tf32" else 0)
+        return raw
+    packed = _packed_weights(net, kind, flat, film, use_dir)
+
+    def launch(ls):
+        check(lib().b2r_mlp_tc_fwd(kind, ptr(packed), int(use_dir), C.byref(inp), ptr(raw), int(sigma_only), ls, _stream(flat)),
+              "b2r_mlp_tc_fwd")
+    spr = z.shape[1] if rays is not None else (int(samples_per_ray) if (x is not None and samples_per_ray) else 0)
+    want_last = (_EXACT_LAST if exact_last_sample is None else bool(exact_last_sample)) and spr > 0 and not sigma_only \
+        and rows % spr == 0
     with torch.cuda.device(dev):
-        if precision == "bf16":
-            packed = _packed_weights(net, kind, flat, film, use_dir)
-            spr = z.shape[1] if rays is not None else (int(samples_per_ray) if (x is not None and samples_per_ray) else 0)
-            want_last = (_EXACT_LAST if exact_last_sample is None else bool(exact_last_sample)) and spr > 0 and not sigma_only \
-                and rows % spr == 0
-            ls, ls_keep = _last_sample_begin(kind, rows, spr, dev) if want_last else (None, None)
-            check(lib().b2r_mlp_tc_fwd(kind, ptr(packed), int(use_dir), C.byref(inp), ptr(raw), int(sigma_only),
-                                       C.byref(ls) if ls is not None else None, _stream(flat)), "b2r_mlp_tc_fwd")
-            if ls is not None:
-                _last_sample_finish(kind, flat, film, use_dir, 1, 0, inp, spr, ls_keep, raw)
-        else:
-            ws_bytes = lib().b2r_mlp_f32_workspace_bytes(kind, rows, 0)
-            ws = torch.empty((max(ws_bytes, 16) // 4,), dtype=torch.float32, device=dev)
-            check(lib().b2r_mlp_f32_fwd(kind, ptr(flat), ptr(film), int(use_dir), C.byref(inp), ptr(raw), ptr(ws), ws_bytes, 0,
-                                        1 if precision == "tf32" else 0, _stream(flat)), "b2r_mlp_f32_fwd")
+        _with_last_sample(want_last, launch, kind, inp, spr, raw, (flat, film, use_dir))
     del keep
     return raw
-
-
-def mlp_points(model, x: torch.Tensor) -> torch.Tensor:
-    """``network(x)`` for x[M,6] (the call of nerf/render.py:73 and pi_GAN/utils.py:86)."""
-    return mlp(model, x=x)
 
 
 def mlp_film_batched(model, film: torch.Tensor, rays: torch.Tensor, z: torch.Tensor, rows_per_latent: int,
                      sigma_only: bool = False, exact_last_sample: bool | None = None) -> torch.Tensor:
     """FiLM-SIREN on (rays, z) rows for B latents in ONE launch (Generator.forward's per-latent loop, pi_GAN/modules.py:176-184):
     film[B,9,512]; rows [b * rows_per_latent, (b+1) * rows_per_latent) use latent b.  Inference only (bf16 tensor-core kernel)."""
-    kind = models.model_kind(model)
-    if kind != models.KIND_FILM:
+    if models.model_kind(model) != models.KIND_FILM:
         raise TypeError("mlp_film_batched needs a FilmSirenNeRF model")
-    net = model.module if isinstance(model, torch.nn.DataParallel) else model
-    use_dir = bool(getattr(net, "use_dir", True))
-    ps = models.param_list(net, kind)
-    dev = ps[0].device
-    if dev.type != "cuda":
-        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    net, kind, use_dir, ps, dev = _model_args(model)
     film = _cuda_f32(film.detach(), "film")
     if film.dim() != 3 or tuple(film.shape[1:]) != (9, 512):
         raise RuntimeError(f"film must be [B,9,512], got {tuple(film.shape)}")
@@ -772,17 +738,14 @@ def mlp_film_batched(model, film: torch.Tensor, rays: torch.Tensor, z: torch.Ten
     if rows == 0:
         return raw
     n_lat = film.shape[0]
-    packed = torch.empty((n_lat, lib().b2r_mlp_tc_packed_bytes(kind)), dtype=torch.uint8, device=dev)
+    packed = _pack_film_batched(flat, film, use_dir, n_lat)
+
+    def launch(ls):
+        check(lib().b2r_mlp_tc_fwd_film_batched(ptr(packed), n_lat, int(rows_per_latent), C.byref(inp), ptr(raw), int(sigma_only), ls,
+                                                _stream(flat)), "b2r_mlp_tc_fwd_film_batched")
+    want_last = (_EXACT_LAST if exact_last_sample is None else bool(exact_last_sample)) and not sigma_only
     with torch.cuda.device(dev):
-        check(lib().b2r_mlp_tc_pack_film_batched(ptr(flat), ptr(film), int(use_dir), n_lat, ptr(packed), _stream(flat)),
-              "b2r_mlp_tc_pack_film_batched")
-        spr = z.shape[1]
-        want_last = (_EXACT_LAST if exact_last_sample is None else bool(exact_last_sample)) and not sigma_only
-        ls, ls_keep = _last_sample_begin(kind, rows, spr, dev) if want_last else (None, None)
-        check(lib().b2r_mlp_tc_fwd_film_batched(ptr(packed), n_lat, int(rows_per_latent), C.byref(inp), ptr(raw), int(sigma_only),
-                                                C.byref(ls) if ls is not None else None, _stream(flat)), "b2r_mlp_tc_fwd_film_batched")
-        if ls is not None:
-            _last_sample_finish(kind, flat, film, use_dir, n_lat, int(rows_per_latent), inp, spr, ls_keep, raw)
+        _with_last_sample(want_last, launch, kind, inp, z.shape[1], raw, (flat, film, use_dir), n_lat, int(rows_per_latent))
     del keep
     return raw
 
@@ -1016,13 +979,21 @@ def filter_components(verts: torch.Tensor, faces: torch.Tensor, ratio: float, no
     return _filter_components(verts, faces, r, normals)
 
 
+def _mesh_adjacency(faces: torch.Tensor, n_verts: int, scratch: torch.Tensor | None = None) -> torch.Tensor:
+    """b2r_mesh_adjacency of ``faces`` over ``n_verts`` vertices into ``scratch`` (allocated for this mesh when None; one sized
+    for a larger mesh also serves, the layout starts at its beginning); returns the scratch."""
+    if scratch is None:
+        scratch = torch.empty((lib().b2r_mesh_adj_scratch_bytes(n_verts, faces.shape[0]),), dtype=torch.uint8, device=faces.device)
+    check(lib().b2r_mesh_adjacency(ptr(faces), faces.shape[0], n_verts, ptr(scratch), _stream(faces)), "b2r_mesh_adjacency")
+    return scratch
+
+
 def _smooth_mesh(verts: torch.Tensor, faces: torch.Tensor, iterations: int, normals: bool):
     """smooth_mesh for faces already known to index [0, V): (verts', normals' | None), no host synchronisation."""
     dev, n_verts, n_faces = verts.device, verts.shape[0], faces.shape[0]
     with torch.cuda.device(dev):
         st = _stream(verts)
-        scratch = torch.empty((lib().b2r_mesh_adj_scratch_bytes(n_verts, n_faces),), dtype=torch.uint8, device=dev)
-        check(lib().b2r_mesh_adjacency(ptr(faces), n_faces, n_verts, ptr(scratch), st), "b2r_mesh_adjacency")
+        scratch = _mesh_adjacency(faces, n_verts)
         out = verts
         if iterations:
             out = torch.empty_like(verts)
@@ -1065,12 +1036,12 @@ def _decimate_mesh(verts: torch.Tensor, faces: torch.Tensor, max_faces: int, sta
         scratch = torch.empty((lib().b2r_mesh_decimate_scratch_bytes(n_verts, n_faces),), dtype=torch.uint8, device=dev)
         sel_keys = torch.empty((n_verts,), dtype=torch.int64, device=dev)
         counts = torch.empty((2,), dtype=torch.int64, device=dev)
-        check(lib().b2r_mesh_adjacency(ptr(faces), n_faces, n_verts, ptr(adj), st), "b2r_mesh_adjacency")
+        _mesh_adjacency(faces, n_verts, adj)
         quadrics = torch.empty((n_verts, 10), dtype=torch.float64, device=dev)
         check(lib().b2r_mesh_quadrics(ptr(verts), n_faces, n_verts, ptr(adj), ptr(quadrics), st), "b2r_mesh_quadrics")
         while n_faces > max_faces:
             if rounds:
-                check(lib().b2r_mesh_adjacency(ptr(faces), n_faces, n_verts, ptr(adj), st), "b2r_mesh_adjacency")
+                _mesh_adjacency(faces, n_verts, adj)
             check(lib().b2r_mesh_decimate_round(ptr(verts), ptr(quadrics), n_faces, n_verts, ptr(adj), ptr(scratch), ptr(sel_keys),
                                                 ptr(counts), st), "b2r_mesh_decimate_round")
             selected = int(counts[0])

@@ -98,8 +98,7 @@ def render_batch(model, film_params, poses, width, height, focal, near, far, coa
     after the sigma head; the images are bit-identical either way."""
     b = film_params.shape[0]
     w, h, sc, sf = int(width), int(height), int(coarse_sample_num), int(fine_sample_num)
-    if next(model.parameters()).device.type != "cuda":
-        raise RuntimeError("model parameters must live on a CUDA device: the B200 render path has no CPU fallback")
+    dev = ops._model_args(model)[4]
     used = precision or ops.get_mlp_precision()
     grad = torch.is_grad_enabled() and _needs_grad(model, film_params)
     grad_ok = ops.get_grad_precision() == "bf16" and isinstance(film_params, torch.Tensor)
@@ -113,7 +112,6 @@ def render_batch(model, film_params, poses, width, height, focal, near, far, coa
                                      fine_sample_num, t_rand=tr, precision=precision, exact_last_sample=exact_last_sample,
                                      coarse_sigma_only=coarse_sigma_only))
         return torch.stack(imgs).permute(0, 3, 1, 2).contiguous()
-    dev = next(model.parameters()).device
     n = w * h
     with torch.no_grad():
         if isinstance(poses, torch.Tensor) and poses.is_cuda:

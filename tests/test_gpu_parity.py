@@ -210,7 +210,7 @@ def test_mlp_fp32_nerf(golden):
     c, f = seeded_nerf()
     with torch.no_grad():
         out_c = ops.mlp(c, x=cu(k["mlp_x"]), precision="fp32").cpu().numpy()
-        out_f = f(cu(k["mlp_x"]))          # module call -> ops.mlp_points (default precision applies)
+        out_f = f(cu(k["mlp_x"]))          # module call -> ops.mlp (default precision applies)
         out_f32 = ops.mlp(f, x=cu(k["mlp_x"]), precision="fp32").cpu().numpy()
     np.testing.assert_allclose(out_c, k["nerf_seed0_coarse_out"], atol=1e-4, rtol=0)
     np.testing.assert_allclose(out_f32, k["nerf_seed0_fine_out"], atol=1e-4, rtol=0)
