@@ -404,6 +404,30 @@ int b2r_mesh_decimate_compact(const float* verts, const double* quadrics, const 
                               const long long* sel_keys, const long long* cut_or_null, void* scratch, float* verts_out,
                               double* quadrics_out, int* faces_out, void* stream);
 
+/* ---- texture atlas of a triangle mesh (no reference counterpart: colour detail of exported meshes beyond the vertices) -----
+ * Same mesh conventions and PRECONDITION as above; the layout, a pure function of (n_faces F, size R), is that of
+ * oracle/mesh_texture.py.  R is in [16, 16384].  Faces 2k and 2k+1 share cell k; the P = ceil(F / 2) cells sit C per row, C the
+ * smallest integer with C C >= P, each s = R / C texels square, with top-left texel (X, Y) = ((k % C) s, (k / C) s), row 0 at
+ * the top.  F must be at most 2 (R / 4)^2, so that s >= 4.  With L = s - 3, face 2k's corners 0, 1, 2 sit at the local texel
+ * centres (0, 0), (L, 0), (0, L) and face 2k+1's at (s-1, s-1), (2, s-1), (s-1, 2).  A local texel (x, y) is baked for face
+ * 2k+1 when x + y >= s and that face exists, for face 2k otherwise, so a bilinear lookup inside a face's UV triangle reads only
+ * texels baked for that face.  Texel weights: (a, b) = (x, y) for face 2k, (s-1-x, s-1-y) for 2k+1; (w0, w1, w2) =
+ * ((L-a-b) / L, a / L, b / L) when a + b <= L, (0, a / (a+b), b / (a+b)) otherwise.  Row r = k s^2 + y s + x, for the
+ * P s^2 rows of the used cells; [row_begin, +row_count) must lie within them.  Every float operation is rounded separately (no
+ * FMA; division and sqrt correctly rounded), so the results are reproducible bit for bit.
+ *   b2r_mesh_atlas_uvs:     uvs[F,3,2] (fp32): corner (x, y) of cell (X, Y) gets u = ((X+x) + 0.5) / R, v = 1 - ((Y+y) + 0.5) / R.
+ *   b2r_mesh_atlas_rows:    x[row_count,6] (fp32): row row_begin + i gets [p, -n^], p = (w0 v0 + w1 v1) + w2 v2 of its face's
+ *                           vertices per component, n^ the same sum of the vertex normals divided by sqrt((x x + y y) + z z), or
+ *                           (0, 0, 0) when that is 0 (the MLP query of b2r_mlp_tc_fwd on x then sees the surface point along -n^).
+ *   b2r_mesh_atlas_texture: raw[row_count,4] (fp32, 16-byte aligned; the MLP output on those rows): writes the b2r_to8b quantisation
+ *                           of raw[i][0..2] into the texel of row row_begin + i of texture[R,R,3] (uint8); other texels are left
+ *                           as they are (the caller zeroes the texture first). */
+int b2r_mesh_atlas_uvs(long long n_faces, int size, float* uvs, void* stream);
+int b2r_mesh_atlas_rows(const float* verts, const float* normals, const int* faces, long long n_faces, int size, long long row_begin,
+                        long long row_count, float* x, void* stream);
+int b2r_mesh_atlas_texture(const float* raw, long long n_faces, int size, long long row_begin, long long row_count,
+                           unsigned char* texture, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

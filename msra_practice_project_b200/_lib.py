@@ -108,6 +108,9 @@ SIGNATURES = {
                                           C.c_void_p]),
     "b2r_mesh_decimate_compact": (C.c_int, [c_float_p, C.c_void_p, C.c_void_p, c_ll, c_ll, C.c_void_p, C.c_void_p, C.c_void_p,
                                             c_float_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "b2r_mesh_atlas_uvs": (C.c_int, [c_ll, C.c_int, c_float_p, C.c_void_p]),
+    "b2r_mesh_atlas_rows": (C.c_int, [c_float_p, c_float_p, C.c_void_p, c_ll, C.c_int, c_ll, c_ll, c_float_p, C.c_void_p]),
+    "b2r_mesh_atlas_texture": (C.c_int, [c_float_p, c_ll, C.c_int, c_ll, c_ll, C.c_void_p, C.c_void_p]),
 }
 
 _lock = threading.Lock()

@@ -1247,6 +1247,102 @@ struct DecEmit {
     __device__ unsigned target(unsigned u) const { return dec_target(part, sel_keys, cut, u); }
 };
 
+// ---- texture atlas (b2r_mesh_atlas_uvs / _rows / _texture) -------------------------------------------------------------------
+// The layout is oracle/mesh_texture.py's: one chart per face, no unwrapping.  Faces 2k ("A") and 2k+1 ("B") share cell k of a
+// grid of C cells per row, each s x s texels (s = R / C, L = s - 3), with its top-left texel at ((k % C) s, (k / C) s).  A's
+// corners 0, 1, 2 sit at the local texel centres (0, 0), (L, 0), (0, L); B is A reflected through the cell centre.  A texel with
+// x + y >= s belongs to B (when B exists), any other to A, so a bilinear lookup inside a face's UV triangle reads only texels baked
+// for that face.  A texel's barycentric weights are integers over integers, each division correctly rounded.  Rows are numbered
+// r = k s^2 + y s + x over the used cells; one thread per row (or per face for the UVs).
+struct Atlas {
+    unsigned n_faces, per_row, s;
+};
+
+// The face texel (x, y) of cell k is baked for, and its weights on that face's corners 0, 1, 2: with (a, b) = (x, y) for A and
+// (s-1-x, s-1-y) for B, (L-a-b, a, b) / L inside the triangle, (0, a, b) / (a+b) beyond its hypotenuse.
+__device__ __forceinline__ unsigned atlas_texel(const Atlas& at, unsigned k, unsigned x, unsigned y, float (&w)[3]) {
+    const bool b_face = x + y >= at.s && 2 * k + 1 < at.n_faces;
+    const unsigned a = b_face ? at.s - 1 - x : x, b = b_face ? at.s - 1 - y : y, l = at.s - 3;
+    if (a + b <= l) {
+        w[0] = __fdiv_rn((float)(l - a - b), (float)l);
+        w[1] = __fdiv_rn((float)a, (float)l);
+        w[2] = __fdiv_rn((float)b, (float)l);
+    } else {
+        w[0] = 0.f;
+        w[1] = __fdiv_rn((float)a, (float)(a + b));
+        w[2] = __fdiv_rn((float)b, (float)(a + b));
+    }
+    return 2 * k + (b_face ? 1u : 0u);
+}
+
+// x[i] = [p, -n^] of row row_begin + i: p = (w0 p0 + w1 p1) + w2 p2 per component, n^ the same sum of the corner normals divided
+// by sqrt((x x + y y) + z z), or (0, 0, 0) when that is 0 (mesh_normals_kernel's division), every operation rounded separately.
+__global__ void __launch_bounds__(kThreads) atlas_rows_kernel(const float* __restrict__ p, const float* __restrict__ nrm,
+                                                              const int* __restrict__ faces, Atlas at, long long row_begin,
+                                                              long long n, float* __restrict__ x) {
+    const long long i = blockIdx.x * (long long)kThreads + threadIdx.x;
+    if (i >= n) return;
+    const unsigned long long r = (unsigned long long)(row_begin + i), ss = (unsigned long long)at.s * at.s;
+    const unsigned t = (unsigned)(r % ss);
+    float w[3];
+    const unsigned f = atlas_texel(at, (unsigned)(r / ss), t % at.s, t / at.s, w);
+    float q[3], m[3];
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const size_t v = 3 * (size_t)faces[3 * (size_t)f + c];
+#pragma unroll
+        for (int k = 0; k < 3; ++k) {
+            const float pq = __fmul_rn(w[c], p[v + k]), pm = __fmul_rn(w[c], nrm[v + k]);
+            q[k] = c ? __fadd_rn(q[k], pq) : pq;
+            m[k] = c ? __fadd_rn(m[k], pm) : pm;
+        }
+    }
+    const float len = __fsqrt_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], m[0]), __fmul_rn(m[1], m[1])), __fmul_rn(m[2], m[2])));
+    float* o = x + 6 * (size_t)i;
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        o[k] = q[k];
+        o[3 + k] = -(len > 0.f ? __fdiv_rn(m[k], len) : 0.f);
+    }
+}
+
+// b2r_to8b's quantisation: (uint8)(255 * clip(v, 0, 1)), float32 product, truncation toward zero.
+__device__ __forceinline__ unsigned char atlas_to8b(float v) {
+    return (unsigned char)__float2uint_rz(__fmul_rn(255.0f, fminf(fmaxf(v, 0.0f), 1.0f)));
+}
+
+// The rgb of raw[i] (row row_begin + i) quantised into its texel of the uint8 [R, R, 3] texture.
+__global__ void __launch_bounds__(kThreads) atlas_texture_kernel(const float4* __restrict__ raw, Atlas at, unsigned size,
+                                                                 long long row_begin, long long n, unsigned char* __restrict__ tex) {
+    const long long i = blockIdx.x * (long long)kThreads + threadIdx.x;
+    if (i >= n) return;
+    const unsigned long long r = (unsigned long long)(row_begin + i), ss = (unsigned long long)at.s * at.s;
+    const unsigned k = (unsigned)(r / ss), t = (unsigned)(r % ss);
+    const size_t col = (size_t)(k % at.per_row) * at.s + t % at.s, row = (size_t)(k / at.per_row) * at.s + t / at.s;
+    const float4 v = raw[i];
+    unsigned char* o = tex + 3 * (row * size + col);
+    o[0] = atlas_to8b(v.x);
+    o[1] = atlas_to8b(v.y);
+    o[2] = atlas_to8b(v.z);
+}
+
+// uv[f][c] = (((X + x) + 0.5) / R, 1 - ((Y + y) + 0.5) / R) of face f's corner c at local texel (x, y) of its cell.
+__global__ void __launch_bounds__(kThreads) atlas_uvs_kernel(Atlas at, unsigned size, float* __restrict__ uv) {
+    const unsigned f = blockIdx.x * kThreads + threadIdx.x;
+    if (f >= at.n_faces) return;
+    const unsigned k = f >> 1, s = at.s, l = s - 3;
+    const unsigned cx = (k % at.per_row) * s, cy = (k / at.per_row) * s;
+    const unsigned ax[3] = {0, l, 0}, ay[3] = {0, 0, l};
+    const float rf = (float)size;
+    float* o = uv + 6 * (size_t)f;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        const unsigned x = f & 1u ? s - 1 - ax[c] : ax[c], y = f & 1u ? s - 1 - ay[c] : ay[c];
+        o[2 * c] = __fdiv_rn(__fadd_rn((float)(cx + x), 0.5f), rf);
+        o[2 * c + 1] = __fsub_rn(1.0f, __fdiv_rn(__fadd_rn((float)(cy + y), 0.5f), rf));
+    }
+}
+
 int check_grid(const char* what, int n0, int n1, int n2) {
     B2R_CHECK_ARG(n0 >= 2 && n1 >= 2 && n2 >= 2, "%s: every axis needs n >= 2 (got %d x %d x %d)", what, n0, n1, n2);
     B2R_CHECK_ARG((long long)n0 * n1 * n2 <= INT32_MAX, "%s: n0*n1*n2 = %lld exceeds INT32_MAX", what, (long long)n0 * n1 * n2);
@@ -1657,6 +1753,78 @@ extern "C" int b2r_mesh_decimate_compact(const float* verts, const double* quadr
     compact_kernel<<<tiles, kThreads, 0, st>>>(
         DecEmit{verts, quadrics, part, sel_keys, cut_or_null, (const float*)(s + l.place), verts_out, quadrics_out}, faces,
         (unsigned)n_faces, (unsigned)n_verts, (const unsigned*)(s + l.tail.vword), (const longlong2*)(s + l.tail.offsets), faces_out);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+namespace {
+
+// The atlas of n_faces faces in a size x size texture and its row count (cells * s^2), after the checks every atlas call shares.
+int atlas_args(const char* what, long long n_faces, int size, b2r::mc::Atlas& at, long long& rows) {
+    B2R_CHECK_ARG(n_faces >= 0 && n_faces <= INT32_MAX, "%s: n_faces = %lld must be in [0, INT32_MAX]", what, n_faces);
+    B2R_CHECK_ARG(size >= 16 && size <= 16384, "%s: size = %d must be in [16, 16384]", what, size);
+    const long long q = size / 4;
+    B2R_CHECK_ARG(n_faces <= 2 * q * q, "%s: %lld faces do not fit a %d x %d atlas, which holds at most %lld (cells of 4 x 4 texels)",
+                  what, n_faces, size, size, 2 * q * q);
+    const long long cells = (n_faces + 1) / 2;
+    long long c = (long long)std::sqrt((double)cells);
+    while (c * c < cells) ++c;
+    while (c > 0 && (c - 1) * (c - 1) >= cells) --c;
+    at.n_faces = (unsigned)n_faces;
+    at.per_row = (unsigned)c;
+    at.s = c ? (unsigned)(size / c) : 0u;
+    rows = cells * at.s * at.s;
+    return 0;
+}
+
+int atlas_rows_args(const char* what, long long n_faces, int size, long long row_begin, long long row_count, b2r::mc::Atlas& at) {
+    long long rows = 0;
+    if (int rc = atlas_args(what, n_faces, size, at, rows)) return rc;
+    B2R_CHECK_ARG(row_begin >= 0 && row_count >= 0 && row_begin <= rows - row_count,
+                  "%s: rows [%lld, +%lld) outside the atlas's %lld rows", what, row_begin, row_count, rows);
+    return 0;
+}
+
+}  // namespace
+
+extern "C" int b2r_mesh_atlas_uvs(long long n_faces, int size, float* uvs, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_atlas_uvs";
+    Atlas at;
+    long long rows = 0;
+    if (int rc = atlas_args(what, n_faces, size, at, rows)) return rc;
+    B2R_CHECK_ARG(uvs || !n_faces, "%s: NULL uvs with n_faces > 0", what);
+    if (!n_faces) return 0;
+    atlas_uvs_kernel<<<blocks_of(n_faces, kThreads), kThreads, 0, (cudaStream_t)stream>>>(at, (unsigned)size, uvs);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_atlas_rows(const float* verts, const float* normals, const int* faces, long long n_faces, int size,
+                                   long long row_begin, long long row_count, float* x, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_atlas_rows";
+    Atlas at;
+    if (int rc = atlas_rows_args(what, n_faces, size, row_begin, row_count, at)) return rc;
+    B2R_CHECK_ARG((verts && normals && faces && x) || !row_count, "%s: NULL verts / normals / faces / x with row_count > 0", what);
+    if (!row_count) return 0;
+    atlas_rows_kernel<<<blocks_of(row_count, kThreads), kThreads, 0, (cudaStream_t)stream>>>(verts, normals, faces, at, row_begin,
+                                                                                             row_count, x);
+    B2R_LAUNCH_CHECK(what);
+    return 0;
+}
+
+extern "C" int b2r_mesh_atlas_texture(const float* raw, long long n_faces, int size, long long row_begin, long long row_count,
+                                      unsigned char* texture, void* stream) {
+    using namespace b2r::mc;
+    const char* what = "b2r_mesh_atlas_texture";
+    Atlas at;
+    if (int rc = atlas_rows_args(what, n_faces, size, row_begin, row_count, at)) return rc;
+    B2R_CHECK_ARG((raw && texture) || !row_count, "%s: NULL raw / texture with row_count > 0", what);
+    if (!row_count) return 0;
+    B2R_CHECK_ARG(((uintptr_t)raw & 15) == 0, "%s: raw must be 16-byte aligned", what);
+    atlas_texture_kernel<<<blocks_of(row_count, kThreads), kThreads, 0, (cudaStream_t)stream>>>((const float4*)raw, at, (unsigned)size,
+                                                                                                row_begin, row_count, texture);
     B2R_LAUNCH_CHECK(what);
     return 0;
 }

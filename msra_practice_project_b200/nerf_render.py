@@ -310,7 +310,7 @@ def density_lattice(model, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), 
 
 def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), box_max=(1.5, 1.5, 1.5), threshold=50.0,
                 normals=True, colors=True, precision=None, max_batch=256 ** 3, min_component_ratio=0.0, smooth_iterations=0,
-                max_faces=None, narrow_band=None):
+                max_faces=None, narrow_band=None, texture=None):
     """Mesh of a trained NeRF / SirenNeRF field on the device: the level set ``sigma = threshold`` of ``density_lattice``
     (marching cubes on -sigma at -threshold, so triangle and vertex normals point out of the object, toward lower density),
     the unit vertex normals, and the uint8 colour the model's rgb head gives each vertex seen by a camera looking along the
@@ -339,7 +339,15 @@ def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), 
     which side of the threshold any brick corner is on, such as a blob smaller than a brick -- is missed.  It adds one host
     synchronisation, to size the band.  The lattice may hold at most 2^31 - 1 points (RuntimeError before any launch
     otherwise), and the band's index list takes 4 B per lattice point beside the field.  None (the default) queries every
-    lattice point."""
+    lattice point.
+    ``texture`` (an int R in [16, 16384]) bakes the colour of the final mesh -- after the component filter, the smoothing and
+    the decimation -- into an R x R texture (mesh.bake_texture: one chart per face, every texel queried on the surface along
+    the inward normal that the vertex colours use, ``max_batch`` rows per launch), so the colour detail no longer depends on
+    the vertex count.  The mesh may have at most 2 * (R // 4)^2 faces (ValueError otherwise; ``max_faces`` bounds it).  The
+    result gains ``(uvs [F,3,2] float32, texture [R,R,3] uint8)``; with ``ply_filename`` the PLY's faces carry
+    ``texcoord`` lists, its header names the texture, and the texture is written as ``<stem>.png`` beside it.  None (the
+    default) bakes nothing."""
+    texture = None if texture is None else ops._check_int("texture", texture, *ops.ATLAS_SIZES)
     stride = None if narrow_band is None else ops._check_int("narrow_band", narrow_band, 2, ops._INT32_MAX)
     if stride is None:
         sigma, origin, voxel = density_lattice(model, box_min, box_max, N, max_batch=max_batch, precision=precision)
@@ -351,4 +359,4 @@ def create_mesh(model, ply_filename=None, N=256, *, box_min=(-1.5, -1.5, -1.5), 
                                        max_batch=int(max_batch), precision=precision)
         bricks = (stride, flags)
     return mesh.export(model, field, -float(threshold), voxel, origin, ply_filename, normals, colors, precision,
-                       min_component_ratio, smooth_iterations, max_faces, bricks)
+                       min_component_ratio, smooth_iterations, max_faces, bricks, texture, int(max_batch))

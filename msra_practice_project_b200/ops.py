@@ -1084,3 +1084,47 @@ def decimate_mesh(verts: torch.Tensor, faces: torch.Tensor, max_faces: int):
     max_faces = _check_int("max_faces", max_faces, 1)
     verts, faces, _ = _mesh_args(verts, faces)
     return _decimate_mesh(verts, faces, max_faces)
+
+
+ATLAS_SIZES = (16, 16384)
+
+
+def atlas_layout(n_faces: int, size: int):
+    """``(cells, per_row, s)`` of the per-face texture atlas of ``n_faces`` triangles in a ``size`` x ``size`` texture
+    (include/b2r.h, oracle/mesh_texture.py): faces 2k and 2k+1 share cell k, ``cells = ceil(n_faces / 2)`` cells sit ``per_row``
+    to a row (the smallest C with C * C >= cells) and each is ``s = size // per_row`` texels square; the atlas has
+    ``cells * s * s`` texel rows.  ``size`` must be an int in [16, 16384] and ``n_faces`` at most ``2 * (size // 4) ** 2``, so
+    that every cell has at least 4 x 4 texels (ValueError otherwise).  Host arithmetic only."""
+    size = _check_int("texture size", size, *ATLAS_SIZES)
+    n_faces = _check_int("n_faces", n_faces, 0, _INT32_MAX)
+    limit = 2 * (size // 4) ** 2
+    if n_faces > limit:
+        raise ValueError(f"{n_faces} faces do not fit a {size} x {size} texture atlas: it holds at most {limit} "
+                         f"(2 * (size // 4)^2, cells of 4 x 4 texels); use a larger texture or fewer faces (max_faces)")
+    cells = (n_faces + 1) // 2
+    per_row = math.isqrt(cells - 1) + 1 if cells else 0
+    return cells, per_row, size // per_row if per_row else 0
+
+
+def _atlas_uvs(n_faces: int, size: int, device) -> torch.Tensor:
+    """float32 [F,3,2] UVs of the atlas of ``n_faces`` faces (b2r_mesh_atlas_uvs); the layout is known to fit."""
+    uvs = torch.empty((n_faces, 3, 2), dtype=torch.float32, device=device)
+    with torch.cuda.device(device):
+        check(lib().b2r_mesh_atlas_uvs(n_faces, size, ptr(uvs), torch.cuda.current_stream(device).cuda_stream), "b2r_mesh_atlas_uvs")
+    return uvs
+
+
+def _atlas_rows(verts: torch.Tensor, faces: torch.Tensor, normals: torch.Tensor, size: int, begin: int, count: int) -> torch.Tensor:
+    """x rows [count,6] = [surface point, -unit normal] of atlas texel rows [begin, +count) (b2r_mesh_atlas_rows), for a mesh
+    already checked by _mesh_args and a layout known to fit."""
+    x = torch.empty((count, 6), dtype=torch.float32, device=verts.device)
+    check(lib().b2r_mesh_atlas_rows(ptr(verts), ptr(normals), ptr(faces), faces.shape[0], size, begin, count, ptr(x), _stream(verts)),
+          "b2r_mesh_atlas_rows")
+    return x
+
+
+def _atlas_texture(raw: torch.Tensor, n_faces: int, size: int, begin: int, texture: torch.Tensor) -> None:
+    """Quantises raw[:, :3] (the MLP output of atlas rows [begin, +len(raw))) into ``texture`` [R,R,3] uint8
+    (b2r_mesh_atlas_texture)."""
+    check(lib().b2r_mesh_atlas_texture(ptr(raw), n_faces, size, begin, raw.shape[0], ptr(texture), _stream(raw)),
+          "b2r_mesh_atlas_texture")

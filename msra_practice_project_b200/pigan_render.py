@@ -187,7 +187,7 @@ def create_mesh_sdf(generator, N=256, max_batch=64 ** 3, *, z=None, precision=No
 
 
 def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level=-20.0, z=None, precision=None, normals=False,
-                colors=False, min_component_ratio=0.0, smooth_iterations=0, max_faces=None, narrow_band=None):
+                colors=False, min_component_ratio=0.0, smooth_iterations=0, max_faces=None, narrow_band=None, texture=None):
     """``create_mesh`` (pi_GAN/utils.py:42-180) on the device: the sdf of ``create_mesh_sdf`` never leaves the GPU,
     ``ops.marching_cubes`` extracts its level set (the reference's skimage call at level -20: below = sigma > 20, so the
     triangle normals point out of the object), and only the mesh crosses to the host.  Returns ``(verts [V,3] float32,
@@ -219,7 +219,15 @@ def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level
     which side of the level any brick corner is on, such as a blob smaller than a brick -- is missed.  It adds one host
     synchronisation, to size the band.  The lattice may hold at most 2^31 - 1 points (RuntimeError before any launch
     otherwise), and the band's index list takes 4 B per lattice point beside the field.  None (the default) queries every
-    lattice point; ``create_mesh_sdf`` and ``density_grid`` always do."""
+    lattice point; ``create_mesh_sdf`` and ``density_grid`` always do.
+    ``texture`` (an int R in [16, 16384]) bakes the conditioned generator's colour on the final mesh -- after the component
+    filter, the smoothing and the decimation -- into an R x R texture (mesh.bake_texture: one chart per face, every texel
+    queried on the surface along the inward normal, ``max_batch`` rows per launch).  The mesh may have at most 2 * (R // 4)^2
+    faces (ValueError otherwise; ``max_faces`` bounds it).  The return value is then ``(verts, faces, normals | None,
+    colors | None, uvs [F,3,2] float32, texture [R,R,3] uint8)``; with ``ply_filename`` the PLY's faces carry ``texcoord``
+    lists, its header names the texture, and the texture is written as ``<stem>.png`` beside it.  None (the default) bakes
+    nothing."""
+    texture = None if texture is None else ops._check_int("texture", texture, *ops.ATLAS_SIZES)
     stride = None if narrow_band is None else ops._check_int("narrow_band", narrow_band, 2, ops._INT32_MAX)
     if stride is None:
         sdf, bricks = _sdf_device(generator, N, max_batch, z, precision), None
@@ -228,5 +236,5 @@ def create_mesh(generator, ply_filename=None, N=256, max_batch=64 ** 3, *, level
         sdf, flags = _sdf_device(generator, N, max_batch, z, precision, (float(level), stride))
         bricks = (stride, flags)
     out = _export_mesh(generator.film_siren_nerf, sdf, level, 0.2 / (N - 1), (-0.1, -0.1, -0.1), ply_filename, normals, colors,
-                       precision, min_component_ratio, smooth_iterations, max_faces, bricks)
-    return out if (normals or colors) else out[:2]
+                       precision, min_component_ratio, smooth_iterations, max_faces, bricks, texture, int(max_batch))
+    return out if (normals or colors or texture is not None) else out[:2]

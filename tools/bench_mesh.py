@@ -30,7 +30,16 @@ and on the NeRF 512^3 mesh down to 1,000,000: the number of rounds and the colla
 and the peak of torch's allocator over the call above what was allocated before it.  For the NeRF mesh also one whole
 create_mesh(max_faces=1_000_000) call against create_mesh() on the same field, each split into the call without a PLY (device
 work and the host reads) and the D2H copy + PLY write of its outputs, and whether the decimated call equals its stages
-(ops.decimate_mesh, the mesh normals, the colour query)."""
+(ops.decimate_mesh, the mesh normals, the colour query).
+
+The "texture" entries (``--texture`` runs them and the decimation entries) time texture baking (mesh.bake_texture) on the NeRF
+512^3 mesh decimated to 1,000,000 faces with a 4096^2 texture and on the pi-GAN 512^3 mesh decimated to 25,000 faces with a
+2048^2 texture (when the decimation stops above the budget and the atlas cannot hold the mesh, the refusal is recorded
+and the smallest power-of-two texture that holds it is baked instead): device ms (events, median of 5 after a warm-up) of the UVs (b2r_mesh_atlas_uvs), the rows (b2r_mesh_atlas_rows),
+the MLP query on them and the texture write (b2r_mesh_atlas_texture); the least bytes each new kernel moves against the copy
+peak; the D2H copy of the UVs and the texture; the host time of the PNG and of the textured PLY; and one whole
+create_mesh(max_faces=..., texture=...) call against the same call without the texture (device work and host reads, then with
+the files written), with whether the textured call equals its stages."""
 import json
 import os
 import statistics
@@ -379,6 +388,113 @@ def decimation_lines(gen):
     return res
 
 
+TEX_NERF, TEX_PIGAN = 4096, 2048
+
+
+def atlas_bytes(n_verts, n_faces, rows):
+    """Least bytes of the atlas kernels, from the mesh's and atlas's sizes: the UVs write 24 B per face; the rows read every face
+    (12 B) and its vertices and normals (24 B per vertex) once and write 24 B per row; the texture write reads 16 B and writes 3 B
+    per row."""
+    return {"uvs": 24 * n_faces, "rows": 12 * n_faces + 24 * n_verts + 24 * rows, "texture": 19 * rows}
+
+
+def texture_times(model, verts, faces, normals, size):
+    """Device ms of the atlas stages (one batch: every row at once), their least bytes against the copy peak, the D2H copy and
+    the PNG / PLY host time, and a check against mesh.bake_texture."""
+    dev = verts.device
+    nf = faces.shape[0]
+    cells, per_row, s = ops.atlas_layout(nf, size)
+    rows = cells * s * s
+    ms = {}
+    ms["uvs"], uvs = _timed(lambda: ops._atlas_uvs(nf, size, dev), 5)
+    ms["rows"], x = _timed(lambda: ops._atlas_rows(verts, faces, normals, size, 0, rows), 5)
+    with torch.no_grad():
+        ms["mlp"], raw = _timed(lambda: ops.mlp(model, x=x), 5)
+    tex = torch.zeros((size, size, 3), dtype=torch.uint8, device=dev)
+    ms["texture"], _ = _timed(lambda: ops._atlas_texture(raw, nf, size, 0, tex), 5)
+    ref = mesh.bake_texture(model, verts, faces, normals, size)
+    out = {"V": int(verts.shape[0]), "F": int(nf), "size": size, "cells": cells, "per_row": per_row, "cell_texels": s, "rows": rows,
+           "equals_bake_texture": bool(torch.equal(ref[0], uvs) and torch.equal(ref[1], tex))}
+    nb = atlas_bytes(int(verts.shape[0]), nf, rows)
+    for k in ("uvs", "rows", "mlp", "texture"):
+        out[f"{k}_ms"] = round(ms[k], 4)
+        if k in nb:
+            out[f"{k}_min_bytes"] = nb[k]
+            out[f"{k}_GBs"] = round(nb[k] / (ms[k] * 1e-3) / 1e9, 1)
+            out[f"{k}_frac_of_copy_peak"] = round(nb[k] / (ms[k] * 1e-3) / 1e9 / COPY_PEAK_GBS, 3)
+    out["mlp_rows_per_s_G"] = round(rows / (ms["mlp"] * 1e-3) / 1e9, 3)
+    out["bake_device_ms"] = round(sum(ms.values()), 3)
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    uv_h, tex_h = uvs.cpu().numpy(), tex.cpu().numpy()
+    out["d2h_uvs_texture_ms"] = round((time.perf_counter() - t0) * 1e3, 2)
+    with tempfile.TemporaryDirectory() as tmp:
+        t0 = time.perf_counter()
+        mesh.write_png(os.path.join(tmp, "m.png"), tex_h)
+        out["png_host_ms"] = round((time.perf_counter() - t0) * 1e3, 1)
+        out["png_bytes"] = os.path.getsize(os.path.join(tmp, "m.png"))
+        v_h, f_h, n_h = verts.cpu().numpy(), faces.cpu().numpy(), normals.cpu().numpy()
+        t0 = time.perf_counter()
+        mesh.write_ply(os.path.join(tmp, "m.ply"), v_h, f_h, n_h, None, uv_h, "m.png")
+        out["textured_ply_host_ms"] = round((time.perf_counter() - t0) * 1e3, 1)
+        out["textured_ply_bytes"] = os.path.getsize(os.path.join(tmp, "m.ply"))
+    del x, raw, tex, uvs, ref
+    torch.cuda.empty_cache()
+    return out
+
+
+def _wall(fn):
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    out = fn()
+    torch.cuda.synchronize()
+    return (time.perf_counter() - t0) * 1e3, out
+
+
+def texture_lines(gen, z):
+    res = {}
+    torch.manual_seed(0)
+    net = models.NeRF().cuda()
+    with torch.no_grad():
+        net.output_layer_sigma.weight.mul_(100.0)
+        net.output_layer_sigma.bias.zero_()
+    sigma, origin, voxel = nerf_render.density_lattice(net, N=512)
+    thr = float(torch.quantile(sigma.flatten()[::97].float(), 0.7))
+    del sigma
+    torch.cuda.empty_cache()
+    cases = (("nerf_512", lambda **kw: nerf_render.create_mesh(net, N=512, threshold=thr, **kw), net, DEC_NERF, TEX_NERF),
+             ("pigan_512", lambda **kw: pigan_render.create_mesh(gen, N=512, z=z, normals=True, colors=True, **kw), gen.film_siren_nerf,
+              DEC_PIGAN, TEX_PIGAN))
+    for name, call, model, budget, size in cases:
+        plain_ms, plain = _wall(lambda: call(max_faces=budget))
+        asked = {"texture_asked": size}
+        try:
+            ops.atlas_layout(plain[1].shape[0], size)
+        except ValueError as e:
+            # the decimation can stop above the budget (no edge left that passes its rules); bake at the smallest power of two
+            # whose atlas holds the mesh
+            asked["texture_asked_error"] = str(e)
+            size = next(r for r in (8192, 16384) if plain[1].shape[0] <= 2 * (r // 4) ** 2)
+        d = {**asked, **texture_times(model, plain[0], plain[1], plain[2], size)}
+        d["create_mesh_no_texture_no_files_ms"] = round(plain_ms, 1)
+        tex_ms, out = _wall(lambda: call(max_faces=budget, texture=size))
+        d["create_mesh_texture_no_files_ms"] = round(tex_ms, 1)
+        ref = mesh.bake_texture(model, plain[0], plain[1], plain[2], size)
+        d["create_mesh_texture_equals_stages"] = bool(all(torch.equal(a, b) for a, b in zip(out, tuple(plain) + ref)))
+        del out, ref
+        with tempfile.TemporaryDirectory() as tmp:
+            path = os.path.join(tmp, "m.ply")
+            ms, _ = _wall(lambda: call(max_faces=budget, ply_filename=path))
+            d["create_mesh_no_texture_with_ply_ms"] = round(ms, 1)
+            ms, _ = _wall(lambda: call(max_faces=budget, texture=size, ply_filename=path))
+            d["create_mesh_texture_with_ply_png_ms"] = round(ms, 1)
+            d["ply_bytes"], d["png_bytes"] = os.path.getsize(path), os.path.getsize(os.path.join(tmp, "m.png"))
+        res[name] = d
+        del plain
+        torch.cuda.empty_cache()
+    return res
+
+
 def main():
     smi = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
     print("gpu:", smi.stdout.strip().splitlines()[0] if smi.returncode == 0 and smi.stdout.strip() else "unknown")
@@ -392,6 +508,12 @@ def main():
         net.output_layer_sigma[0].weight.mul_(100.0)
         net.output_layer_sigma[0].bias.zero_()
         gen.set_film_params(gen.get_mapping(z)[0])
+    if "--texture" in sys.argv[1:]:
+        smi2 = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"], capture_output=True,
+                              text=True)
+        print(json.dumps({"metric": "texture baking and decimation on the device", "gpu": smi2.stdout.strip(), "copy_peak_GBs": COPY_PEAK_GBS,
+                          "texture": texture_lines(gen, z), "decimation": decimation_lines(gen)}))
+        return
     if "--decimation" in sys.argv[1:]:
         print(json.dumps({"metric": "mesh decimation on the device", "gpu": smi.stdout.strip(), "decimation": decimation_lines(gen)}))
         return
